@@ -81,7 +81,13 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-verify", action="store_true", help="skip the oracle check of one window per distinct shard (outside the timed region)")
     ap.add_argument("--cli-sample-kb", type=int, default=5000, help="BAM sample for the command-line (from-BAM) tier; 0 = skip (one fixture holds at most ~12 Mb of this depth: 32-bit base offsets)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the result arrays of the last timed step (every shard, in shard order; rank 0 under "
+                         "torchrun) as float64 DIR/<name>.npy, at most 64 MB in all; every shard then gets its own seeded inputs unless "
+                         "--distinct-shards is given, so that runs with the same arguments can be compared output for output")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     a.cfg = dict(CONFIGS[a.config])
     if a.quality == "wide":
         a.cfg["edge_mode"] = 2
@@ -216,6 +222,43 @@ def verify_shard(sh, res_arrays, an_names, an):
     return w, dev
 
 
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(out_dir, per_shard):
+    """Result arrays of every shard, concatenated in shard order, as float64 out_dir/<name>.npy; seg_off is rebased to the
+    concatenation, and a 64-bit word becomes two columns, its low and high 32 bits (float64 holds those exactly).  Every
+    value written is finite: where a statistic is NaN (the reference prints "NA": too few sites or SNPs) or infinite, the
+    value is 0 and out_dir/<name>_na.npy holds 1 there (0 elsewhere).  An array too large for its share of DUMP_BYTES is
+    cut to a fixed, seeded sample of its rows (the same rows of <name>_na), whose row numbers go to out_dir/<name>_rows.npy."""
+    out = {}
+    for k in per_shard[0]:
+        parts = [r[k] for r in per_shard]
+        if k == "seg_off":
+            base = np.cumsum([0] + [int(p[-1]) for p in parts])
+            parts = [p[:-1] + b for p, b in zip(parts, base[:-1])] + [base[-1:]]
+        a = np.concatenate(parts)
+        if a.size == 0:
+            continue
+        if a.dtype == np.uint64:
+            a = np.stack([a & np.uint64(0xffffffff), a >> np.uint64(32)], axis=1)
+        a = a.astype(np.float64)
+        na = ~np.isfinite(a)
+        out[k] = {k: np.where(na, 0.0, a), k + "_na": na.astype(np.float64)} if na.any() else {k: a}
+    os.makedirs(out_dir, exist_ok=True)
+    left = DUMP_BYTES - 3 * 256 * len(out)                   # room for the .npy headers
+    for i, (k, g) in enumerate(sorted(out.items(), key=lambda kv: sum(a.nbytes for a in kv[1].values()))):
+        share = left // (len(out) - i)
+        n, nbytes = len(g[k]), sum(a.nbytes for a in g.values())
+        if nbytes > share:
+            rows = np.sort(np.random.default_rng(0).choice(n, share // (nbytes // n + 8), replace=False))
+            g = {name: a[rows] for name, a in g.items()}
+            g[k + "_rows"] = rows.astype(np.float64)
+        for name, a in g.items():
+            np.save(os.path.join(out_dir, name + ".npy"), a)
+            left -= a.nbytes
+
+
 def run_b200(args):
     import torch
     import pbtest
@@ -233,13 +276,14 @@ def run_b200(args):
         an |= pbtest.AN[a]
     shards = []
     t_gen = time.time()
-    distinct = args.distinct_shards or (n_shards if (os.cpu_count() or 8) // world >= 8 else min(n_shards, 3))
+    # a dump must see the same inputs whatever the host's cores and free memory are
+    distinct = args.distinct_shards or (n_shards if args.dump_outputs or (os.cpu_count() or 8) // world >= 8 else min(n_shards, 3))
     bytes_per_pos = (cfg["n_ingroup"] + cfg["has_outgroup"]) * cfg["depth"] * 1.75          # pinned bytes per reference position
     try:        # pinned + transient copies of every distinct shard and rank: stay well inside the host's memory
         import psutil
         per_shard = 2.2 * bytes_per_pos * shard_len
         fit = int(psutil.virtual_memory().available * 0.5 / max(1, world) / per_shard)
-        if not args.distinct_shards:
+        if not args.distinct_shards and not args.dump_outputs:
             distinct = max(1, min(distinct, fit))
     except Exception:
         pass
@@ -380,6 +424,7 @@ def run_b200(args):
         torch.cuda.synchronize()
         step_ms += e0.elapsed_time(e1)
     barrier()
+    last_step = [pbtest.result_arrays(c.res) for c in ctxs] if args.dump_outputs and rank == 0 else None
     launches = sum(c.kernel_launches() for c in ctxs) - launches0
     # the stages alone: one more pass with the shards strictly one after the other (library events, pb_stage_times)
     seq_ms = 0.0
@@ -461,6 +506,8 @@ def run_b200(args):
         if args.cli_sample_kb != 0:
             cli_len = int(min(args.contig_mb, 5.0) * 1e6) if args.cli_sample_kb < 0 else int(min(args.cli_sample_kb * 1000, args.contig_mb * 1e6))
             line["cli_from_bam"] = cli_from_bam(args, cli_len)
+    if last_step:
+        dump_outputs(args.dump_outputs, last_step)
     if rank == 0:
         print(json.dumps(line))
     for c in ctxs:

@@ -272,7 +272,7 @@ def test_index_builder_serves_the_same_records(tmp_path, fxname):
         assert np.array_equal(got["pos"], pos[idx])
 
 
-@pytest.mark.skipif(not pbtest.have_ref(), reason="reference binary not built (needs /root/reference)")
+@pytest.mark.skipif(not pbtest.have_ref(), reason="the original POPBAM 0.3 is not built into oracle/_ref/ (make -C oracle ref REF=<its sources>)")
 def test_reference_reads_our_index(tmp_path):
     """The unmodified reference, given the index `popbam index` wrote, prints its golden output."""
     popbam_b200.build()

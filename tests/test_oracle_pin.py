@@ -75,7 +75,7 @@ def test_site_logic_known_answers():
         assert (cb[:n] == r["cb_out"][:n]).all()
 
 
-@pytest.mark.skipif(not pbtest.have_ref(), reason="reference binary not built (no /root/reference)")
+@pytest.mark.skipif(not pbtest.have_ref(), reason="the original POPBAM 0.3 is not built into oracle/_ref/ (make -C oracle ref REF=<its sources>)")
 def test_oracle_vs_live_reference(tmp_path):
     fx = pbtest.Fixture(contig_len=20500, n_ingroup=7, has_outgroup=1, depth=16.0, snp_density=0.02, edge_mode=1, seed=977)
     bam, fa = fx.write_files(tmp_path / "live")
