@@ -61,6 +61,10 @@ typedef enum pb_status {
 #define PB_AN_HAPLO_DXY     0x200u  /* pop_haplo.cpp:325   calc_minDxy    (haplo -o 2)    */
 #define PB_AN_SNP           0x400u  /* pop_snp.cpp:148     per-segregating-site rows      */
 #define PB_AN_TREE          0x800u  /* pop_tree.cpp:472    difference matrix incl. the reference taxon (tree) */
+/* extensions (no counterpart in the reference; each is the companion of one reference bit, --extra-stats)    */
+#define PB_AN_THETA_W       0x1000u /* Watterson's theta from the SFS pass             (with nucdiv)          */
+#define PB_AN_FULI          0x2000u /* Fu & Li's D (outgroup only) and D*              (with sfs)             */
+#define PB_AN_LD_DPRIME     0x4000u /* Lewontin's |D'| over the ZnS pairs              (with ld -o 0)         */
 
 /* Run parameters == the fields of popbamData the hot path reads (popbam.h:218-265) plus
  * the population tables assign_pops builds (popbam.cpp:145-171).                           */
@@ -174,6 +178,23 @@ typedef struct pb_region_result {
     const uint16_t *tree_diff;    /* [NW*(n+1)*(n+1)] treeData::diff_matrix (pop_tree.cpp:472-494), taxon 0 = reference */
 } pb_region_result;
 
+/* Extension statistics of the last region (PB_AN_THETA_W, PB_AN_FULI, PB_AN_LD_DPRIME): a struct of its own, so that
+ * pb_region_result keeps its size for callers built against the reference-only interface.  Same lifetime as the
+ * pb_region_result arrays; an array is NULL unless its bit was requested.  m = pop_nsmpl[p]; xi_j = the window's site
+ * frequency spectrum of population p as calc_sfs bins it (outgroup flip with PB_FLAG_OUTGROUP); S = sum xi_j over
+ * 0<j<m; a = sum_{i<m} 1/i.  All arrays [NW*P].  (With PB_AN_LD_DPRIME pb_region_result.ld_num_snps is set too.)     */
+typedef struct pb_region_extras {
+    const int32_t *pop_segsites;  /* S                                                   (THETA_W or FULI)  */
+    const double  *theta_w;       /* S / a, not yet divided by num_sites; NaN if m < 2   (THETA_W)          */
+    const double  *fuli_d;        /* Fu & Li's D with eta_e; NaN without an outgroup, if m < 3 or S = 0 (FULI) */
+    const double  *fuli_ds;       /* Fu & Li's D* with eta_s; NaN if m < 4 (at m = 3 it is 0/0) or S = 0 (FULI) */
+    const int32_t *fuli_eta_e;    /* xi_1 (0 if m < 2)                                   (FULI)             */
+    const int32_t *fuli_eta_s;    /* xi_1 + xi_{m-1}, counted once when m = 2            (FULI)             */
+    const int32_t *ld_kept;       /* K: SNPs with min_freq <= count <= m - min_freq, the ZnS pairs (LD_DPRIME) */
+    const double  *ld_dprime;     /* mean |D'| over the K(K-1)/2 pairs; NaN if K < 2     (LD_DPRIME)        */
+    const int64_t *ld_complete;   /* pairs with |D'| = 1 (complete LD)                   (LD_DPRIME)        */
+} pb_region_extras;
+
 typedef struct pb_ctx pb_ctx;
 
 /* ---- life cycle ---------------------------------------------------------------------- */
@@ -216,6 +237,8 @@ int pb_push_record(pb_ctx *ctx, const void *core32, const void *data, int32_t l_
 /* replaces: bam_plbuf_push(0, buf) + calc_X (pop_nucdiv.cpp:112-116).  Runs the kernels,
  * copies the window results back and fills *out.                                          */
 int pb_region_end(pb_ctx *ctx, pb_region_result *out);
+/* The extension arrays of the region pb_region_end / pb_region_wait returned last.                                  */
+int pb_region_get_extras(const pb_ctx *ctx, pb_region_extras *out);
 
 /* Asynchronous split of pb_region_end for overlap / device timing: launch enqueues every
  * kernel and the result copies on the context's stream; wait blocks and fills *out.       */
@@ -276,6 +299,11 @@ typedef struct pb_print_opts {
 } pb_print_opts;
 int64_t pb_format_window(const pb_ctx *ctx, const pb_region_result *res, int32_t window,
                          uint32_t analysis, const pb_print_opts *opts, char *buf, int64_t cap);
+/* The same, where `analysis` may also be a reference bit OR-ed with its extension (NUCDIV|THETA_W, SFS|FULI,
+ * LD_ZNS|LD_DPRIME): the extension's columns (theta[pop]; FuLiD*[pop] and, with PB_FLAG_OUTGROUP, FuLiD[pop];
+ * Dp[pop] and Dp1[pop]) then follow the reference's, before the newline.  `ext` may be NULL for reference bits.     */
+int64_t pb_format_window_ext(const pb_ctx *ctx, const pb_region_result *res, const pb_region_extras *ext, int32_t window,
+                             uint32_t analysis, const pb_print_opts *opts, char *buf, int64_t cap);
 
 #ifdef __cplusplus
 }

@@ -10,12 +10,14 @@ PKG = Path(__file__).resolve().parent
 MAXS = 64
 
 AN = dict(NUCDIV=0x001, SFS=0x002, LD_ZNS=0x004, LD_OMEGA=0x008, LD_WALL=0x010, DIVERGE_IND=0x020,
-          DIVERGE_POP=0x040, HAPLO_K=0x080, HAPLO_EHHS=0x100, HAPLO_DXY=0x200, SNP=0x400, TREE=0x800)
+          DIVERGE_POP=0x040, HAPLO_K=0x080, HAPLO_EHHS=0x100, HAPLO_DXY=0x200, SNP=0x400, TREE=0x800,
+          THETA_W=0x1000, FULI=0x2000, LD_DPRIME=0x4000)
 FLAG = dict(ILLUMINA=0x02, SUBSTITUTE=0x10, HETEROZYGOTE=0x20, OUTGROUP=0x40, EMIT_CB=0x10000)
 
 EXPORTS = ["pb_create", "pb_destroy", "pb_last_error", "pb_version", "pb_set_contig", "pb_region_begin", "pb_push_batch", "pb_push_batch_async",
            "pb_push_record", "pb_region_reserve", "pb_region_end", "pb_region_launch", "pb_region_wait", "pb_region_relaunch", "pb_stream",
-           "pb_kernel_launches", "pb_region_path", "pb_region_reruns", "pb_stage_times", "pb_window_grid", "pb_build_errmod_tables", "pb_errmod_tables_cached", "pb_errmod_tables_cached_ex", "pb_host_alloc", "pb_host_free", "pb_format_window"]
+           "pb_kernel_launches", "pb_region_path", "pb_region_reruns", "pb_stage_times", "pb_window_grid", "pb_build_errmod_tables", "pb_errmod_tables_cached", "pb_errmod_tables_cached_ex", "pb_host_alloc", "pb_host_free", "pb_format_window",
+           "pb_region_get_extras", "pb_format_window_ext"]
 
 
 def _p(t):
@@ -60,6 +62,16 @@ class Result(C.Structure):
                 ("cb", _p(C.c_uint64)), ("site_type", _p(C.c_uint64)), ("site_flag", _p(C.c_uint8)),
                 ("reads_pushed", C.c_int64), ("reads_used", C.c_int64), ("aligned_bases", C.c_int64),
                 ("tree_diff", _p(C.c_uint16))]
+
+
+class Extras(C.Structure):
+    """pb_region_extras: the PB_AN_THETA_W / FULI / LD_DPRIME arrays, [NW*P] each."""
+    _fields_ = [("pop_segsites", _p(C.c_int32)), ("theta_w", _p(C.c_double)), ("fuli_d", _p(C.c_double)),
+                ("fuli_ds", _p(C.c_double)), ("fuli_eta_e", _p(C.c_int32)), ("fuli_eta_s", _p(C.c_int32)),
+                ("ld_kept", _p(C.c_int32)), ("ld_dprime", _p(C.c_double)), ("ld_complete", _p(C.c_int64))]
+
+
+EXT_BITS = AN["THETA_W"] | AN["FULI"] | AN["LD_DPRIME"]
 
 
 class PrintOpts(C.Structure):
@@ -125,6 +137,9 @@ def lib():
         L.pb_host_free.argtypes = [C.c_void_p]
         L.pb_format_window.restype = C.c_int64
         L.pb_format_window.argtypes = [C.c_void_p, _p(Result), C.c_int32, C.c_uint32, _p(PrintOpts), C.c_char_p, C.c_int64]
+        L.pb_region_get_extras.argtypes = [C.c_void_p, _p(Extras)]
+        L.pb_format_window_ext.restype = C.c_int64
+        L.pb_format_window_ext.argtypes = [C.c_void_p, _p(Result), _p(Extras), C.c_int32, C.c_uint32, _p(PrintOpts), C.c_char_p, C.c_int64]
         _lib = L
     return _lib
 
@@ -148,6 +163,7 @@ class Context:
             raise PopbamError("pb_create failed (%d): %s" % (st.value, L.pb_last_error(None).decode()))
         self.L, self.params = L, params
         self.res = Result()
+        self.ext = Extras()
 
     def _chk(self, rc):
         if rc != 0:
@@ -181,6 +197,7 @@ class Context:
 
     def region_end(self):
         self._chk(self.L.pb_region_end(self.h, C.byref(self.res)))
+        self._chk(self.L.pb_region_get_extras(self.h, C.byref(self.ext)))
         return self.res
 
     def launch(self):
@@ -191,6 +208,7 @@ class Context:
 
     def wait(self):
         self._chk(self.L.pb_region_wait(self.h, C.byref(self.res)))
+        self._chk(self.L.pb_region_get_extras(self.h, C.byref(self.ext)))
         return self.res
 
     def stage_times(self):
@@ -212,11 +230,11 @@ class Context:
         out = []
         buf = C.create_string_buffer(1 << 20)
         for w in (range(self.res.n_windows) if windows is None else windows):
-            k = self.L.pb_format_window(self.h, C.byref(self.res), w, analysis, C.byref(opts), buf, len(buf))
+            k = self.L.pb_format_window_ext(self.h, C.byref(self.res), C.byref(self.ext), w, analysis, C.byref(opts), buf, len(buf))
             if k < 0:
                 raise PopbamError("pb_format_window failed: %d" % k)
             if k >= len(buf):
                 buf = C.create_string_buffer(int(k) + 16)
-                k = self.L.pb_format_window(self.h, C.byref(self.res), w, analysis, C.byref(opts), buf, len(buf))
+                k = self.L.pb_format_window_ext(self.h, C.byref(self.res), C.byref(self.ext), w, analysis, C.byref(opts), buf, len(buf))
             out.append(buf.raw[:k].decode())
         return "".join(out)

@@ -189,9 +189,20 @@ void nj_newick(Out &out, const uint16_t *diff, int T, int num_sites, const pb_pr
 
 extern "C" int64_t pb_format_window(const pb_ctx *ctx, const pb_region_result *r, int32_t w, uint32_t an, const pb_print_opts *o,
                                     char *buf, int64_t cap) {
+    if (an & (PB_AN_THETA_W | PB_AN_FULI | PB_AN_LD_DPRIME)) return PB_ERR_ARG;
+    return pb_format_window_ext(ctx, r, nullptr, w, an, o, buf, cap);
+}
+
+extern "C" int64_t pb_format_window_ext(const pb_ctx *ctx, const pb_region_result *r, const pb_region_extras *e, int32_t w, uint32_t an,
+                                        const pb_print_opts *o, char *buf, int64_t cap) {
     const pb_params *p = pb_ctx_params(ctx);
     if (!p || !r || !o || w < 0 || w >= r->n_windows) return PB_ERR_ARG;
-    if (!(r->analyses & an)) return PB_ERR_ARG;
+    if ((r->analyses & an) != an) return PB_ERR_ARG;
+    // one reference bit, optionally with its extension, whose columns follow the reference's
+    const uint32_t ext = an & (PB_AN_THETA_W | PB_AN_FULI | PB_AN_LD_DPRIME);
+    an &= ~ext;
+    if (ext && (!e || ext != (an == PB_AN_NUCDIV ? PB_AN_THETA_W : an == PB_AN_SFS ? PB_AN_FULI : an == PB_AN_LD_ZNS ? PB_AN_LD_DPRIME : 0u)))
+        return PB_ERR_ARG;
     Out out;
     const int P = r->n_pops, n = r->n_samples;
     const int ns = r->num_sites[w];
@@ -315,6 +326,19 @@ extern "C" int64_t pb_format_window(const pb_ctx *ctx, const pb_region_result *r
                 }
             break;
         default: return PB_ERR_ARG;
+        }
+        for (int i = 0; ext && i < P; ++i) {
+            const size_t x = wp + i;
+            if (ext == PB_AN_THETA_W) out.stat("theta", o->pop_names[i], ok && !std::isnan(e->theta_w[x]), e->theta_w[x] / ns);
+            else if (ext == PB_AN_FULI) {
+                out.stat("FuLiD*", o->pop_names[i], !std::isnan(e->fuli_ds[x]), e->fuli_ds[x]);
+                if (p->flags & PB_FLAG_OUTGROUP) out.stat("FuLiD", o->pop_names[i], !std::isnan(e->fuli_d[x]), e->fuli_d[x]);
+            } else {
+                const bool good = r->ld_num_snps[x] >= o->min_snps && e->ld_kept[x] >= 2;
+                out.stat("Dp", o->pop_names[i], good, e->ld_dprime[x]);
+                if (good) out.f("\tDp1[%s]:\t%lld", o->pop_names[i], (long long)e->ld_complete[x]);
+                else out.f("\tDp1[%s]:\t%7s", o->pop_names[i], "NA");
+            }
         }
         out.f("\n");
         }

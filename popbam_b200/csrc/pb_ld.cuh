@@ -16,6 +16,11 @@
 //                shared memory; Lsum_i = sum_{k<i} r^2, Rsum_i = sum_{k>i} r^2 (ZnS only needs Rsum)
 //   k_ld_finish  grid (pop x window): ZnS = 2/(S'(S'-1)) * sum Rsum; omega_max by the running-sum scan
 //                of SURVEY Q11 expressed through Lsum/Rsum (no S x S matrix, no O(S^3) loop)
+// Extension (no reference counterpart, PB_AN_LD_DPRIME): Lewontin's |D'| = |num| / Dmax over the same kept pairs, with
+// num = n n11 - m_j m_k and Dmax = min(m_j (n-m_k), (n-m_j) m_k) if num > 0, else min(m_j m_k, (n-m_j)(n-m_k)): an integer in
+// [1, n^2/4] = [1, 1024], so the division is a multiply by a shared-memory table of 1/k.  k_ld_rows<true> adds the sum of
+// |D'| and the number of pairs with |num| = Dmax (complete LD) over k > i to every row; k_ld_rows<false> (ZnS / omega only)
+// is the kernel without them.
 // The summation ORDER differs from the reference's (parallel partial sums; r^2 through reciprocals):
 // relative differences ~1e-15, inside the 1e-9 tolerance of the parity contract.
 #pragma once
@@ -41,9 +46,12 @@ struct PbLdArgs {
     double *lsum, *rsum;
     int32_t *kcount;          // [NW][P] kept SNPs
     int32_t *nsnps;           // [NW][P] S' of the reference's counting rule
+    double *dpsum;            // per row: sum of |D'| over k > i       (PB_AN_LD_DPRIME)
+    int32_t *dpfull;          // per row: pairs k > i in complete LD   (PB_AN_LD_DPRIME)
     // outputs
     int32_t *ld_num_snps;
     double *zns, *omegamax;
+    int32_t *ld_kept; double *ld_dprime; int64_t *ld_complete;
 };
 
 __global__ void __launch_bounds__(PB_LD_THREADS) k_ld_keep(const PbLdArgs a) {
@@ -83,6 +91,7 @@ __global__ void __launch_bounds__(PB_LD_THREADS) k_ld_keep(const PbLdArgs a) {
 // XU pipe, which the two POPCs of every pair already keep busy (profiles/r1_ld_rows_raw.txt)
 __device__ __forceinline__ double pb_u2d(unsigned n) { return __hiloint2double(0x43300000, (int)n) - 4503599627370496.0; }
 
+template <bool DPRIME>
 __global__ void __launch_bounds__(PB_LD_THREADS) k_ld_rows(const PbLdArgs a, int need_left, int n_row_blocks) {
     __shared__ uint64_t st[PB_LD_THREADS];
     __shared__ double sinv[PB_LD_THREADS];
@@ -99,6 +108,21 @@ __global__ void __launch_bounds__(PB_LD_THREADS) k_ld_rows(const PbLdArgs a, int
     const uint64_t ti = live ? a.kt[base + i] : 0;
     const int mi = live ? a.km[base + i] : 0;
     double l = 0.0, r = 0.0;
+    double dps = 0.0;      // DPRIME: sum of |D'| over the partners k > i
+    int dpf = 0;           //         partners k > i in complete LD
+    double *dinv = nullptr;
+    if constexpr (DPRIME) {
+        __shared__ double dtab[1025];      // 1/k, k = Dmax <= np^2/4 <= 1024
+        for (int k = tid; k <= (np * np) / 4; k += PB_LD_THREADS) dtab[k] = k ? 1.0 / (double)k : 0.0;
+        dinv = dtab;       // (visible after the first tile's barrier)
+    }
+    // |D'| of the pair (i, k) from its numerator and the partner's marginal count
+    auto dprime = [&](int num, int mk) {
+        const int dmax = num > 0 ? min(mi * (np - mk), (np - mi) * mk) : min(mi * mk, (np - mi) * (np - mk));
+        const int an = abs(num);
+        dps = fma(pb_u2d((unsigned)an), dinv[dmax], dps);
+        dpf += an == dmax;
+    };
     // partner tiles: all of them for omega (left and right sums), only those at or right of the diagonal for ZnS
     for (int k0 = need_left ? 0 : i0; k0 < K; k0 += PB_LD_THREADS) {
         __syncthreads();
@@ -116,12 +140,17 @@ __global__ void __launch_bounds__(PB_LD_THREADS) k_ld_rows(const PbLdArgs a, int
             for (int k = 0; k < kn; ++k) {
                 const int num = np * __popcll(ti & st[k]) - mi * sm[k];
                 r = fma(pb_u2d((unsigned)(num * num)), sinv[k], r);
+                if constexpr (DPRIME) dprime(num, sm[k]);
             }
         } else {                                   // the diagonal tile
             for (int k = 0; k < kn; ++k) {
                 const int num = np * __popcll(ti & st[k]) - mi * sm[k];
                 const double v = pb_u2d((unsigned)(num * num)) * sinv[k];
-                if (k0 + k < i) l += v; else if (k0 + k > i) r += v;
+                if (k0 + k < i) l += v;
+                else if (k0 + k > i) {
+                    r += v;
+                    if constexpr (DPRIME) dprime(num, sm[k]);
+                }
             }
         }
     }
@@ -129,6 +158,7 @@ __global__ void __launch_bounds__(PB_LD_THREADS) k_ld_rows(const PbLdArgs a, int
         const double inv_i = a.kinv[base + i];
         a.rsum[base + i] = r * inv_i;
         if (need_left) a.lsum[base + i] = l * inv_i;
+        if constexpr (DPRIME) { a.dpsum[base + i] = dps; a.dpfull[base + i] = dpf; }
     }
 }
 
@@ -142,6 +172,23 @@ __global__ void __launch_bounds__(PB_LD_THREADS) k_ld_finish(const PbLdArgs a) {
     for (int i = tid; i < K; i += PB_LD_THREADS) part += a.rsum[base + i];
     for (int o = 16; o > 0; o >>= 1) part += __shfl_xor_sync(0xffffffffu, part, o);
     if ((tid & 31) == 0) sh[tid >> 5] = part;
+    if (a.analyses & 0x4000u) {                    // PB_AN_LD_DPRIME: mean |D'| and complete pairs over the K(K-1)/2 pairs
+        __shared__ double shd[PB_LD_THREADS / 32];
+        __shared__ long long shf[PB_LD_THREADS / 32];
+        double dp = 0.0;
+        long long full = 0;
+        for (int i = tid; i < K; i += PB_LD_THREADS) { dp += a.dpsum[base + i]; full += a.dpfull[base + i]; }
+        for (int o = 16; o > 0; o >>= 1) { dp += __shfl_xor_sync(0xffffffffu, dp, o); full += __shfl_xor_sync(0xffffffffu, full, o); }
+        if ((tid & 31) == 0) { shd[tid >> 5] = dp; shf[tid >> 5] = full; }
+        __syncthreads();
+        if (tid == 0) {
+            dp = 0.0; full = 0;
+            for (int i = 0; i < PB_LD_THREADS / 32; ++i) { dp += shd[i]; full += shf[i]; }
+            a.ld_kept[oi] = K;
+            a.ld_dprime[oi] = K < 2 ? nan("") : dp / ((double)K * (double)(K - 1) / 2.0);
+            a.ld_complete[oi] = full;
+        }
+    }
     __syncthreads();
     if (tid != 0) return;
     double total = 0.0;

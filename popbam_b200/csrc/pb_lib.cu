@@ -91,7 +91,7 @@ struct pb_ctx {
     bool no_async = false;                 // POPBAM_B200_SYNC=1: always take the host round trips (A/B measurements)
     int64_t seg_cap = 0;                   // device layout of the segregating-site arrays (async: sized by the span)
     DevBuf d_seg_type;     // arena of the segregating-site arrays (seg_layout)
-    DevBuf d_hap, d_kt, d_km, d_lsum, d_rsum, d_wall_u, d_stats, d_ld_kt, d_ld_km, d_ld_inv, d_ld_cnt;
+    DevBuf d_hap, d_kt, d_km, d_lsum, d_rsum, d_wall_u, d_stats, d_ld_kt, d_ld_km, d_ld_inv, d_ld_cnt, d_ld_dp;
     // pinned results
     HostBuf h_ctr, h_small, h_seg, h_span;
     PbCounters ctr_host;
@@ -100,6 +100,7 @@ struct pb_ctx {
     unsigned char need_qval[64] = {0};
     int64_t s_total = 0;
     pb_region_result res;
+    pb_region_extras ext;
     // bam_fetch_f shim staging (pb_push_record)
     std::vector<int32_t> r_pos;
     std::vector<uint32_t> r_meta, r_cig_off, r_cigar, r_base_off;
@@ -193,6 +194,8 @@ struct SmallLayout {
     uint16_t *ind_div, *pop_div; int32_t *div_num_snps;
     int32_t *nhaps; double *hdiv, *ehhs;
     uint16_t *tree_diff;
+    int32_t *pop_segsites; double *theta_w, *fuli_d, *fuli_ds; int32_t *fuli_eta_e, *fuli_eta_s;
+    int32_t *ld_kept; double *ld_dprime; int64_t *ld_complete;
     size_t bytes;
 };
 SmallLayout small_layout(void *base, int NW, int P, int n, bool with_tree) {
@@ -207,6 +210,9 @@ SmallLayout small_layout(void *base, int NW, int P, int n, bool with_tree) {
     L.ind_div = cv.take<uint16_t>(wn); L.pop_div = cv.take<uint16_t>(wp); L.div_num_snps = cv.take<int32_t>(wp);
     L.nhaps = cv.take<int32_t>(wp); L.hdiv = cv.take<double>(wp); L.ehhs = cv.take<double>(wp);
     L.tree_diff = cv.take<uint16_t>(with_tree ? (size_t)NW * (n + 1) * (n + 1) : 1);
+    L.pop_segsites = cv.take<int32_t>(wp); L.theta_w = cv.take<double>(wp); L.fuli_d = cv.take<double>(wp); L.fuli_ds = cv.take<double>(wp);
+    L.fuli_eta_e = cv.take<int32_t>(wp); L.fuli_eta_s = cv.take<int32_t>(wp);
+    L.ld_kept = cv.take<int32_t>(wp); L.ld_dprime = cv.take<double>(wp); L.ld_complete = cv.take<int64_t>(wp);
     L.bytes = (cv.off + 255) & ~(size_t)255;
     return L;
 }
@@ -359,7 +365,7 @@ int run_pipeline(pb_ctx *c, int attempt = 0, bool allow_async = true) {
     // BESIDE k_pile_reads instead of in front of it, and fill_result compares what it found with what was assumed (and looks
     // at the sorted / too-long flags) once the region is done.  No host round trip in the middle of the pipeline, so one
     // context keeps a GPU busy.
-    const uint32_t sync_bits = PB_AN_SNP | PB_AN_LD_ZNS | PB_AN_LD_OMEGA;          // their buffers / grids are sized by the number of segregating sites
+    const uint32_t sync_bits = PB_AN_SNP | PB_AN_LD_ZNS | PB_AN_LD_OMEGA | PB_AN_LD_DPRIME;          // their buffers / grids are sized by the number of segregating sites
     const bool async = allow_async && !c->no_async && fast_try && c->spec_valid && attempt == 0 && !(c->analyses & sync_bits) && !(P.flags & PB_FLAG_EMIT_CB);
     c->async_run = async;
     if (!async) PB_CUDA(c, cudaStreamWaitEvent(st, c->fk[2], 0));    // join
@@ -598,7 +604,8 @@ int run_pipeline(pb_ctx *c, int attempt = 0, bool allow_async = true) {
 
     // ---- window statistics
     const uint32_t stat_bits = PB_AN_NUCDIV | PB_AN_SFS | PB_AN_LD_WALL | PB_AN_DIVERGE_IND |
-                               PB_AN_DIVERGE_POP | PB_AN_HAPLO_K | PB_AN_HAPLO_EHHS | PB_AN_HAPLO_DXY | PB_AN_TREE;
+                               PB_AN_DIVERGE_POP | PB_AN_HAPLO_K | PB_AN_HAPLO_EHHS | PB_AN_HAPLO_DXY | PB_AN_TREE |
+                               PB_AN_THETA_W | PB_AN_FULI;
     if (c->analyses & stat_bits) {
         PbStatArgs sa;
         memset(&sa, 0, sizeof sa);
@@ -625,12 +632,14 @@ int run_pipeline(pb_ctx *c, int attempt = 0, bool allow_async = true) {
         sa.wall_num_snps = dl.wall_num_snps; sa.wallb = dl.wallb; sa.wallq = dl.wallq;
         sa.ind_div = dl.ind_div; sa.pop_div = dl.pop_div; sa.div_num_snps = dl.div_num_snps; sa.tree_diff = dl.tree_diff;
         sa.nhaps = dl.nhaps; sa.hdiv = dl.hdiv; sa.ehhs = dl.ehhs;
+        sa.pop_segsites = dl.pop_segsites; sa.theta_w = dl.theta_w; sa.fuli_d = dl.fuli_d; sa.fuli_ds = dl.fuli_ds;
+        sa.fuli_eta_e = dl.fuli_eta_e; sa.fuli_eta_s = dl.fuli_eta_s;
         k_window_stats<<<NW, PB_ST_THREADS, (size_t)n * n * sizeof(uint16_t), st>>>(sa);
         c->launches += 1;
         PB_CUDA(c, cudaGetLastError());
     }
-    // ---- pairwise LD (ld -o 0 / -o 1): keep list, tiled pair kernel, finish
-    if (c->analyses & (PB_AN_LD_ZNS | PB_AN_LD_OMEGA)) {
+    // ---- pairwise LD (ld -o 0 / -o 1, D'): keep list, tiled pair kernel, finish
+    if (c->analyses & (PB_AN_LD_ZNS | PB_AN_LD_OMEGA | PB_AN_LD_DPRIME)) {
         PbLdArgs la;
         memset(&la, 0, sizeof la);
         la.P = P.n_pops;
@@ -649,10 +658,16 @@ int run_pipeline(pb_ctx *c, int attempt = 0, bool allow_async = true) {
         la.lsum = dp<double>(c->d_lsum); la.rsum = dp<double>(c->d_rsum);
         la.kcount = dp<int32_t>(c->d_ld_cnt); la.nsnps = la.kcount + (size_t)NW * P.n_pops;
         la.ld_num_snps = dl.ld_num_snps; la.zns = dl.zns; la.omegamax = dl.omegamax;
+        la.ld_kept = dl.ld_kept; la.ld_dprime = dl.ld_dprime; la.ld_complete = dl.ld_complete;
+        const bool dprime = (c->analyses & PB_AN_LD_DPRIME) != 0;
+        if (dprime) {      // per-row |D'| sums (double) and complete-pair counts (int32)
+            PB_TRY(dev_reserve(c, c->d_ld_dp, (sizeof(double) + sizeof(int32_t)) * cnt));
+            la.dpsum = dp<double>(c->d_ld_dp); la.dpfull = reinterpret_cast<int32_t *>(la.dpsum + cnt);
+        }
         const unsigned pw = (unsigned)NW * (unsigned)P.n_pops;
         const int nrb = std::max(1, (s_max + PB_LD_THREADS - 1) / PB_LD_THREADS);
         k_ld_keep<<<pw, PB_LD_THREADS, 0, st>>>(la);
-        k_ld_rows<<<pw * (unsigned)nrb, PB_LD_THREADS, 0, st>>>(la, (c->analyses & PB_AN_LD_OMEGA) ? 1 : 0, nrb);
+        (dprime ? k_ld_rows<true> : k_ld_rows<false>)<<<pw * (unsigned)nrb, PB_LD_THREADS, 0, st>>>(la, (c->analyses & PB_AN_LD_OMEGA) ? 1 : 0, nrb);
         k_ld_finish<<<pw, PB_LD_THREADS, 0, st>>>(la);
         c->launches += 3;
         PB_CUDA(c, cudaGetLastError());
@@ -737,6 +752,12 @@ int fill_result(pb_ctx *c, pb_region_result *out) {
     if (an & PB_AN_LD_WALL) { r.wall_num_snps = hl.wall_num_snps; r.wallb = hl.wallb; r.wallq = hl.wallq; }
     if (an & PB_AN_DIVERGE_IND) r.ind_div = hl.ind_div;
     if (an & PB_AN_TREE) r.tree_diff = hl.tree_diff;
+    pb_region_extras &e = c->ext;
+    memset(&e, 0, sizeof e);
+    if (an & (PB_AN_THETA_W | PB_AN_FULI)) e.pop_segsites = hl.pop_segsites;
+    if (an & PB_AN_THETA_W) e.theta_w = hl.theta_w;
+    if (an & PB_AN_FULI) { e.fuli_d = hl.fuli_d; e.fuli_ds = hl.fuli_ds; e.fuli_eta_e = hl.fuli_eta_e; e.fuli_eta_s = hl.fuli_eta_s; }
+    if (an & PB_AN_LD_DPRIME) { r.ld_num_snps = hl.ld_num_snps; e.ld_kept = hl.ld_kept; e.ld_dprime = hl.ld_dprime; e.ld_complete = hl.ld_complete; }
     if (an & PB_AN_DIVERGE_POP) { r.pop_div = hl.pop_div; r.div_num_snps = hl.div_num_snps; }
     if (an & (PB_AN_HAPLO_K | PB_AN_HAPLO_EHHS)) { r.nhaps = hl.nhaps; r.hdiv = hl.hdiv; }
     if (an & PB_AN_HAPLO_EHHS) r.ehhs = hl.ehhs;
@@ -1058,6 +1079,12 @@ int pb_region_wait(pb_ctx *c, pb_region_result *out) {
 int pb_region_end(pb_ctx *c, pb_region_result *out) {
     PB_TRY(pb_region_launch(c));
     return pb_region_wait(c, out);
+}
+
+int pb_region_get_extras(const pb_ctx *c, pb_region_extras *out) {
+    if (!c || !out) return PB_ERR_ARG;
+    *out = c->ext;
+    return PB_OK;
 }
 
 void *pb_host_alloc(size_t bytes) {

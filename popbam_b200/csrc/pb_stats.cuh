@@ -8,6 +8,8 @@
 //   calc_wall                      pop_ld.cpp:375-458
 //   calc_diverge                   pop_diverge.cpp:220-257
 //   calc_nhaps / calc_ehhs         pop_haplo.cpp:208-254, :256-323
+//   extensions (no reference counterpart): Watterson's theta and Fu & Li's D / D* on calc_sfs's spectrum,
+//   the closed forms of tests/ext_oracle.c in the same operation order
 //
 // Integer results are exact.  Floating-point statistics use the reference's formulas term by term
 // (the library is compiled with -fmad=false so products and sums round separately, as on x86-64);
@@ -42,6 +44,7 @@ struct PbStatArgs {
     uint16_t *ind_div, *pop_div; int32_t *div_num_snps;
     int32_t *nhaps; double *hdiv, *ehhs;
     uint16_t *tree_diff;  // [NW][(n+1)*(n+1)]
+    int32_t *pop_segsites; double *theta_w, *fuli_d, *fuli_ds; int32_t *fuli_eta_e, *fuli_eta_s;
 };
 
 // analysis bits (include/popbam_b200.h)
@@ -56,6 +59,8 @@ struct PbStatArgs {
 #define PBA_HAPLO_K 0x080u
 #define PBA_HAPLO_EHHS 0x100u
 #define PBA_HAPLO_DXY 0x200u
+#define PBA_THETA_W 0x1000u
+#define PBA_FULI 0x2000u
 #define PBA_FLAG_OUTGROUP 0x40u
 
 __device__ __forceinline__ int pb_block_sum_int(int v, int *sh /* [32] */) {
@@ -105,6 +110,32 @@ __device__ int pb_compact_sites(const uint64_t *__restrict__ T, int S, uint64_t 
     __syncthreads();
     *n_before = before;
     return carry;
+}
+
+// Watterson's theta and Fu & Li's D / D* of one (window, population) from the spectrum's S, xi_1 and xi_{np-1}
+__device__ __forceinline__ void pb_sfs_ext(int np, int seg, int xi1, int xin1, bool outg, int32_t *segs, double *theta_w, double *fuli_d,
+                                        double *fuli_ds, int32_t *eta_e, int32_t *eta_s) {
+    const int ee = np >= 2 ? xi1 : 0, es = np >= 3 ? xi1 + xin1 : ee;
+    double thw = nan(""), fd = nan(""), fds = nan("");
+    if (np >= 2) {
+        double a1 = 0.0, a2 = 0.0;
+        for (int j = 1; j < np; ++j) a1 += 1.0 / (double)j;
+        for (int j = 1; j < np; ++j) a2 += 1.0 / ((double)j * (double)j);
+        thw = (double)seg / a1;
+        if (np >= 3 && seg > 0) {
+            const double nn = (double)np, Sd = (double)seg, ap = a1 + 1.0 / nn, r = nn / (nn - 1.0);
+            const double c = 2.0 * (nn * a1 - 2.0 * (nn - 1.0)) / ((nn - 1.0) * (nn - 2.0));
+            const double vd = 1.0 + a1 * a1 / (a2 + a1 * a1) * (c - (nn + 1.0) / (nn - 1.0)), ud = a1 - 1.0 - vd;
+            const double d = c + (nn - 2.0) / ((nn - 1.0) * (nn - 1.0)) + 2.0 / (nn - 1.0) * (1.5 - (2.0 * ap - 3.0) / (nn - 2.0) - 1.0 / nn);
+            const double vds = (r * r * a2 + a1 * a1 * d - 2.0 * nn * a1 * (a1 + 1.0) / ((nn - 1.0) * (nn - 1.0))) / (a1 * a1 + a2);
+            const double uds = r * (a1 - r) - vds;
+            if (outg) fd = (Sd - a1 * (double)ee) / sqrt(ud * Sd + vd * Sd * Sd);
+            if (np >= 4) fds = (r * Sd - a1 * (double)es) / sqrt(uds * Sd + vds * Sd * Sd);      // n = 3: eta_s = S, 0 / 0
+        }
+    }
+    *segs = seg;
+    if (theta_w) *theta_w = thw;
+    if (fuli_d) { *fuli_d = fd; *fuli_ds = fds; *eta_e = ee; *eta_s = es; }
 }
 
 __global__ void __launch_bounds__(PB_ST_THREADS) k_window_stats(const PbStatArgs a) {
@@ -226,7 +257,7 @@ __global__ void __launch_bounds__(PB_ST_THREADS) k_window_stats(const PbStatArgs
         const int np = a.pop_nsmpl[pi];
         const size_t oi = (size_t)w * P + pi;
 
-        if (an & (PBA_SFS | PBA_DIVERGE_POP)) {
+        if (an & (PBA_SFS | PBA_DIVERGE_POP | PBA_THETA_W | PBA_FULI)) {
             __syncthreads();
             for (int i = tid; i < 66; i += PB_ST_THREADS) sfs_s[i] = 0;
             __syncthreads();
@@ -268,6 +299,11 @@ __global__ void __launch_bounds__(PB_ST_THREADS) k_window_stats(const PbStatArgs
                                      (9.0 * m * ((m - 1) * (m - 1)))));
                     } else { td = nan(""); fwh = nan(""); }
                     a.td[oi] = td; a.fwh[oi] = fwh;
+                }
+                if (an & (PBA_THETA_W | PBA_FULI)) {
+                    const bool fl = (an & PBA_FULI) != 0;
+                    pb_sfs_ext(np, seg, sfs_s[1], sfs_s[np > 0 ? np - 1 : 0], outg, a.pop_segsites + oi, (an & PBA_THETA_W) ? a.theta_w + oi : nullptr,
+                               fl ? a.fuli_d + oi : nullptr, fl ? a.fuli_ds + oi : nullptr, fl ? a.fuli_eta_e + oi : nullptr, fl ? a.fuli_eta_s + oi : nullptr);
                 }
             }
         }

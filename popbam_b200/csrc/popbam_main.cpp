@@ -11,7 +11,9 @@
 // Shards are independent (every window starts from an empty pileup, SURVEY.md §8(e)), so the GPUs of
 // a box each take every G-th shard and no data crosses between them.
 //
-// Extra options (not in the reference): --gpus N, --shard-mb X, --threads T.
+// Extra options (not in the reference): --gpus N, --shard-mb X, --threads T, and --extra-stats: statistics the
+// reference does not compute, as extra columns after its own (nucdiv: Watterson's theta; sfs: Fu & Li's D* and, with
+// -p, D; ld -o 0: mean |D'| and the number of SNP pairs in complete LD).
 #include <algorithm>
 #include <atomic>
 #include <condition_variable>
@@ -45,6 +47,7 @@ struct Options {
     bool window = false, illumina = false, het = false, min_freq2 = false, substitute = false, has_p = false, has_h = false;
     std::vector<std::string> positional;
     int gpus = 1, threads = 0;
+    bool extra_stats = false;
     double shard_mb = 2.0;
 };
 
@@ -65,7 +68,8 @@ void usage(const char *cmd) {
             "Usage:   popbam %s [options] <in.bam> [region]\n"
             "Options: -f FILE reference fastA   -w INT window (kb)   -m/-x INT min/max depth   -q INT min rms mapQ\n"
             "         -s INT min snpQ   -a/-b INT min mapQ / baseQ   -k INT min sites   -o INT output mode   -p STR outgroup\n"
-            "         -i Illumina 1.3+ qualities   --gpus N   --shard-mb X   --threads T\n", cmd);
+            "         -i Illumina 1.3+ qualities   --gpus N   --shard-mb X   --threads T\n"
+            "         --extra-stats  nucdiv: theta[pop]; sfs: FuLiD*[pop] (and FuLiD[pop] with -p); ld -o 0: Dp[pop], Dp1[pop]\n", cmd);
 }
 
 Options parse(int argc, char **argv) {
@@ -78,6 +82,7 @@ Options parse(int argc, char **argv) {
         const std::string a = argv[i];
         if (a.rfind("--", 0) == 0) {
             auto val = [&]() -> const char * { if (i + 1 >= argc) fatal("missing value for " + a); return argv[++i]; };
+            if (a == "--extra-stats") { o.extra_stats = true; continue; }
             if (a == "--gpus") o.gpus = atoi(val());
             else if (a == "--shard-mb") o.shard_mb = atof(val());
             else if (a == "--threads") o.threads = atoi(val());
@@ -135,6 +140,8 @@ Options parse(int argc, char **argv) {
         }
         o.positional.push_back(a);
     }
+    if (o.extra_stats && !(o.cmd == "nucdiv" || o.cmd == "sfs" || (o.cmd == "ld" && o.output == 0)))
+        fatal("--extra-stats is only available for nucdiv, sfs and ld -o 0");
     return o;
 }
 
@@ -288,6 +295,7 @@ void gpu_worker(Run *R, int g, int G, int device) {
         }
         if (err.empty() && sh.error.empty()) {
             pb_region_result res;
+            pb_region_extras ext;
             int rc = pb_region_begin(ctx, R->analysis, sh.w1 - sh.w0, &R->wb[sh.w0], &R->we[sh.w0]);
             {
                 int64_t nr = 0, nc = 0, nb = 0;
@@ -306,11 +314,12 @@ void gpu_worker(Run *R, int g, int G, int device) {
                 rc = R->pinned ? pb_push_batch_async(ctx, &rb) : pb_push_batch(ctx, &rb);
             }
             if (rc == PB_OK) rc = pb_region_end(ctx, &res);
+            if (rc == PB_OK) rc = pb_region_get_extras(ctx, &ext);
             if (rc != PB_OK) sh.error = pb_last_error(ctx);
             else
                 for (int w = 0; w < res.n_windows; ++w) {
-                    int64_t k = pb_format_window(ctx, &res, w, R->analysis, &po, line.data(), (int64_t)line.size());
-                    if (k >= (int64_t)line.size()) { line.resize((size_t)k + 16); k = pb_format_window(ctx, &res, w, R->analysis, &po, line.data(), (int64_t)line.size()); }
+                    int64_t k = pb_format_window_ext(ctx, &res, &ext, w, R->analysis, &po, line.data(), (int64_t)line.size());
+                    if (k >= (int64_t)line.size()) { line.resize((size_t)k + 16); k = pb_format_window_ext(ctx, &res, &ext, w, R->analysis, &po, line.data(), (int64_t)line.size()); }
                     if (k < 0) { sh.error = "formatting failed"; break; }
                     sh.text.append(line.data(), (size_t)k);
                 }
@@ -472,6 +481,7 @@ int main(int argc, char **argv) {
     else if (o.cmd == "tree") R.analysis = PB_AN_TREE;
     else R.analysis = PB_AN_SNP;
     if (o.output < 0 || o.output > 2) fatal("invalid output option");
+    if (o.extra_stats) R.analysis |= o.cmd == "nucdiv" ? PB_AN_THETA_W : o.cmd == "sfs" ? PB_AN_FULI : PB_AN_LD_DPRIME;
 
     // window grid of the region, then shards = runs of whole windows
     const int64_t nw = pb_window_grid(R.beg, R.end, o.window ? o.win_size : 0, 0, nullptr, nullptr);
