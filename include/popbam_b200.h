@@ -65,6 +65,7 @@ typedef enum pb_status {
 #define PB_AN_THETA_W       0x1000u /* Watterson's theta from the SFS pass             (with nucdiv)          */
 #define PB_AN_FULI          0x2000u /* Fu & Li's D (outgroup only) and D*              (with sfs)             */
 #define PB_AN_LD_DPRIME     0x4000u /* Lewontin's |D'| over the ZnS pairs              (with ld -o 0)         */
+#define PB_AN_FST           0x8000u /* F_ST (Hudson, Weir & Cockerham) and Snn per population pair (with nucdiv) */
 
 /* Run parameters == the fields of popbamData the hot path reads (popbam.h:218-265) plus
  * the population tables assign_pops builds (popbam.cpp:145-171).                           */
@@ -195,6 +196,31 @@ typedef struct pb_region_extras {
     const int64_t *ld_complete;   /* pairs with |D'| = 1 (complete LD)                   (LD_DPRIME)        */
 } pb_region_extras;
 
+/* Differentiation between the populations of every pair i < j of the last region (PB_AN_FST): a struct of its own,
+ * like pb_region_extras.  Same lifetime as the pb_region_result arrays; NULL unless PB_AN_FST was requested (snn_p and
+ * snn_ge: unless pb_set_snn_perms asked for permutations too).  All arrays [NW*P*P], index i*P+(j-(i+1)) like pib.
+ * n1, n2 = pop_nsmpl[i], pop_nsmpl[j]; for every segregating site of the window, c1 and c2 = the samples of i and j that
+ * carry the derived allele.  Calls count as haploid, one per sample, as for pi and dxy (with PB_FLAG_HETEROZYGOTE a
+ * heterozygous call counts as derived).  No outgroup flip: every statistic is the same with the allele labels of a site
+ * swapped.  The sums are exact integers:
+ *   hud_den = sum (n1-1)(n2-1) [c1 (n2-c2) + c2 (n1-c1)]           (= dxy sum * (n1-1)(n2-1))
+ *   hud_num = hud_den - sum [c1 (n1-c1) n2 (n2-1) + c2 (n2-c2) n1 (n1-1)]
+ *   wc_num  = sum (c1 n2 - c2 n1)^2 (n1+n2-2) - G (n1+n2),           G = c1 (n1-c1) n2 + c2 (n2-c2) n1
+ *   wc_den  = sum (c1 n2 - c2 n1)^2 (n1+n2-2) + G (2 n1 n2 - n1 - n2)
+ * i.e. Hudson's F_ST as a ratio of averages (Hudson, Slatkin & Maddison 1992; Bhatia et al. 2013) scaled by
+ * n1 n2 (n1-1)(n2-1), and Weir & Cockerham's theta for haploid data (Weir 1996, r = 2) scaled by n1 n2 (n1+n2)(n1+n2-2).
+ * Snn is Hudson's (2000) nearest-neighbour statistic on the window's pairwise difference matrix (the one nucdiv uses).
+ * Every double is NaN if n1 < 2 or n2 < 2; fst_hudson / fst_wc also if their denominator is 0.                        */
+typedef struct pb_region_fst {
+    const int64_t *hud_num, *hud_den;   /* Hudson's numerator and denominator sums                              */
+    const int64_t *wc_num, *wc_den;     /* Weir & Cockerham's                                                  */
+    const double  *fst_hudson;          /* hud_num / hud_den                                                   */
+    const double  *fst_wc;              /* wc_num / wc_den (1 for a window of fixed differences only)          */
+    const double  *snn;                 /* Snn = (1/(n1+n2)) sum_x |NN(x) in pop(x)| / |NN(x)|                  */
+    const double  *snn_p;               /* (1 + snn_ge) / (1 + n_perms)                          (permutations) */
+    const int64_t *snn_ge;              /* permutations of the pooled labels with Snn >= Snn_obs - 1e-12       */
+} pb_region_fst;
+
 typedef struct pb_ctx pb_ctx;
 
 /* ---- life cycle ---------------------------------------------------------------------- */
@@ -239,6 +265,13 @@ int pb_push_record(pb_ctx *ctx, const void *core32, const void *data, int32_t l_
 int pb_region_end(pb_ctx *ctx, pb_region_result *out);
 /* The extension arrays of the region pb_region_end / pb_region_wait returned last.                                  */
 int pb_region_get_extras(const pb_ctx *ctx, pb_region_extras *out);
+/* The PB_AN_FST arrays of the region pb_region_end / pb_region_wait returned last.                                  */
+int pb_region_get_fst(const pb_ctx *ctx, pb_region_fst *out);
+/* Permutation test of Snn for the regions that follow (PB_AN_FST): n_perms random re-partitions of each pair's pooled
+ * samples (default 0: none), drawn from a counter-based stream keyed on (seed, contig tid, window begin, i, j,
+ * permutation), so the result does not depend on how a contig is cut into regions or spread over GPUs.  The generator is
+ * written down in popbam_b200/csrc/pb_stats.cuh (k_snn_perm).  PB_ERR_ARG if n_perms < 0 or > 2^31 - 1.                */
+int pb_set_snn_perms(pb_ctx *ctx, int64_t n_perms, uint64_t seed);
 
 /* Asynchronous split of pb_region_end for overlap / device timing: launch enqueues every
  * kernel and the result copies on the context's stream; wait blocks and fills *out.       */
@@ -304,6 +337,12 @@ int64_t pb_format_window(const pb_ctx *ctx, const pb_region_result *res, int32_t
  * Dp[pop] and Dp1[pop]) then follow the reference's, before the newline.  `ext` may be NULL for reference bits.     */
 int64_t pb_format_window_ext(const pb_ctx *ctx, const pb_region_result *res, const pb_region_extras *ext, int32_t window,
                              uint32_t analysis, const pb_print_opts *opts, char *buf, int64_t cap);
+/* nucdiv with F_ST: `analysis` is PB_AN_NUCDIV, optionally OR-ed with PB_AN_THETA_W and / or PB_AN_FST.  After the
+ * reference's columns and theta[pop] come, per population pair in dxy order, Fst[A-B] (Hudson), FstWC[A-B] and Snn[A-B],
+ * plus SnnP[A-B] when permutations ran; NA where the window has fewer than min_sites sites or the value is NaN.
+ * `ext` may be NULL without PB_AN_THETA_W, `fst` without PB_AN_FST.                                                   */
+int64_t pb_format_window_fst(const pb_ctx *ctx, const pb_region_result *res, const pb_region_extras *ext, const pb_region_fst *fst,
+                             int32_t window, uint32_t analysis, const pb_print_opts *opts, char *buf, int64_t cap);
 
 #ifdef __cplusplus
 }

@@ -11,13 +11,13 @@ MAXS = 64
 
 AN = dict(NUCDIV=0x001, SFS=0x002, LD_ZNS=0x004, LD_OMEGA=0x008, LD_WALL=0x010, DIVERGE_IND=0x020,
           DIVERGE_POP=0x040, HAPLO_K=0x080, HAPLO_EHHS=0x100, HAPLO_DXY=0x200, SNP=0x400, TREE=0x800,
-          THETA_W=0x1000, FULI=0x2000, LD_DPRIME=0x4000)
+          THETA_W=0x1000, FULI=0x2000, LD_DPRIME=0x4000, FST=0x8000)
 FLAG = dict(ILLUMINA=0x02, SUBSTITUTE=0x10, HETEROZYGOTE=0x20, OUTGROUP=0x40, EMIT_CB=0x10000)
 
 EXPORTS = ["pb_create", "pb_destroy", "pb_last_error", "pb_version", "pb_set_contig", "pb_region_begin", "pb_push_batch", "pb_push_batch_async",
            "pb_push_record", "pb_region_reserve", "pb_region_end", "pb_region_launch", "pb_region_wait", "pb_region_relaunch", "pb_stream",
            "pb_kernel_launches", "pb_region_path", "pb_region_reruns", "pb_stage_times", "pb_window_grid", "pb_build_errmod_tables", "pb_errmod_tables_cached", "pb_errmod_tables_cached_ex", "pb_host_alloc", "pb_host_free", "pb_format_window",
-           "pb_region_get_extras", "pb_format_window_ext"]
+           "pb_region_get_extras", "pb_format_window_ext", "pb_region_get_fst", "pb_set_snn_perms", "pb_format_window_fst"]
 
 
 def _p(t):
@@ -72,6 +72,13 @@ class Extras(C.Structure):
 
 
 EXT_BITS = AN["THETA_W"] | AN["FULI"] | AN["LD_DPRIME"]
+
+
+class Fst(C.Structure):
+    """pb_region_fst: the PB_AN_FST arrays, [NW*P*P] each, indexed like pib (snn_p / snn_ge only with permutations)."""
+    _fields_ = [("hud_num", _p(C.c_int64)), ("hud_den", _p(C.c_int64)), ("wc_num", _p(C.c_int64)), ("wc_den", _p(C.c_int64)),
+                ("fst_hudson", _p(C.c_double)), ("fst_wc", _p(C.c_double)), ("snn", _p(C.c_double)), ("snn_p", _p(C.c_double)),
+                ("snn_ge", _p(C.c_int64))]
 
 
 class PrintOpts(C.Structure):
@@ -140,6 +147,11 @@ def lib():
         L.pb_region_get_extras.argtypes = [C.c_void_p, _p(Extras)]
         L.pb_format_window_ext.restype = C.c_int64
         L.pb_format_window_ext.argtypes = [C.c_void_p, _p(Result), _p(Extras), C.c_int32, C.c_uint32, _p(PrintOpts), C.c_char_p, C.c_int64]
+        L.pb_region_get_fst.argtypes = [C.c_void_p, _p(Fst)]
+        L.pb_set_snn_perms.argtypes = [C.c_void_p, C.c_int64, C.c_uint64]
+        L.pb_format_window_fst.restype = C.c_int64
+        L.pb_format_window_fst.argtypes = [C.c_void_p, _p(Result), _p(Extras), _p(Fst), C.c_int32, C.c_uint32, _p(PrintOpts), C.c_char_p,
+                                           C.c_int64]
         _lib = L
     return _lib
 
@@ -164,6 +176,7 @@ class Context:
         self.L, self.params = L, params
         self.res = Result()
         self.ext = Extras()
+        self.fst = Fst()
 
     def _chk(self, rc):
         if rc != 0:
@@ -198,6 +211,7 @@ class Context:
     def region_end(self):
         self._chk(self.L.pb_region_end(self.h, C.byref(self.res)))
         self._chk(self.L.pb_region_get_extras(self.h, C.byref(self.ext)))
+        self._chk(self.L.pb_region_get_fst(self.h, C.byref(self.fst)))
         return self.res
 
     def launch(self):
@@ -209,7 +223,12 @@ class Context:
     def wait(self):
         self._chk(self.L.pb_region_wait(self.h, C.byref(self.res)))
         self._chk(self.L.pb_region_get_extras(self.h, C.byref(self.ext)))
+        self._chk(self.L.pb_region_get_fst(self.h, C.byref(self.fst)))
         return self.res
+
+    def set_snn_perms(self, n_perms, seed=0):
+        """Snn permutations per (window, population pair) for the regions that follow (PB_AN_FST); 0 = none."""
+        self._chk(self.L.pb_set_snn_perms(self.h, n_perms, seed))
 
     def stage_times(self):
         ms = (C.c_double * 4)()
@@ -229,12 +248,18 @@ class Context:
     def text(self, analysis, opts, windows=None):
         out = []
         buf = C.create_string_buffer(1 << 20)
+
+        def fmt(w, buf):
+            if analysis & AN["FST"]:
+                return self.L.pb_format_window_fst(self.h, C.byref(self.res), C.byref(self.ext), C.byref(self.fst), w, analysis, C.byref(opts),
+                                                   buf, len(buf))
+            return self.L.pb_format_window_ext(self.h, C.byref(self.res), C.byref(self.ext), w, analysis, C.byref(opts), buf, len(buf))
         for w in (range(self.res.n_windows) if windows is None else windows):
-            k = self.L.pb_format_window_ext(self.h, C.byref(self.res), C.byref(self.ext), w, analysis, C.byref(opts), buf, len(buf))
+            k = fmt(w, buf)
             if k < 0:
                 raise PopbamError("pb_format_window failed: %d" % k)
             if k >= len(buf):
                 buf = C.create_string_buffer(int(k) + 16)
-                k = self.L.pb_format_window_ext(self.h, C.byref(self.res), C.byref(self.ext), w, analysis, C.byref(opts), buf, len(buf))
+                k = fmt(w, buf)
             out.append(buf.raw[:k].decode())
         return "".join(out)

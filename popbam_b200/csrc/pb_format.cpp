@@ -185,22 +185,16 @@ void nj_newick(Out &out, const uint16_t *diff, int T, int num_sites, const pb_pr
     f.newick(out);
 }
 
-}  // namespace
-
-extern "C" int64_t pb_format_window(const pb_ctx *ctx, const pb_region_result *r, int32_t w, uint32_t an, const pb_print_opts *o,
-                                    char *buf, int64_t cap) {
-    if (an & (PB_AN_THETA_W | PB_AN_FULI | PB_AN_LD_DPRIME)) return PB_ERR_ARG;
-    return pb_format_window_ext(ctx, r, nullptr, w, an, o, buf, cap);
-}
-
-extern "C" int64_t pb_format_window_ext(const pb_ctx *ctx, const pb_region_result *r, const pb_region_extras *e, int32_t w, uint32_t an,
-                                        const pb_print_opts *o, char *buf, int64_t cap) {
+// every printer: one reference bit, optionally with its extension, whose columns follow the reference's, and (nucdiv
+// only, checked by pb_format_window_fst) the F_ST columns after those
+int64_t format_window(const pb_ctx *ctx, const pb_region_result *r, const pb_region_extras *e, const pb_region_fst *fs, int32_t w,
+                      uint32_t an, const pb_print_opts *o, char *buf, int64_t cap) {
     const pb_params *p = pb_ctx_params(ctx);
     if (!p || !r || !o || w < 0 || w >= r->n_windows) return PB_ERR_ARG;
     if ((r->analyses & an) != an) return PB_ERR_ARG;
-    // one reference bit, optionally with its extension, whose columns follow the reference's
     const uint32_t ext = an & (PB_AN_THETA_W | PB_AN_FULI | PB_AN_LD_DPRIME);
-    an &= ~ext;
+    const bool with_fst = (an & PB_AN_FST) != 0;
+    an &= ~(ext | PB_AN_FST);
     if (ext && (!e || ext != (an == PB_AN_NUCDIV ? PB_AN_THETA_W : an == PB_AN_SFS ? PB_AN_FULI : an == PB_AN_LD_ZNS ? PB_AN_LD_DPRIME : 0u)))
         return PB_ERR_ARG;
     Out out;
@@ -340,6 +334,15 @@ extern "C" int64_t pb_format_window_ext(const pb_ctx *ctx, const pb_region_resul
                 else out.f("\tDp1[%s]:\t%7s", o->pop_names[i], "NA");
             }
         }
+        for (int i = 0; with_fst && i < P - 1; ++i)
+            for (int j = i + 1; j < P; ++j) {
+                snprintf(nm, sizeof nm, "%s-%s", o->pop_names[i], o->pop_names[j]);
+                const size_t x = wp * P + i * P + (j - (i + 1));
+                out.stat("Fst", nm, ok && !std::isnan(fs->fst_hudson[x]), fs->fst_hudson[x]);
+                out.stat("FstWC", nm, ok && !std::isnan(fs->fst_wc[x]), fs->fst_wc[x]);
+                out.stat("Snn", nm, ok && !std::isnan(fs->snn[x]), fs->snn[x]);
+                if (fs->snn_p) out.stat("SnnP", nm, ok && !std::isnan(fs->snn_p[x]), fs->snn_p[x]);
+            }
         out.f("\n");
         }
     }
@@ -350,4 +353,25 @@ extern "C" int64_t pb_format_window_ext(const pb_ctx *ctx, const pb_region_resul
         buf[k] = 0;
     }
     return len;
+}
+
+}  // namespace
+
+extern "C" int64_t pb_format_window(const pb_ctx *ctx, const pb_region_result *r, int32_t w, uint32_t an, const pb_print_opts *o,
+                                    char *buf, int64_t cap) {
+    if (an & (PB_AN_THETA_W | PB_AN_FULI | PB_AN_LD_DPRIME | PB_AN_FST)) return PB_ERR_ARG;
+    return format_window(ctx, r, nullptr, nullptr, w, an, o, buf, cap);
+}
+
+extern "C" int64_t pb_format_window_ext(const pb_ctx *ctx, const pb_region_result *r, const pb_region_extras *e, int32_t w, uint32_t an,
+                                        const pb_print_opts *o, char *buf, int64_t cap) {
+    if (an & PB_AN_FST) return PB_ERR_ARG;
+    return format_window(ctx, r, e, nullptr, w, an, o, buf, cap);
+}
+
+extern "C" int64_t pb_format_window_fst(const pb_ctx *ctx, const pb_region_result *r, const pb_region_extras *e, const pb_region_fst *f,
+                                        int32_t w, uint32_t an, const pb_print_opts *o, char *buf, int64_t cap) {
+    if ((an & ~(PB_AN_THETA_W | PB_AN_FST)) != PB_AN_NUCDIV) return PB_ERR_ARG;
+    if ((an & PB_AN_FST) && (!f || !f->fst_hudson || !f->fst_wc || !f->snn)) return PB_ERR_ARG;
+    return format_window(ctx, r, e, f, w, an, o, buf, cap);
 }

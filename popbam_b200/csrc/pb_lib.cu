@@ -91,7 +91,10 @@ struct pb_ctx {
     bool no_async = false;                 // POPBAM_B200_SYNC=1: always take the host round trips (A/B measurements)
     int64_t seg_cap = 0;                   // device layout of the segregating-site arrays (async: sized by the span)
     DevBuf d_seg_type;     // arena of the segregating-site arrays (seg_layout)
-    DevBuf d_hap, d_kt, d_km, d_lsum, d_rsum, d_wall_u, d_stats, d_ld_kt, d_ld_km, d_ld_inv, d_ld_cnt, d_ld_dp;
+    DevBuf d_hap, d_kt, d_km, d_lsum, d_rsum, d_wall_u, d_stats, d_ld_kt, d_ld_km, d_ld_inv, d_ld_cnt, d_ld_dp, d_snn_nn;
+    int64_t snn_perms = 0;                 // pb_set_snn_perms: Snn permutations per (window, pair) and the stream's seed
+    uint64_t snn_seed = 0;
+    int64_t snn_perms_run = 0;             // ... as the last pipeline run used them
     // pinned results
     HostBuf h_ctr, h_small, h_seg, h_span;
     PbCounters ctr_host;
@@ -101,6 +104,7 @@ struct pb_ctx {
     int64_t s_total = 0;
     pb_region_result res;
     pb_region_extras ext;
+    pb_region_fst fst;
     // bam_fetch_f shim staging (pb_push_record)
     std::vector<int32_t> r_pos;
     std::vector<uint32_t> r_meta, r_cig_off, r_cigar, r_base_off;
@@ -196,9 +200,10 @@ struct SmallLayout {
     uint16_t *tree_diff;
     int32_t *pop_segsites; double *theta_w, *fuli_d, *fuli_ds; int32_t *fuli_eta_e, *fuli_eta_s;
     int32_t *ld_kept; double *ld_dprime; int64_t *ld_complete;
+    int64_t *hud_num, *hud_den, *wc_num, *wc_den; double *fst_hudson, *fst_wc, *snn, *snn_p; int64_t *snn_ge;
     size_t bytes;
 };
-SmallLayout small_layout(void *base, int NW, int P, int n, bool with_tree) {
+SmallLayout small_layout(void *base, int NW, int P, int n, bool with_tree, bool with_fst) {
     Carver cv(base);
     SmallLayout L;
     const size_t wp = (size_t)NW * P, wpp = (size_t)NW * P * P, wn = (size_t)NW * n;
@@ -213,6 +218,12 @@ SmallLayout small_layout(void *base, int NW, int P, int n, bool with_tree) {
     L.pop_segsites = cv.take<int32_t>(wp); L.theta_w = cv.take<double>(wp); L.fuli_d = cv.take<double>(wp); L.fuli_ds = cv.take<double>(wp);
     L.fuli_eta_e = cv.take<int32_t>(wp); L.fuli_eta_s = cv.take<int32_t>(wp);
     L.ld_kept = cv.take<int32_t>(wp); L.ld_dprime = cv.take<double>(wp); L.ld_complete = cv.take<int64_t>(wp);
+    L.hud_num = L.hud_den = L.wc_num = L.wc_den = L.snn_ge = nullptr; L.fst_hudson = L.fst_wc = L.snn = L.snn_p = nullptr;
+    if (with_fst) {         // the pair arrays of PB_AN_FST (none without it: the arena is what it was before them)
+        L.hud_num = cv.take<int64_t>(wpp); L.hud_den = cv.take<int64_t>(wpp); L.wc_num = cv.take<int64_t>(wpp); L.wc_den = cv.take<int64_t>(wpp);
+        L.fst_hudson = cv.take<double>(wpp); L.fst_wc = cv.take<double>(wpp); L.snn = cv.take<double>(wpp); L.snn_p = cv.take<double>(wpp);
+        L.snn_ge = cv.take<int64_t>(wpp);
+    }
     L.bytes = (cv.off + 255) & ~(size_t)255;
     return L;
 }
@@ -539,10 +550,10 @@ int run_pipeline(pb_ctx *c, int attempt = 0, bool allow_async = true) {
     PB_CUDA(c, cudaEventRecord(c->ev[3], st));
 
     // ---- per-window site counts, offsets of the segregating-site lists
-    const SmallLayout dl0 = small_layout(nullptr, NW, P.n_pops, n, (c->analyses & PB_AN_TREE) != 0);
+    const SmallLayout dl0 = small_layout(nullptr, NW, P.n_pops, n, (c->analyses & PB_AN_TREE) != 0, (c->analyses & PB_AN_FST) != 0);
     PB_TRY(dev_reserve(c, c->d_stats, dl0.bytes));
     PB_TRY(host_reserve(c, c->h_small, dl0.bytes));
-    const SmallLayout dl = small_layout(c->d_stats.p, NW, P.n_pops, n, (c->analyses & PB_AN_TREE) != 0);
+    const SmallLayout dl = small_layout(c->d_stats.p, NW, P.n_pops, n, (c->analyses & PB_AN_TREE) != 0, (c->analyses & PB_AN_FST) != 0);
     PB_CUDA(c, cudaMemsetAsync(c->d_stats.p, 0, dl.bytes, st));
     k_window_sites<false><<<NW, 256, 0, st>>>(c->span_beg, pa.win_beg, pa.win_end, pa.site_flag, pa.site_type, pa.ref, pa.ref_len, nullptr, n,
                                              dl.num_sites, dl.segsites, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr);
@@ -551,7 +562,7 @@ int run_pipeline(pb_ctx *c, int attempt = 0, bool allow_async = true) {
     PB_CUDA(c, cudaGetLastError());
     int64_t *h_total = reinterpret_cast<int64_t *>(c->h_ctr.p) + (sizeof(PbCounters) + 7) / 8;   // h_ctr has a page
     PB_CUDA(c, cudaMemcpyAsync(h_total, dl.seg_off + NW, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
-    const SmallLayout hl0 = small_layout(c->h_small.p, NW, P.n_pops, n, (c->analyses & PB_AN_TREE) != 0);
+    const SmallLayout hl0 = small_layout(c->h_small.p, NW, P.n_pops, n, (c->analyses & PB_AN_TREE) != 0, (c->analyses & PB_AN_FST) != 0);
     PB_CUDA(c, cudaMemcpyAsync(hl0.segsites, dl.segsites, sizeof(int32_t) * (size_t)NW, cudaMemcpyDeviceToHost, st));
     PbCounters *h_final = reinterpret_cast<PbCounters *>(reinterpret_cast<unsigned char *>(c->h_ctr.p) + 2 * sizeof(PbCounters));
     if (async) PB_CUDA(c, cudaStreamWaitEvent(st, c->fk[2], 0));     // the per-read chain that ran beside the pileup
@@ -605,7 +616,7 @@ int run_pipeline(pb_ctx *c, int attempt = 0, bool allow_async = true) {
     // ---- window statistics
     const uint32_t stat_bits = PB_AN_NUCDIV | PB_AN_SFS | PB_AN_LD_WALL | PB_AN_DIVERGE_IND |
                                PB_AN_DIVERGE_POP | PB_AN_HAPLO_K | PB_AN_HAPLO_EHHS | PB_AN_HAPLO_DXY | PB_AN_TREE |
-                               PB_AN_THETA_W | PB_AN_FULI;
+                               PB_AN_THETA_W | PB_AN_FULI | PB_AN_FST;
     if (c->analyses & stat_bits) {
         PbStatArgs sa;
         memset(&sa, 0, sizeof sa);
@@ -614,7 +625,7 @@ int run_pipeline(pb_ctx *c, int attempt = 0, bool allow_async = true) {
         sa.analyses = c->analyses; sa.flags = P.flags; sa.outidx = P.outidx; sa.min_freq = P.min_freq;
         sa.num_sites = dl.num_sites; sa.segsites = dl.segsites; sa.seg_off = dl.seg_off; sa.seg_type = sl.seg_type;
         sa.s_total = S;
-        if (c->analyses & (PB_AN_NUCDIV | PB_AN_HAPLO_K | PB_AN_HAPLO_EHHS | PB_AN_HAPLO_DXY | PB_AN_DIVERGE_IND | PB_AN_TREE)) {
+        if (c->analyses & (PB_AN_NUCDIV | PB_AN_HAPLO_K | PB_AN_HAPLO_EHHS | PB_AN_HAPLO_DXY | PB_AN_DIVERGE_IND | PB_AN_TREE | PB_AN_FST)) {
             PB_TRY(dev_reserve(c, c->d_hap, sizeof(uint64_t) * (size_t)n * (size_t)(S / 64 + NW + 1)));
             sa.hap = dp<uint64_t>(c->d_hap);
         }
@@ -634,9 +645,31 @@ int run_pipeline(pb_ctx *c, int attempt = 0, bool allow_async = true) {
         sa.nhaps = dl.nhaps; sa.hdiv = dl.hdiv; sa.ehhs = dl.ehhs;
         sa.pop_segsites = dl.pop_segsites; sa.theta_w = dl.theta_w; sa.fuli_d = dl.fuli_d; sa.fuli_ds = dl.fuli_ds;
         sa.fuli_eta_e = dl.fuli_eta_e; sa.fuli_eta_s = dl.fuli_eta_s;
-        k_window_stats<<<NW, PB_ST_THREADS, (size_t)n * n * sizeof(uint16_t), st>>>(sa);
+        const int npairs = P.n_pops * (P.n_pops - 1) / 2;
+        const bool perms = (c->analyses & PB_AN_FST) && c->snn_perms > 0 && npairs > 0;
+        c->snn_perms_run = perms ? c->snn_perms : 0;
+        if (c->analyses & PB_AN_FST) {
+            sa.hud_num = dl.hud_num; sa.hud_den = dl.hud_den; sa.wc_num = dl.wc_num; sa.wc_den = dl.wc_den;
+            sa.fst_hudson = dl.fst_hudson; sa.fst_wc = dl.fst_wc; sa.snn = dl.snn;
+            if (perms) {        // nearest-neighbour masks of every (window, pair, sample) for k_snn_perm
+                PB_TRY(dev_reserve(c, c->d_snn_nn, sizeof(uint64_t) * (size_t)NW * P.n_pops * P.n_pops * n));
+                sa.snn_nn = dp<uint64_t>(c->d_snn_nn);
+            }
+        }
+        ((c->analyses & PB_AN_FST) ? k_window_stats<true> : k_window_stats<false>)<<<NW, PB_ST_THREADS, (size_t)n * n * sizeof(uint16_t), st>>>(sa);
         c->launches += 1;
         PB_CUDA(c, cudaGetLastError());
+        if (perms) {
+            PbSnnArgs ka;
+            memset(&ka, 0, sizeof ka);
+            ka.n = n; ka.P = P.n_pops; ka.tid = c->ref_tid;
+            for (int i = 0; i < PB_MAX_SAMPLES; ++i) { ka.pop_mask[i] = P.pop_mask[i]; ka.pop_nsmpl[i] = P.pop_nsmpl[i]; }
+            ka.win_beg = dp<int32_t>(c->d_wbeg); ka.nn = sa.snn_nn; ka.snn = dl.snn; ka.snn_p = dl.snn_p; ka.snn_ge = dl.snn_ge;
+            ka.n_perms = c->snn_perms; ka.seed = c->snn_seed;
+            k_snn_perm<<<dim3((unsigned)NW, (unsigned)npairs), PB_ST_THREADS, 0, st>>>(ka);
+            c->launches += 1;
+            PB_CUDA(c, cudaGetLastError());
+        }
     }
     // ---- pairwise LD (ld -o 0 / -o 1, D'): keep list, tiled pair kernel, finish
     if (c->analyses & (PB_AN_LD_ZNS | PB_AN_LD_OMEGA | PB_AN_LD_DPRIME)) {
@@ -736,7 +769,7 @@ int fill_result(pb_ctx *c, pb_region_result *out) {
     cudaEventElapsedTime(&c->ms_pileup, c->ev[2], c->ev[3]);
     cudaEventElapsedTime(&c->ms_sites, c->ev[3], c->ev[4]);
     cudaEventElapsedTime(&c->ms_stats, c->ev[4], c->ev[5]);
-    const SmallLayout hl = small_layout(c->h_small.p, NW, P.n_pops, n, (c->analyses & PB_AN_TREE) != 0);
+    const SmallLayout hl = small_layout(c->h_small.p, NW, P.n_pops, n, (c->analyses & PB_AN_TREE) != 0, (c->analyses & PB_AN_FST) != 0);
     const bool with_cb = (c->analyses & PB_AN_SNP) != 0;
     const SegLayout sl = seg_layout(c->h_seg.p, c->s_total, n, with_cb);
     pb_region_result &r = c->res;
@@ -758,6 +791,13 @@ int fill_result(pb_ctx *c, pb_region_result *out) {
     if (an & PB_AN_THETA_W) e.theta_w = hl.theta_w;
     if (an & PB_AN_FULI) { e.fuli_d = hl.fuli_d; e.fuli_ds = hl.fuli_ds; e.fuli_eta_e = hl.fuli_eta_e; e.fuli_eta_s = hl.fuli_eta_s; }
     if (an & PB_AN_LD_DPRIME) { r.ld_num_snps = hl.ld_num_snps; e.ld_kept = hl.ld_kept; e.ld_dprime = hl.ld_dprime; e.ld_complete = hl.ld_complete; }
+    pb_region_fst &f = c->fst;
+    memset(&f, 0, sizeof f);
+    if (an & PB_AN_FST) {
+        f.hud_num = hl.hud_num; f.hud_den = hl.hud_den; f.wc_num = hl.wc_num; f.wc_den = hl.wc_den;
+        f.fst_hudson = hl.fst_hudson; f.fst_wc = hl.fst_wc; f.snn = hl.snn;
+        if (c->snn_perms_run > 0) { f.snn_p = hl.snn_p; f.snn_ge = hl.snn_ge; }
+    }
     if (an & PB_AN_DIVERGE_POP) { r.pop_div = hl.pop_div; r.div_num_snps = hl.div_num_snps; }
     if (an & (PB_AN_HAPLO_K | PB_AN_HAPLO_EHHS)) { r.nhaps = hl.nhaps; r.hdiv = hl.hdiv; }
     if (an & PB_AN_HAPLO_EHHS) r.ehhs = hl.ehhs;
@@ -1084,6 +1124,19 @@ int pb_region_end(pb_ctx *c, pb_region_result *out) {
 int pb_region_get_extras(const pb_ctx *c, pb_region_extras *out) {
     if (!c || !out) return PB_ERR_ARG;
     *out = c->ext;
+    return PB_OK;
+}
+
+int pb_region_get_fst(const pb_ctx *c, pb_region_fst *out) {
+    if (!c || !out) return PB_ERR_ARG;
+    *out = c->fst;
+    return PB_OK;
+}
+
+int pb_set_snn_perms(pb_ctx *c, int64_t n_perms, uint64_t seed) {
+    if (!c) return PB_ERR_ARG;
+    if (n_perms < 0 || n_perms > 0x7fffffffLL) return fail(c, PB_ERR_ARG, "pb_set_snn_perms: n_perms must be in 0 .. 2^31 - 1");
+    c->snn_perms = n_perms; c->snn_seed = seed;
     return PB_OK;
 }
 

@@ -9,7 +9,8 @@
 //   calc_diverge                   pop_diverge.cpp:220-257
 //   calc_nhaps / calc_ehhs         pop_haplo.cpp:208-254, :256-323
 //   extensions (no reference counterpart): Watterson's theta and Fu & Li's D / D* on calc_sfs's spectrum,
-//   the closed forms of tests/ext_oracle.c in the same operation order
+//   the closed forms of tests/ext_oracle.c in the same operation order; F_ST and Snn between population pairs
+//   (PB_AN_FST, pb_fst_pairs and k_snn_perm below, restated by tests/fst_oracle.c)
 //
 // Integer results are exact.  Floating-point statistics use the reference's formulas term by term
 // (the library is compiled with -fmad=false so products and sums round separately, as on x86-64);
@@ -45,6 +46,9 @@ struct PbStatArgs {
     int32_t *nhaps; double *hdiv, *ehhs;
     uint16_t *tree_diff;  // [NW][(n+1)*(n+1)]
     int32_t *pop_segsites; double *theta_w, *fuli_d, *fuli_ds; int32_t *fuli_eta_e, *fuli_eta_s;
+    // PB_AN_FST, [NW][P*P] indexed like pib; snn_nn [NW][P*P][n]: nearest-neighbour masks for k_snn_perm (null without permutations)
+    int64_t *hud_num, *hud_den, *wc_num, *wc_den; double *fst_hudson, *fst_wc, *snn;
+    uint64_t *snn_nn;
 };
 
 // analysis bits (include/popbam_b200.h)
@@ -61,6 +65,7 @@ struct PbStatArgs {
 #define PBA_HAPLO_DXY 0x200u
 #define PBA_THETA_W 0x1000u
 #define PBA_FULI 0x2000u
+#define PBA_FST 0x8000u
 #define PBA_FLAG_OUTGROUP 0x40u
 
 __device__ __forceinline__ int pb_block_sum_int(int v, int *sh /* [32] */) {
@@ -138,6 +143,170 @@ __device__ __forceinline__ void pb_sfs_ext(int np, int seg, int xi1, int xin1, b
     if (fuli_d) { *fuli_d = fd; *fuli_ds = fds; *eta_e = ee; *eta_s = es; }
 }
 
+// ---- F_ST and Snn of every population pair i < j of one window (PB_AN_FST; include/popbam_b200.h, pb_region_fst).
+// n1, n2 = pop_nsmpl[i], pop_nsmpl[j]; per segregating site T: c1 = popc(T & pop_mask[i]), c2 = popc(T & pop_mask[j]).
+// Hudson (Bhatia et al. 2013), every term scaled by n1 n2 (n1-1) (n2-1):
+//   hud_den = sum (n1-1)(n2-1) [c1 (n2-c2) + c2 (n1-c1)],  hud_num = hud_den - sum [c1 (n1-c1) n2 (n2-1) + c2 (n2-c2) n1 (n1-1)]
+// Weir & Cockerham's haploid theta (r = 2), scaled by n1 n2 (n1+n2) (n1+n2-2), with G = c1 (n1-c1) n2 + c2 (n2-c2) n1:
+//   wc_num = sum (c1 n2 - c2 n1)^2 (n1+n2-2) - G (n1+n2),  wc_den = sum (c1 n2 - c2 n1)^2 (n1+n2-2) + G (2 n1 n2 - n1 - n2)
+// Every site term is an integer below 2^31 for n <= 64, so the int64 window sums are exact and independent of the order.
+// Snn (Hudson 2000): NN(x) = the other pooled samples at the least diff[x][y]; X_x = |NN(x) & pop(x)| / |NN(x)|;
+// Snn = (sum of X_x in ascending sample order, one thread) / (n1 + n2).  All three are NaN if n1 < 2 or n2 < 2.
+__device__ __forceinline__ void pb_block_sum_i64x4(long long v[4], long long (*sh)[4] /* [warps][4] */) {
+    for (int k = 0; k < 4; ++k)
+        for (int o = 16; o > 0; o >>= 1) v[k] += __shfl_xor_sync(0xffffffffu, v[k], o);
+    __syncthreads();
+    if ((threadIdx.x & 31) == 0)
+        for (int k = 0; k < 4; ++k) sh[threadIdx.x >> 5][k] = v[k];
+    __syncthreads();
+    for (int k = 0; k < 4; ++k) {
+        long long t = 0;
+        for (int i = 0; i < (int)(blockDim.x >> 5); ++i) t += sh[i][k];
+        v[k] = t;
+    }
+}
+
+__device__ __forceinline__ void pb_fst_pairs(const PbStatArgs &a, int w, const uint64_t *__restrict__ T, int S, const uint16_t *diff) {
+    __shared__ long long red[PB_ST_THREADS / 32][4];
+    __shared__ double xs[64];
+    const int tid = threadIdx.x, n = a.n, P = a.P;
+    for (int i = 0; i < P - 1; ++i)
+        for (int j = i + 1; j < P; ++j) {
+            const uint64_t mi = a.pop_mask[i], mj = a.pop_mask[j], pool = mi | mj;
+            const long long n1 = a.pop_nsmpl[i], n2 = a.pop_nsmpl[j];
+            const long long hf = (n1 - 1) * (n2 - 1), wa = n1 + n2 - 2, wb = n1 + n2, wc = 2 * n1 * n2 - n1 - n2;
+            const size_t x = (size_t)w * P * P + i * P + (j - (i + 1));
+            long long v[4] = {0, 0, 0, 0};      // hud_num, hud_den, wc_num, wc_den
+            for (int s = tid; s < S; s += PB_ST_THREADS) {
+                const uint64_t t = T[s];
+                const long long c1 = __popcll(t & mi), c2 = __popcll(t & mj);
+                const long long hd = hf * (c1 * (n2 - c2) + c2 * (n1 - c1));
+                const long long hw = c1 * (n1 - c1) * n2 * (n2 - 1) + c2 * (n2 - c2) * n1 * (n1 - 1);
+                const long long dd = c1 * n2 - c2 * n1, msp = dd * dd * wa, g = c1 * (n1 - c1) * n2 + c2 * (n2 - c2) * n1;
+                v[0] += hd - hw; v[1] += hd; v[2] += msp - g * wb; v[3] += msp + g * wc;
+            }
+            pb_block_sum_i64x4(v, red);
+            const bool two = n1 >= 2 && n2 >= 2;
+            if (two && tid < n && (pool >> tid & 1)) {
+                unsigned mn = 0xffffffffu;
+                uint64_t nn = 0;
+                for (int y = 0; y < n; ++y) {
+                    if (y == tid || !(pool >> y & 1)) continue;
+                    const unsigned d = diff[tid * n + y];
+                    if (d < mn) { mn = d; nn = 0; }
+                    if (d == mn) nn |= 1ULL << y;
+                }
+                const uint64_t own = (mi >> tid & 1) ? mi : mj;
+                xs[tid] = (double)__popcll(nn & own) / (double)__popcll(nn);
+                if (a.snn_nn) a.snn_nn[x * n + tid] = nn;
+            }
+            __syncthreads();
+            if (tid == 0) {
+                a.hud_num[x] = v[0]; a.hud_den[x] = v[1]; a.wc_num[x] = v[2]; a.wc_den[x] = v[3];
+                a.fst_hudson[x] = two && v[1] != 0 ? (double)v[0] / (double)v[1] : nan("");
+                a.fst_wc[x] = two && v[3] != 0 ? (double)v[2] / (double)v[3] : nan("");
+                double snn = nan("");
+                if (two) {
+                    double sum = 0.0;
+                    for (int y = 0; y < n; ++y)
+                        if (pool >> y & 1) sum += xs[y];
+                    snn = sum / (double)(n1 + n2);
+                }
+                a.snn[x] = snn;
+            }
+            __syncthreads();     // xs and red are reused by the next pair
+        }
+}
+
+// ---- Snn permutation test (PB_AN_FST with pb_set_snn_perms): grid (window, pair q in dxy order), threads stride over
+// the permutations.  NN(x) does not depend on the labels, so a permutation only re-partitions the pool: population i is
+// the n1 samples a partial Fisher-Yates shuffle of the pool (ascending sample order) puts first.  snn_ge counts the
+// permutations whose Snn >= Snn_obs - 1e-12; snn_p = (1 + snn_ge) / (1 + n_perms).
+// Random stream (counter-based, so it does not depend on how a region is cut into windows, shards or GPUs):
+//   mix(z)   = splitmix64's finaliser: z = (z ^ z>>30) * 0xbf58476d1ce4e5b9; z = (z ^ z>>27) * 0x94d049bb133111eb; z ^ z>>31
+//   key      h = mix(seed + G); then h = mix((h ^ v) + G) for v = tid, win_beg, i, j, permutation index in turn
+//            (G = 0x9e3779b97f4a7c15; each v as a 64-bit two's-complement integer)
+//   draw k   z_k = mix(h + (k + 1) G), k = 0, 1, ...  (the k-th output of a splitmix64 generator started at h)
+//   index    in [0, r): ((z >> 32) * r) >> 32;  shuffle step k swaps slot k with slot k + index(z_k, m - k)
+#define PB_GOLDEN64 0x9e3779b97f4a7c15ULL
+__device__ __forceinline__ uint64_t pb_mix64(uint64_t z) {
+    z = (z ^ (z >> 30)) * 0xbf58476d1ce4e5b9ULL;
+    z = (z ^ (z >> 27)) * 0x94d049bb133111ebULL;
+    return z ^ (z >> 31);
+}
+
+struct PbSnnArgs {
+    int n, P, tid;
+    uint64_t pop_mask[64];
+    uint8_t pop_nsmpl[64];
+    const int32_t *win_beg;
+    const uint64_t *nn;        // PbStatArgs::snn_nn
+    const double *snn;
+    double *snn_p;
+    int64_t *snn_ge;
+    long long n_perms;
+    uint64_t seed;
+};
+
+__global__ void __launch_bounds__(PB_ST_THREADS) k_snn_perm(const PbSnnArgs a) {
+    __shared__ uint64_t nn[64];
+    __shared__ unsigned long long red[PB_ST_THREADS / 32];
+    const int w = blockIdx.x, P = a.P, n = a.n, tid = threadIdx.x;
+    int i = 0, r = blockIdx.y;
+    while (r >= P - 1 - i) { r -= P - 1 - i; ++i; }
+    const int j = i + 1 + r;
+    const size_t x = (size_t)w * P * P + i * P + (j - (i + 1));
+    const int n1 = a.pop_nsmpl[i], m = n1 + a.pop_nsmpl[j];
+    if (n1 < 2 || a.pop_nsmpl[j] < 2) {
+        if (tid == 0) { a.snn_ge[x] = 0; a.snn_p[x] = nan(""); }
+        return;
+    }
+    const uint64_t pool = a.pop_mask[i] | a.pop_mask[j];
+    if (tid < n) nn[tid] = a.nn[x * n + tid];
+    __syncthreads();
+    const double thr = a.snn[x] - 1e-12;
+    uint64_t key = pb_mix64(a.seed + PB_GOLDEN64);
+    key = pb_mix64((key ^ (uint64_t)(int64_t)a.tid) + PB_GOLDEN64);
+    key = pb_mix64((key ^ (uint64_t)(int64_t)a.win_beg[w]) + PB_GOLDEN64);
+    key = pb_mix64((key ^ (uint64_t)(int64_t)i) + PB_GOLDEN64);
+    key = pb_mix64((key ^ (uint64_t)(int64_t)j) + PB_GOLDEN64);
+    unsigned long long ge = 0;
+    for (long long k = tid; k < a.n_perms; k += PB_ST_THREADS) {
+        const uint64_t h = pb_mix64((key ^ (uint64_t)k) + PB_GOLDEN64);
+        uint8_t idx[64];
+        {
+            uint64_t t = pool;
+            for (int c = 0; c < m; ++c) { idx[c] = (uint8_t)(__ffsll((long long)t) - 1); t &= t - 1; }
+        }
+        uint64_t A = 0;
+        for (int c = 0; c < n1; ++c) {
+            const uint64_t z = pb_mix64(h + (uint64_t)(c + 1) * PB_GOLDEN64);
+            const int rr = c + (int)(((z >> 32) * (uint64_t)(m - c)) >> 32);
+            const uint8_t s = idx[rr];
+            idx[rr] = idx[c]; idx[c] = s;
+            A |= 1ULL << s;
+        }
+        const uint64_t B = pool & ~A;
+        double sum = 0.0;
+        for (uint64_t t = pool; t; t &= t - 1) {
+            const int y = __ffsll((long long)t) - 1;
+            sum += (double)__popcll(nn[y] & ((A >> y & 1) ? A : B)) / (double)__popcll(nn[y]);
+        }
+        ge += sum / (double)m >= thr;
+    }
+    for (int o = 16; o > 0; o >>= 1) ge += __shfl_xor_sync(0xffffffffu, ge, o);
+    if ((tid & 31) == 0) red[tid >> 5] = ge;
+    __syncthreads();
+    if (tid == 0) {
+        unsigned long long t = 0;
+        for (int k = 0; k < PB_ST_THREADS / 32; ++k) t += red[k];
+        a.snn_ge[x] = (int64_t)t;
+        a.snn_p[x] = (1.0 + (double)t) / (1.0 + (double)a.n_perms);
+    }
+}
+
+// k_window_stats<true> adds the F_ST pass (PB_AN_FST); k_window_stats<false> compiles to the kernel without it
+template <bool FST>
 __global__ void __launch_bounds__(PB_ST_THREADS) k_window_stats(const PbStatArgs a) {
     extern __shared__ __align__(16) unsigned char st_smem[];
     uint16_t *diff = reinterpret_cast<uint16_t *>(st_smem);                   // [n*n]
@@ -156,7 +325,7 @@ __global__ void __launch_bounds__(PB_ST_THREADS) k_window_stats(const PbStatArgs
     const bool outg = (a.flags & PBA_FLAG_OUTGROUP) != 0;
 
     // ---- haplotype words: bit s of hap[i] = sample i carries the derived allele at segsite s
-    if (an & (PBA_NUCDIV | PBA_HAPLO_K | PBA_HAPLO_EHHS | PBA_HAPLO_DXY | PBA_DIVERGE_IND | PBA_TREE)) {
+    if (an & (PBA_NUCDIV | PBA_HAPLO_K | PBA_HAPLO_EHHS | PBA_HAPLO_DXY | PBA_DIVERGE_IND | PBA_TREE | (FST ? PBA_FST : 0u))) {
         for (int idx = tid; idx < n * nwords; idx += PB_ST_THREADS) {
             const int i = idx / nwords, kw = idx - i * nwords;
             uint64_t word = 0;
@@ -191,7 +360,7 @@ __global__ void __launch_bounds__(PB_ST_THREADS) k_window_stats(const PbStatArgs
         }
     }
     // ---- pairwise difference matrix (unsigned short, wraps)
-    if (an & (PBA_NUCDIV | PBA_HAPLO_K | PBA_HAPLO_EHHS | PBA_HAPLO_DXY)) {
+    if (an & (PBA_NUCDIV | PBA_HAPLO_K | PBA_HAPLO_EHHS | PBA_HAPLO_DXY | (FST ? PBA_FST : 0u))) {
         for (int pi = tid; pi < n * n; pi += PB_ST_THREADS) {
             const int i = pi / n, j = pi - i * n;
             unsigned d = 0;
@@ -224,6 +393,8 @@ __global__ void __launch_bounds__(PB_ST_THREADS) k_window_stats(const PbStatArgs
             }
         }
     }
+    // ---- F_ST and Snn of every population pair (extension)
+    if constexpr (FST) pb_fst_pairs(a, w, T, S, diff);
     // ---- haplotype count / diversity (literal, within-population ranks index the matrix: SURVEY Q12)
     if (an & (PBA_HAPLO_K | PBA_HAPLO_EHHS)) {
         for (int i = tid; i < P; i += PB_ST_THREADS) {

@@ -13,7 +13,9 @@
 //
 // Extra options (not in the reference): --gpus N, --shard-mb X, --threads T, and --extra-stats: statistics the
 // reference does not compute, as extra columns after its own (nucdiv: Watterson's theta; sfs: Fu & Li's D* and, with
-// -p, D; ld -o 0: mean |D'| and the number of SNP pairs in complete LD).
+// -p, D; ld -o 0: mean |D'| and the number of SNP pairs in complete LD); for nucdiv only, --fst: F_ST (Hudson, and Weir &
+// Cockerham) and Hudson's Snn for every population pair, after the --extra-stats columns, with --snn-perms N: a permutation
+// p-value of Snn from N random re-partitions of the pair's samples, drawn from a stream seeded by --seed S (default 0).
 #include <algorithm>
 #include <atomic>
 #include <condition_variable>
@@ -48,6 +50,9 @@ struct Options {
     std::vector<std::string> positional;
     int gpus = 1, threads = 0;
     bool extra_stats = false;
+    bool fst = false, snn_opts = false;
+    long long snn_perms = 0;
+    unsigned long long seed = 0;
     double shard_mb = 2.0;
 };
 
@@ -69,7 +74,9 @@ void usage(const char *cmd) {
             "Options: -f FILE reference fastA   -w INT window (kb)   -m/-x INT min/max depth   -q INT min rms mapQ\n"
             "         -s INT min snpQ   -a/-b INT min mapQ / baseQ   -k INT min sites   -o INT output mode   -p STR outgroup\n"
             "         -i Illumina 1.3+ qualities   --gpus N   --shard-mb X   --threads T\n"
-            "         --extra-stats  nucdiv: theta[pop]; sfs: FuLiD*[pop] (and FuLiD[pop] with -p); ld -o 0: Dp[pop], Dp1[pop]\n", cmd);
+            "         --extra-stats  nucdiv: theta[pop]; sfs: FuLiD*[pop] (and FuLiD[pop] with -p); ld -o 0: Dp[pop], Dp1[pop]\n"
+            "         --fst  nucdiv: Fst[A-B] (Hudson), FstWC[A-B] (Weir & Cockerham), Snn[A-B] (Hudson's nearest neighbours)\n"
+            "         --snn-perms N  with --fst: SnnP[A-B], p-value of Snn from N permutations   --seed S  their random stream (0)\n", cmd);
 }
 
 Options parse(int argc, char **argv) {
@@ -83,6 +90,16 @@ Options parse(int argc, char **argv) {
         if (a.rfind("--", 0) == 0) {
             auto val = [&]() -> const char * { if (i + 1 >= argc) fatal("missing value for " + a); return argv[++i]; };
             if (a == "--extra-stats") { o.extra_stats = true; continue; }
+            if (a == "--fst") { o.fst = true; continue; }
+            if (a == "--snn-perms" || a == "--seed") {
+                const char *v = val();
+                char *end = nullptr;
+                if (a == "--seed") o.seed = strtoull(v, &end, 10);
+                else o.snn_perms = strtoll(v, &end, 10);
+                if (!*v || *end || v[0] == '-' || o.snn_perms > 0x7fffffffLL) fatal("invalid value for " + a + ": " + v);
+                o.snn_opts = true;
+                continue;
+            }
             if (a == "--gpus") o.gpus = atoi(val());
             else if (a == "--shard-mb") o.shard_mb = atof(val());
             else if (a == "--threads") o.threads = atoi(val());
@@ -142,6 +159,8 @@ Options parse(int argc, char **argv) {
     }
     if (o.extra_stats && !(o.cmd == "nucdiv" || o.cmd == "sfs" || (o.cmd == "ld" && o.output == 0)))
         fatal("--extra-stats is only available for nucdiv, sfs and ld -o 0");
+    if ((o.fst || o.snn_opts) && o.cmd != "nucdiv") fatal("--fst, --snn-perms and --seed are only available for nucdiv");
+    if (o.snn_opts && !o.fst) fatal("--snn-perms and --seed go with --fst");
     return o;
 }
 
@@ -277,6 +296,7 @@ void gpu_worker(Run *R, int g, int G, int device) {
     std::string err;
     if (!ctx) err = std::string("cannot initialise GPU ") + std::to_string(device) + ": " + pb_last_error(nullptr);
     else if (pb_set_contig(ctx, R->tid, R->ref.data(), (int64_t)R->ref.size()) != PB_OK) err = pb_last_error(ctx);
+    else if (pb_set_snn_perms(ctx, R->opt.snn_perms, R->opt.seed) != PB_OK) err = pb_last_error(ctx);
     std::vector<const char *> pops, smps;
     for (auto &s : R->st.pops) pops.push_back(s.c_str());
     for (auto &s : R->st.samples) smps.push_back(s.c_str());
@@ -296,6 +316,7 @@ void gpu_worker(Run *R, int g, int G, int device) {
         if (err.empty() && sh.error.empty()) {
             pb_region_result res;
             pb_region_extras ext;
+            pb_region_fst fst;
             int rc = pb_region_begin(ctx, R->analysis, sh.w1 - sh.w0, &R->wb[sh.w0], &R->we[sh.w0]);
             {
                 int64_t nr = 0, nc = 0, nb = 0;
@@ -315,11 +336,16 @@ void gpu_worker(Run *R, int g, int G, int device) {
             }
             if (rc == PB_OK) rc = pb_region_end(ctx, &res);
             if (rc == PB_OK) rc = pb_region_get_extras(ctx, &ext);
+            if (rc == PB_OK) rc = pb_region_get_fst(ctx, &fst);
+            auto format = [&](int w) {
+                return (R->analysis & PB_AN_FST) ? pb_format_window_fst(ctx, &res, &ext, &fst, w, R->analysis, &po, line.data(), (int64_t)line.size())
+                                                 : pb_format_window_ext(ctx, &res, &ext, w, R->analysis, &po, line.data(), (int64_t)line.size());
+            };
             if (rc != PB_OK) sh.error = pb_last_error(ctx);
             else
                 for (int w = 0; w < res.n_windows; ++w) {
-                    int64_t k = pb_format_window_ext(ctx, &res, &ext, w, R->analysis, &po, line.data(), (int64_t)line.size());
-                    if (k >= (int64_t)line.size()) { line.resize((size_t)k + 16); k = pb_format_window_ext(ctx, &res, &ext, w, R->analysis, &po, line.data(), (int64_t)line.size()); }
+                    int64_t k = format(w);
+                    if (k >= (int64_t)line.size()) { line.resize((size_t)k + 16); k = format(w); }
                     if (k < 0) { sh.error = "formatting failed"; break; }
                     sh.text.append(line.data(), (size_t)k);
                 }
@@ -482,6 +508,7 @@ int main(int argc, char **argv) {
     else R.analysis = PB_AN_SNP;
     if (o.output < 0 || o.output > 2) fatal("invalid output option");
     if (o.extra_stats) R.analysis |= o.cmd == "nucdiv" ? PB_AN_THETA_W : o.cmd == "sfs" ? PB_AN_FULI : PB_AN_LD_DPRIME;
+    if (o.fst) R.analysis |= PB_AN_FST;
 
     // window grid of the region, then shards = runs of whole windows
     const int64_t nw = pb_window_grid(R.beg, R.end, o.window ? o.win_size : 0, 0, nullptr, nullptr);
