@@ -66,6 +66,9 @@ typedef enum pb_status {
 #define PB_AN_FULI          0x2000u /* Fu & Li's D (outgroup only) and D*              (with sfs)             */
 #define PB_AN_LD_DPRIME     0x4000u /* Lewontin's |D'| over the ZnS pairs              (with ld -o 0)         */
 #define PB_AN_FST           0x8000u /* F_ST (Hudson, Weir & Cockerham) and Snn per population pair (with nucdiv) */
+#define PB_AN_ABBA          0x10000u /* ABBA-BABA: Patterson's D, f_d, f_dM per triple (pb_set_abba; alone or with any) */
+
+#define PB_MAX_ABBA_TRIPLES 1024     /* pb_set_abba: most (P1, P2, P3) triples of one region                        */
 
 /* Run parameters == the fields of popbamData the hot path reads (popbam.h:218-265) plus
  * the population tables assign_pops builds (popbam.cpp:145-171).                           */
@@ -221,6 +224,34 @@ typedef struct pb_region_fst {
     const int64_t *snn_ge;              /* permutations of the pooled labels with Snn >= Snn_obs - 1e-12       */
 } pb_region_fst;
 
+/* ABBA-BABA statistics of every window and triple (P1, P2, P3) of the last region against the outgroup population O
+ * (PB_AN_ABBA, pb_set_abba): a struct of its own, like pb_region_fst, with the same lifetime.  Every array is NULL
+ * unless PB_AN_ABBA was requested.  All arrays [NW*NT], index w*NT + t, NT = n_triples.
+ * Per segregating site of the window, k = 1..4 for P1, P2, P3, O: a_k = popcount(seg_type & pop_mask[k]) (calls count
+ * as haploid, as for pi and dxy; with PB_FLAG_HETEROZYGOTE a heterozygous call carries the allele), n_k = pop_nsmpl[k],
+ * m_k = n_k - a_k.  Polarisation: if 2 a_4 > n_4 every a_k and m_k are swapped, so the derived allele is the one O
+ * carries at frequency <= 1/2 (kept as is on a tie; PB_FLAG_OUTGROUP and outidx play no part).  Every site term is an
+ * exact integer on the scale K = n1^2 n2^2 n3^2 n4 (K < 2^29 and |term| <= K for n1 + n2 + n3 + n4 <= 64):
+ *   abba    += m1 a2 a3 m4 n1 n2 n3                                       ((1-p1) p2 p3 (1-p4) K)
+ *   baba    += a1 m2 a3 m4 n1 n2 n3                                       (p1 (1-p2) p3 (1-p4) K)
+ *   fd_den  += (m1 a2^2 - a1 m2 a2) m4 n1 n3^2   if a2 n3 >= a3 n2 (p2 >= p3), else (m1 a3^2 - a1 m3 a3) m4 n1 n2^2
+ *              (Martin, Davey & Jiggins 2015: S(P1, PD, PD, O) K with pD = max(p2, p3))
+ *   fdm_den += the fd_den term if a2 n1 >= a1 n2 (p2 >= p1); else -S(PD, P2, PD, O) K with pD = max(p1, p3):
+ *              (a1^2 m2 - m1 a2 a1) m4 n2 n3^2 if a1 n3 >= a3 n1, else (a3^2 m2 - m3 a2 a3) m4 n1^2 n2  (Malinsky et al. 2015)
+ *   sites   += 1 where the site's abba + baba term is > 0
+ * d = (abba - baba) / (abba + baba) (Patterson's D), fd = (abba - baba) / fd_den, fdm = (abba - baba) / fdm_den, each
+ * as (double) numerator / (double) denominator and NaN where the denominator is 0.  f_d is meant to be read where D > 0.
+ * |fdm| <= 1, and swapping P1 and P2 negates d and fdm exactly.                                                         */
+typedef struct pb_region_abba {
+    int32_t        n_triples;           /* NT                                                                   */
+    int32_t        outgroup_pop;        /* O                                                                    */
+    const int32_t *triples;             /* [3*NT] P1, P2, P3 of every triple, as the region ran with them       */
+    const int32_t *sites;               /* sites with abba + baba > 0                                           */
+    const int64_t *abba, *baba;         /* window sums on the scale K                                           */
+    const int64_t *fd_den, *fdm_den;
+    const double  *d, *fd, *fdm;
+} pb_region_abba;
+
 typedef struct pb_ctx pb_ctx;
 
 /* ---- life cycle ---------------------------------------------------------------------- */
@@ -272,6 +303,13 @@ int pb_region_get_fst(const pb_ctx *ctx, pb_region_fst *out);
  * permutation), so the result does not depend on how a contig is cut into regions or spread over GPUs.  The generator is
  * written down in popbam_b200/csrc/pb_stats.cuh (k_snn_perm).  PB_ERR_ARG if n_perms < 0 or > 2^31 - 1.                */
 int pb_set_snn_perms(pb_ctx *ctx, int64_t n_perms, uint64_t seed);
+/* The PB_AN_ABBA arrays of the region pb_region_end / pb_region_wait returned last.                                  */
+int pb_region_get_abba(const pb_ctx *ctx, pb_region_abba *out);
+/* Triples (P1, P2, P3) and the outgroup population O of the PB_AN_ABBA regions that follow; `triples` holds 3*n_triples
+ * population indices.  A region keeps the list it began with (pb_region_relaunch too).  n_triples = 0 clears the list;
+ * pb_region_begin with PB_AN_ABBA and no list is PB_ERR_STATE.  PB_ERR_ARG for an index outside [0, n_pops), a
+ * population repeated within (P1, P2, P3, O), or n_triples < 0 or > PB_MAX_ABBA_TRIPLES.                             */
+int pb_set_abba(pb_ctx *ctx, int32_t outgroup_pop, int32_t n_triples, const int32_t *triples);
 
 /* Asynchronous split of pb_region_end for overlap / device timing: launch enqueues every
  * kernel and the result copies on the context's stream; wait blocks and fills *out.       */
@@ -343,6 +381,12 @@ int64_t pb_format_window_ext(const pb_ctx *ctx, const pb_region_result *res, con
  * `ext` may be NULL without PB_AN_THETA_W, `fst` without PB_AN_FST.                                                   */
 int64_t pb_format_window_fst(const pb_ctx *ctx, const pb_region_result *res, const pb_region_extras *ext, const pb_region_fst *fst,
                              int32_t window, uint32_t analysis, const pb_print_opts *opts, char *buf, int64_t cap);
+/* One row of `popbam abba`: chrom, begin + 1, end + 1 and num_sites as nucdiv's row starts, then per triple in list order,
+ * labelled A-B-C from pop_names: S[A-B-C] (sites), ABBA[A-B-C] and BABA[A-B-C] (abba / K and baba / K, the window sums
+ * of the frequency products), D[A-B-C], fd[A-B-C] and fdM[A-B-C]; every floating column is NA where the window has
+ * fewer than min_sites sites or the value is NaN.                                                                     */
+int64_t pb_format_window_abba(const pb_ctx *ctx, const pb_region_result *res, const pb_region_abba *abba, int32_t window,
+                              const pb_print_opts *opts, char *buf, int64_t cap);
 
 #ifdef __cplusplus
 }

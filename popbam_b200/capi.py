@@ -11,13 +11,14 @@ MAXS = 64
 
 AN = dict(NUCDIV=0x001, SFS=0x002, LD_ZNS=0x004, LD_OMEGA=0x008, LD_WALL=0x010, DIVERGE_IND=0x020,
           DIVERGE_POP=0x040, HAPLO_K=0x080, HAPLO_EHHS=0x100, HAPLO_DXY=0x200, SNP=0x400, TREE=0x800,
-          THETA_W=0x1000, FULI=0x2000, LD_DPRIME=0x4000, FST=0x8000)
+          THETA_W=0x1000, FULI=0x2000, LD_DPRIME=0x4000, FST=0x8000, ABBA=0x10000)
 FLAG = dict(ILLUMINA=0x02, SUBSTITUTE=0x10, HETEROZYGOTE=0x20, OUTGROUP=0x40, EMIT_CB=0x10000)
 
 EXPORTS = ["pb_create", "pb_destroy", "pb_last_error", "pb_version", "pb_set_contig", "pb_region_begin", "pb_push_batch", "pb_push_batch_async",
            "pb_push_record", "pb_region_reserve", "pb_region_end", "pb_region_launch", "pb_region_wait", "pb_region_relaunch", "pb_stream",
            "pb_kernel_launches", "pb_region_path", "pb_region_reruns", "pb_stage_times", "pb_window_grid", "pb_build_errmod_tables", "pb_errmod_tables_cached", "pb_errmod_tables_cached_ex", "pb_host_alloc", "pb_host_free", "pb_format_window",
-           "pb_region_get_extras", "pb_format_window_ext", "pb_region_get_fst", "pb_set_snn_perms", "pb_format_window_fst"]
+           "pb_region_get_extras", "pb_format_window_ext", "pb_region_get_fst", "pb_set_snn_perms", "pb_format_window_fst",
+           "pb_region_get_abba", "pb_set_abba", "pb_format_window_abba"]
 
 
 def _p(t):
@@ -79,6 +80,13 @@ class Fst(C.Structure):
     _fields_ = [("hud_num", _p(C.c_int64)), ("hud_den", _p(C.c_int64)), ("wc_num", _p(C.c_int64)), ("wc_den", _p(C.c_int64)),
                 ("fst_hudson", _p(C.c_double)), ("fst_wc", _p(C.c_double)), ("snn", _p(C.c_double)), ("snn_p", _p(C.c_double)),
                 ("snn_ge", _p(C.c_int64))]
+
+
+class Abba(C.Structure):
+    """pb_region_abba: the PB_AN_ABBA arrays, [NW*NT] each, index w*NT + t, and the triples the region ran with."""
+    _fields_ = [("n_triples", C.c_int32), ("outgroup_pop", C.c_int32), ("triples", _p(C.c_int32)), ("sites", _p(C.c_int32)),
+                ("abba", _p(C.c_int64)), ("baba", _p(C.c_int64)), ("fd_den", _p(C.c_int64)), ("fdm_den", _p(C.c_int64)),
+                ("d", _p(C.c_double)), ("fd", _p(C.c_double)), ("fdm", _p(C.c_double))]
 
 
 class PrintOpts(C.Structure):
@@ -152,6 +160,10 @@ def lib():
         L.pb_format_window_fst.restype = C.c_int64
         L.pb_format_window_fst.argtypes = [C.c_void_p, _p(Result), _p(Extras), _p(Fst), C.c_int32, C.c_uint32, _p(PrintOpts), C.c_char_p,
                                            C.c_int64]
+        L.pb_region_get_abba.argtypes = [C.c_void_p, _p(Abba)]
+        L.pb_set_abba.argtypes = [C.c_void_p, C.c_int32, C.c_int32, _p(C.c_int32)]
+        L.pb_format_window_abba.restype = C.c_int64
+        L.pb_format_window_abba.argtypes = [C.c_void_p, _p(Result), _p(Abba), C.c_int32, _p(PrintOpts), C.c_char_p, C.c_int64]
         _lib = L
     return _lib
 
@@ -177,6 +189,7 @@ class Context:
         self.res = Result()
         self.ext = Extras()
         self.fst = Fst()
+        self.abba = Abba()
 
     def _chk(self, rc):
         if rc != 0:
@@ -212,6 +225,7 @@ class Context:
         self._chk(self.L.pb_region_end(self.h, C.byref(self.res)))
         self._chk(self.L.pb_region_get_extras(self.h, C.byref(self.ext)))
         self._chk(self.L.pb_region_get_fst(self.h, C.byref(self.fst)))
+        self._chk(self.L.pb_region_get_abba(self.h, C.byref(self.abba)))
         return self.res
 
     def launch(self):
@@ -224,11 +238,17 @@ class Context:
         self._chk(self.L.pb_region_wait(self.h, C.byref(self.res)))
         self._chk(self.L.pb_region_get_extras(self.h, C.byref(self.ext)))
         self._chk(self.L.pb_region_get_fst(self.h, C.byref(self.fst)))
+        self._chk(self.L.pb_region_get_abba(self.h, C.byref(self.abba)))
         return self.res
 
     def set_snn_perms(self, n_perms, seed=0):
         """Snn permutations per (window, population pair) for the regions that follow (PB_AN_FST); 0 = none."""
         self._chk(self.L.pb_set_snn_perms(self.h, n_perms, seed))
+
+    def set_abba(self, outgroup_pop, triples):
+        """Triples [(P1, P2, P3), ...] against population outgroup_pop for the PB_AN_ABBA regions that follow; [] clears them."""
+        flat = np.ascontiguousarray([k for t in triples for k in t], dtype=np.int32)
+        self._chk(self.L.pb_set_abba(self.h, outgroup_pop, len(flat) // 3, flat.ctypes.data_as(_p(C.c_int32)) if len(flat) else None))
 
     def stage_times(self):
         ms = (C.c_double * 4)()
@@ -250,6 +270,8 @@ class Context:
         buf = C.create_string_buffer(1 << 20)
 
         def fmt(w, buf):
+            if analysis & AN["ABBA"]:
+                return self.L.pb_format_window_abba(self.h, C.byref(self.res), C.byref(self.abba), w, C.byref(opts), buf, len(buf))
             if analysis & AN["FST"]:
                 return self.L.pb_format_window_fst(self.h, C.byref(self.res), C.byref(self.ext), C.byref(self.fst), w, analysis, C.byref(opts),
                                                    buf, len(buf))

@@ -34,6 +34,16 @@ struct Out {
         if (ok) f("\t%s[%s]:\t%.5f", name, label, v);
         else f("\t%s[%s]:\t%7s", name, label, "NA");
     }
+    // the text into buf (NUL-terminated, cut to cap - 1 bytes); returns its full length
+    int64_t copy_to(char *buf, int64_t cap) const {
+        const int64_t len = (int64_t)s.size();
+        if (buf && cap > 0) {
+            const int64_t k = std::min<int64_t>(len, cap - 1);
+            memcpy(buf, s.data(), (size_t)k);
+            buf[k] = 0;
+        }
+        return len;
+    }
 };
 
 // bam_nt16_table followed by bam_nt16_rev_table (popbam.cpp:13-31, bam.h): the letter the reference
@@ -346,13 +356,7 @@ int64_t format_window(const pb_ctx *ctx, const pb_region_result *r, const pb_reg
         out.f("\n");
         }
     }
-    const int64_t len = (int64_t)out.s.size();
-    if (buf && cap > 0) {
-        const int64_t k = std::min<int64_t>(len, cap - 1);
-        memcpy(buf, out.s.data(), (size_t)k);
-        buf[k] = 0;
-    }
-    return len;
+    return out.copy_to(buf, cap);
 }
 
 }  // namespace
@@ -374,4 +378,35 @@ extern "C" int64_t pb_format_window_fst(const pb_ctx *ctx, const pb_region_resul
     if ((an & ~(PB_AN_THETA_W | PB_AN_FST)) != PB_AN_NUCDIV) return PB_ERR_ARG;
     if ((an & PB_AN_FST) && (!f || !f->fst_hudson || !f->fst_wc || !f->snn)) return PB_ERR_ARG;
     return format_window(ctx, r, e, f, w, an, o, buf, cap);
+}
+
+extern "C" int64_t pb_format_window_abba(const pb_ctx *ctx, const pb_region_result *r, const pb_region_abba *a, int32_t w,
+                                         const pb_print_opts *o, char *buf, int64_t cap) {
+    const pb_params *p = pb_ctx_params(ctx);
+    if (!p || !r || !a || !o || w < 0 || w >= r->n_windows || !(r->analyses & PB_AN_ABBA)) return PB_ERR_ARG;
+    if (a->n_triples < 1 || !a->triples || !a->sites || !a->abba || !a->baba || !a->d || !a->fd || !a->fdm) return PB_ERR_ARG;
+    const int NT = a->n_triples, og = a->outgroup_pop;
+    if (og < 0 || og >= r->n_pops) return PB_ERR_ARG;
+    Out out;
+    const int ns = r->num_sites[w];
+    const bool ok = ns >= o->min_sites;
+    out.f("%s\t%d\t%d\t%d", o->chrom, r->win_beg[w] + 1, r->win_end[w] + 1, ns);
+    char nm[600];
+    for (int t = 0; t < NT; ++t) {
+        const int32_t *k = a->triples + 3 * t;
+        if (k[0] < 0 || k[0] >= r->n_pops || k[1] < 0 || k[1] >= r->n_pops || k[2] < 0 || k[2] >= r->n_pops) return PB_ERR_ARG;
+        snprintf(nm, sizeof nm, "%s-%s-%s", o->pop_names[k[0]], o->pop_names[k[1]], o->pop_names[k[2]]);
+        // ABBA and BABA as sums of frequency products: the integer sums over K = n1^2 n2^2 n3^2 n4
+        const int64_t n1 = p->pop_nsmpl[k[0]], n2 = p->pop_nsmpl[k[1]], n3 = p->pop_nsmpl[k[2]], n4 = p->pop_nsmpl[og];
+        const double K = (double)(n1 * n1 * n2 * n2 * n3 * n3 * n4);
+        const size_t x = (size_t)w * NT + t;
+        out.f("\tS[%s]:\t%d", nm, a->sites[x]);
+        out.stat("ABBA", nm, ok, (double)a->abba[x] / K);
+        out.stat("BABA", nm, ok, (double)a->baba[x] / K);
+        out.stat("D", nm, ok && !std::isnan(a->d[x]), a->d[x]);
+        out.stat("fd", nm, ok && !std::isnan(a->fd[x]), a->fd[x]);
+        out.stat("fdM", nm, ok && !std::isnan(a->fdm[x]), a->fdm[x]);
+    }
+    out.f("\n");
+    return out.copy_to(buf, cap);
 }

@@ -17,6 +17,7 @@
 #include "pb_pile.cuh"
 #include "pb_stats.cuh"
 #include "pb_ld.cuh"
+#include "pb_abba.cuh"
 
 namespace {
 
@@ -95,8 +96,14 @@ struct pb_ctx {
     int64_t snn_perms = 0;                 // pb_set_snn_perms: Snn permutations per (window, pair) and the stream's seed
     uint64_t snn_seed = 0;
     int64_t snn_perms_run = 0;             // ... as the last pipeline run used them
+    std::vector<int32_t> abba_set;         // pb_set_abba: P1, P2, P3 of every triple, and the outgroup population
+    int32_t abba_og = -1;
+    std::vector<int32_t> abba_run;         // ... as the open region took them at pb_region_begin (relaunches keep them)
+    int32_t abba_run_og = -1;
+    std::vector<PbAbbaTriple> abba_tri;    // their per-triple constants, copied to d_abba_tri
+    DevBuf d_abba_tri, d_abba;             // the constants; the PB_AN_ABBA result arena (abba_layout)
     // pinned results
-    HostBuf h_ctr, h_small, h_seg, h_span;
+    HostBuf h_ctr, h_small, h_seg, h_span, h_abba;
     PbCounters ctr_host;
     bool need_valid = false;
     int need_nl = 0;
@@ -105,6 +112,7 @@ struct pb_ctx {
     pb_region_result res;
     pb_region_extras ext;
     pb_region_fst fst;
+    pb_region_abba abba;
     // bam_fetch_f shim staging (pb_push_record)
     std::vector<int32_t> r_pos;
     std::vector<uint32_t> r_meta, r_cig_off, r_cigar, r_base_off;
@@ -224,6 +232,21 @@ SmallLayout small_layout(void *base, int NW, int P, int n, bool with_tree, bool 
         L.fst_hudson = cv.take<double>(wpp); L.fst_wc = cv.take<double>(wpp); L.snn = cv.take<double>(wpp); L.snn_p = cv.take<double>(wpp);
         L.snn_ge = cv.take<int64_t>(wpp);
     }
+    L.bytes = (cv.off + 255) & ~(size_t)255;
+    return L;
+}
+// the PB_AN_ABBA arrays, [NW*NT] each: an arena of their own, so the small-result arena is the same with or without them
+struct AbbaLayout {
+    int32_t *sites; int64_t *abba, *baba, *fd_den, *fdm_den; double *d, *fd, *fdm;
+    size_t bytes;
+};
+AbbaLayout abba_layout(void *base, int NW, int NT) {
+    Carver cv(base);
+    AbbaLayout L;
+    const size_t wt = (size_t)NW * NT;
+    L.sites = cv.take<int32_t>(wt);
+    L.abba = cv.take<int64_t>(wt); L.baba = cv.take<int64_t>(wt); L.fd_den = cv.take<int64_t>(wt); L.fdm_den = cv.take<int64_t>(wt);
+    L.d = cv.take<double>(wt); L.fd = cv.take<double>(wt); L.fdm = cv.take<double>(wt);
     L.bytes = (cv.off + 255) & ~(size_t)255;
     return L;
 }
@@ -671,6 +694,23 @@ int run_pipeline(pb_ctx *c, int attempt = 0, bool allow_async = true) {
             PB_CUDA(c, cudaGetLastError());
         }
     }
+    // ---- ABBA-BABA sums per (window, triple)
+    const int NT = (int)c->abba_tri.size();
+    const bool with_abba = (c->analyses & PB_AN_ABBA) != 0;
+    if (with_abba) {
+        const AbbaLayout al0 = abba_layout(nullptr, NW, NT);
+        PB_TRY(dev_reserve(c, c->d_abba, al0.bytes));
+        PB_TRY(host_reserve(c, c->h_abba, al0.bytes));
+        const AbbaLayout al = abba_layout(c->d_abba.p, NW, NT);
+        PbAbbaArgs aa;
+        aa.tri = dp<PbAbbaTriple>(c->d_abba_tri); aa.nt = NT;
+        aa.segsites = dl.segsites; aa.seg_off = dl.seg_off; aa.seg_type = sl.seg_type;
+        aa.sites = al.sites; aa.abba = al.abba; aa.baba = al.baba; aa.fd_den = al.fd_den; aa.fdm_den = al.fdm_den;
+        aa.d = al.d; aa.fd = al.fd; aa.fdm = al.fdm;
+        k_abba<<<dim3((unsigned)NW, (unsigned)((NT + PB_ABBA_WARPS - 1) / PB_ABBA_WARPS)), PB_ABBA_WARPS * 32, 0, st>>>(aa);
+        c->launches += 1;
+        PB_CUDA(c, cudaGetLastError());
+    }
     // ---- pairwise LD (ld -o 0 / -o 1, D'): keep list, tiled pair kernel, finish
     if (c->analyses & (PB_AN_LD_ZNS | PB_AN_LD_OMEGA | PB_AN_LD_DPRIME)) {
         PbLdArgs la;
@@ -709,6 +749,7 @@ int run_pipeline(pb_ctx *c, int attempt = 0, bool allow_async = true) {
 
     // ---- results to pinned host memory
     PB_CUDA(c, cudaMemcpyAsync(c->h_small.p, c->d_stats.p, dl.bytes, cudaMemcpyDeviceToHost, st));
+    if (with_abba) PB_CUDA(c, cudaMemcpyAsync(c->h_abba.p, c->d_abba.p, abba_layout(nullptr, NW, NT).bytes, cudaMemcpyDeviceToHost, st));
     if (!async && S > 0) PB_CUDA(c, cudaMemcpyAsync(c->h_seg.p, c->d_seg_type.p, sl.bytes, cudaMemcpyDeviceToHost, st));
     if (P.flags & PB_FLAG_EMIT_CB) {
         Carver cv(nullptr);
@@ -797,6 +838,14 @@ int fill_result(pb_ctx *c, pb_region_result *out) {
         f.hud_num = hl.hud_num; f.hud_den = hl.hud_den; f.wc_num = hl.wc_num; f.wc_den = hl.wc_den;
         f.fst_hudson = hl.fst_hudson; f.fst_wc = hl.fst_wc; f.snn = hl.snn;
         if (c->snn_perms_run > 0) { f.snn_p = hl.snn_p; f.snn_ge = hl.snn_ge; }
+    }
+    pb_region_abba &ab = c->abba;
+    memset(&ab, 0, sizeof ab);
+    if (an & PB_AN_ABBA) {
+        const AbbaLayout al = abba_layout(c->h_abba.p, NW, (int)c->abba_tri.size());
+        ab.n_triples = (int32_t)c->abba_tri.size(); ab.outgroup_pop = c->abba_run_og; ab.triples = c->abba_run.data();
+        ab.sites = al.sites; ab.abba = al.abba; ab.baba = al.baba; ab.fd_den = al.fd_den; ab.fdm_den = al.fdm_den;
+        ab.d = al.d; ab.fd = al.fd; ab.fdm = al.fdm;
     }
     if (an & PB_AN_DIVERGE_POP) { r.pop_div = hl.pop_div; r.div_num_snps = hl.div_num_snps; }
     if (an & (PB_AN_HAPLO_K | PB_AN_HAPLO_EHHS)) { r.nhaps = hl.nhaps; r.hdiv = hl.hdiv; }
@@ -935,7 +984,7 @@ void pb_destroy(pb_ctx *c) {
     if (c->stream2) cudaStreamSynchronize(c->stream2);
     if (c->stream_lo) cudaStreamSynchronize(c->stream_lo);
     for (DevBuf *b : c->bufs) if (b->p) { cudaFree(b->p); b->p = nullptr; b->cap = 0; }
-    HostBuf *hb[] = {&c->h_ctr, &c->h_small, &c->h_seg, &c->h_span};
+    HostBuf *hb[] = {&c->h_ctr, &c->h_small, &c->h_seg, &c->h_span, &c->h_abba};
     for (HostBuf *b : hb) if (b->p) cudaFreeHost(b->p);
     for (auto &ev : c->ev) if (ev) cudaEventDestroy(ev);
     for (auto &ev : c->fk) if (ev) cudaEventDestroy(ev);
@@ -970,8 +1019,25 @@ int pb_region_begin(pb_ctx *c, uint32_t analyses, int32_t n_windows, const int32
         if (i && win_beg[i] < win_end[i - 1]) return fail(c, PB_ERR_ARG, "windows must be sorted and disjoint (window %d)", i);
     }
     if ((int64_t)win_end[n_windows - 1] - win_beg[0] < 1) return fail(c, PB_ERR_ARG, "empty region");
+    if ((analyses & PB_AN_ABBA) && c->abba_set.empty()) return fail(c, PB_ERR_STATE, "pb_region_begin with PB_AN_ABBA before pb_set_abba");
     PB_CUDA(c, cudaSetDevice(c->prm.device));
     PB_CUDA(c, cudaStreamSynchronize(c->stream));
+    c->abba_run.clear(); c->abba_tri.clear(); c->abba_run_og = -1;
+    if (analyses & PB_AN_ABBA) {       // the triples this region runs with, and their constants on the device
+        const pb_params &P = c->prm;
+        c->abba_run = c->abba_set; c->abba_run_og = c->abba_og;
+        for (size_t t = 0; t < c->abba_run.size(); t += 3) {
+            const int k[4] = {c->abba_run[t], c->abba_run[t + 1], c->abba_run[t + 2], c->abba_og};
+            PbAbbaTriple q;
+            q.m1 = P.pop_mask[k[0]]; q.m2 = P.pop_mask[k[1]]; q.m3 = P.pop_mask[k[2]]; q.m4 = P.pop_mask[k[3]];
+            q.n1 = P.pop_nsmpl[k[0]]; q.n2 = P.pop_nsmpl[k[1]]; q.n3 = P.pop_nsmpl[k[2]]; q.n4 = P.pop_nsmpl[k[3]];
+            const long long n1 = q.n1, n2 = q.n2, n3 = q.n3;
+            q.s_ab = n1 * n2 * n3; q.s_d2 = n1 * n3 * n3; q.s_d3 = n1 * n2 * n2; q.s_m1 = n2 * n3 * n3; q.s_m3 = n1 * n1 * n2;
+            c->abba_tri.push_back(q);
+        }
+        PB_TRY(dev_reserve(c, c->d_abba_tri, sizeof(PbAbbaTriple) * c->abba_tri.size()));
+        PB_CUDA(c, cudaMemcpyAsync(c->d_abba_tri.p, c->abba_tri.data(), sizeof(PbAbbaTriple) * c->abba_tri.size(), cudaMemcpyHostToDevice, c->stream));
+    }
     c->analyses = analyses; c->nw = n_windows;
     c->h_wbeg.assign(win_beg, win_beg + n_windows); c->h_wend.assign(win_end, win_end + n_windows);
     c->span_beg = win_beg[0]; c->span_end = win_end[n_windows - 1];
@@ -1137,6 +1203,32 @@ int pb_set_snn_perms(pb_ctx *c, int64_t n_perms, uint64_t seed) {
     if (!c) return PB_ERR_ARG;
     if (n_perms < 0 || n_perms > 0x7fffffffLL) return fail(c, PB_ERR_ARG, "pb_set_snn_perms: n_perms must be in 0 .. 2^31 - 1");
     c->snn_perms = n_perms; c->snn_seed = seed;
+    return PB_OK;
+}
+
+int pb_region_get_abba(const pb_ctx *c, pb_region_abba *out) {
+    if (!c || !out) return PB_ERR_ARG;
+    *out = c->abba;
+    return PB_OK;
+}
+
+int pb_set_abba(pb_ctx *c, int32_t outgroup_pop, int32_t n_triples, const int32_t *triples) {
+    if (!c) return PB_ERR_ARG;
+    if (n_triples < 0 || n_triples > PB_MAX_ABBA_TRIPLES) return fail(c, PB_ERR_ARG, "pb_set_abba: n_triples must be in 0 .. %d", PB_MAX_ABBA_TRIPLES);
+    if (n_triples == 0) { c->abba_set.clear(); c->abba_og = -1; return PB_OK; }
+    const int P = c->prm.n_pops;
+    if (!triples) return fail(c, PB_ERR_ARG, "pb_set_abba: null triples");
+    if (outgroup_pop < 0 || outgroup_pop >= P) return fail(c, PB_ERR_ARG, "pb_set_abba: outgroup population %d outside 0 .. %d", outgroup_pop, P - 1);
+    for (int t = 0; t < n_triples; ++t) {
+        const int32_t k[4] = {triples[3 * t], triples[3 * t + 1], triples[3 * t + 2], outgroup_pop};
+        for (int i = 0; i < 3; ++i)
+            if (k[i] < 0 || k[i] >= P) return fail(c, PB_ERR_ARG, "pb_set_abba: triple %d: population %d outside 0 .. %d", t, k[i], P - 1);
+        for (int i = 0; i < 4; ++i)
+            for (int j = i + 1; j < 4; ++j)
+                if (k[i] == k[j]) return fail(c, PB_ERR_ARG, "pb_set_abba: triple %d repeats population %d within (P1, P2, P3, O)", t, k[i]);
+    }
+    c->abba_set.assign(triples, triples + 3 * (size_t)n_triples);
+    c->abba_og = outgroup_pop;
     return PB_OK;
 }
 

@@ -16,6 +16,10 @@
 // -p, D; ld -o 0: mean |D'| and the number of SNP pairs in complete LD); for nucdiv only, --fst: F_ST (Hudson, and Weir &
 // Cockerham) and Hudson's Snn for every population pair, after the --extra-stats columns, with --snn-perms N: a permutation
 // p-value of Snn from N random re-partitions of the pair's samples, drawn from a stream seeded by --seed S (default 0).
+//
+// One subcommand the reference does not have: `abba -p SAMPLE`, per window Patterson's D, f_d and f_dM of population
+// triples (P1, P2, P3) against the population of SAMPLE as the outgroup; by default every triple with P1 < P2, or the
+// ones --triple A,B,C names, in the order given.
 #include <algorithm>
 #include <atomic>
 #include <condition_variable>
@@ -53,6 +57,7 @@ struct Options {
     bool fst = false, snn_opts = false;
     long long snn_perms = 0;
     unsigned long long seed = 0;
+    std::vector<std::string> triples;      // abba: --triple A,B,C
     double shard_mb = 2.0;
 };
 
@@ -66,6 +71,7 @@ const CmdSpec kCmds[] = {
     {"haplo", "fhomxqsabkw", "i"},
     {"snp", "fhmxqsabozpw", "vi"},
     {"tree", "fhmxqsabkwd", "i"},      // pop_tree.cpp:601-620
+    {"abba", "fhmxqsabkwp", "i"},      // -p: a sample of the outgroup population (required)
 };
 
 void usage(const char *cmd) {
@@ -76,7 +82,9 @@ void usage(const char *cmd) {
             "         -i Illumina 1.3+ qualities   --gpus N   --shard-mb X   --threads T\n"
             "         --extra-stats  nucdiv: theta[pop]; sfs: FuLiD*[pop] (and FuLiD[pop] with -p); ld -o 0: Dp[pop], Dp1[pop]\n"
             "         --fst  nucdiv: Fst[A-B] (Hudson), FstWC[A-B] (Weir & Cockerham), Snn[A-B] (Hudson's nearest neighbours)\n"
-            "         --snn-perms N  with --fst: SnnP[A-B], p-value of Snn from N permutations   --seed S  their random stream (0)\n", cmd);
+            "         --snn-perms N  with --fst: SnnP[A-B], p-value of Snn from N permutations   --seed S  their random stream (0)\n"
+            "         abba: -p STR a sample of the outgroup population (required)   --triple A,B,C (repeatable) the triples to\n"
+            "         report, in this order (default: every P1 < P2, P3 besides them); columns S, ABBA, BABA, D, fd, fdM [A-B-C]\n", cmd);
 }
 
 Options parse(int argc, char **argv) {
@@ -100,6 +108,7 @@ Options parse(int argc, char **argv) {
                 o.snn_opts = true;
                 continue;
             }
+            if (a == "--triple") { o.triples.push_back(val()); continue; }
             if (a == "--gpus") o.gpus = atoi(val());
             else if (a == "--shard-mb") o.shard_mb = atof(val());
             else if (a == "--threads") o.threads = atoi(val());
@@ -161,6 +170,8 @@ Options parse(int argc, char **argv) {
         fatal("--extra-stats is only available for nucdiv, sfs and ld -o 0");
     if ((o.fst || o.snn_opts) && o.cmd != "nucdiv") fatal("--fst, --snn-perms and --seed are only available for nucdiv");
     if (o.snn_opts && !o.fst) fatal("--snn-perms and --seed go with --fst");
+    if (!o.triples.empty() && o.cmd != "abba") fatal("--triple is only available for abba");
+    if (o.cmd == "abba" && !o.has_p) fatal("abba needs -p SAMPLE: a sample of the outgroup population");
     return o;
 }
 
@@ -190,6 +201,8 @@ struct Run {
     std::vector<Shard> shards;
     pb_params prm;
     uint32_t analysis = 0;
+    int32_t abba_og = -1;                  // abba: the outgroup population and the triples (P1, P2, P3, ...)
+    std::vector<int32_t> abba_triples;
     // error-model tables, built once on the host (while the files are opened) and shared by every context
     std::vector<double> fk, beta, lhet;
     std::shared_future<void> tables_ready;
@@ -297,6 +310,8 @@ void gpu_worker(Run *R, int g, int G, int device) {
     if (!ctx) err = std::string("cannot initialise GPU ") + std::to_string(device) + ": " + pb_last_error(nullptr);
     else if (pb_set_contig(ctx, R->tid, R->ref.data(), (int64_t)R->ref.size()) != PB_OK) err = pb_last_error(ctx);
     else if (pb_set_snn_perms(ctx, R->opt.snn_perms, R->opt.seed) != PB_OK) err = pb_last_error(ctx);
+    else if ((R->analysis & PB_AN_ABBA) &&
+             pb_set_abba(ctx, R->abba_og, (int32_t)(R->abba_triples.size() / 3), R->abba_triples.data()) != PB_OK) err = pb_last_error(ctx);
     std::vector<const char *> pops, smps;
     for (auto &s : R->st.pops) pops.push_back(s.c_str());
     for (auto &s : R->st.samples) smps.push_back(s.c_str());
@@ -317,6 +332,7 @@ void gpu_worker(Run *R, int g, int G, int device) {
             pb_region_result res;
             pb_region_extras ext;
             pb_region_fst fst;
+            pb_region_abba abba;
             int rc = pb_region_begin(ctx, R->analysis, sh.w1 - sh.w0, &R->wb[sh.w0], &R->we[sh.w0]);
             {
                 int64_t nr = 0, nc = 0, nb = 0;
@@ -337,7 +353,9 @@ void gpu_worker(Run *R, int g, int G, int device) {
             if (rc == PB_OK) rc = pb_region_end(ctx, &res);
             if (rc == PB_OK) rc = pb_region_get_extras(ctx, &ext);
             if (rc == PB_OK) rc = pb_region_get_fst(ctx, &fst);
+            if (rc == PB_OK) rc = pb_region_get_abba(ctx, &abba);
             auto format = [&](int w) {
+                if (R->analysis & PB_AN_ABBA) return pb_format_window_abba(ctx, &res, &abba, w, &po, line.data(), (int64_t)line.size());
                 return (R->analysis & PB_AN_FST) ? pb_format_window_fst(ctx, &res, &ext, &fst, w, R->analysis, &po, line.data(), (int64_t)line.size())
                                                  : pb_format_window_ext(ctx, &res, &ext, w, R->analysis, &po, line.data(), (int64_t)line.size());
             };
@@ -359,12 +377,56 @@ void gpu_worker(Run *R, int g, int G, int device) {
     if (ctx) pb_destroy(ctx);
 }
 
+// abba: the outgroup population (that of sample -p) and the triples, from --triple or every P1 < P2, P3 besides them
+void abba_triples(Run &R) {
+    const Options &o = R.opt;
+    const int P = (int)R.st.pops.size();
+    int found = -1;
+    for (int i = 0; i < (int)R.st.samples.size(); ++i) if (R.st.samples[i] == o.outgroup) found = i;   // last match wins, as for sfs
+    if (found < 0) fatal("Specified outgroup " + o.outgroup + " not found");
+    const int og = R.st.sample_pop[found];
+    if (P - 1 < 3)
+        fatal("abba needs at least three populations besides the outgroup's (" + R.st.pops[og] + "); found " + std::to_string(P - 1));
+    R.abba_og = og;
+    std::vector<int32_t> &tr = R.abba_triples;
+    if (o.triples.empty()) {
+        for (int i = 0; i < P; ++i)
+            for (int j = i + 1; j < P; ++j)
+                for (int k = 0; k < P; ++k)
+                    if (i != og && j != og && k != og && k != i && k != j) { tr.push_back(i); tr.push_back(j); tr.push_back(k); }
+        if (tr.size() / 3 > PB_MAX_ABBA_TRIPLES)
+            fatal("abba: the default list has " + std::to_string(tr.size() / 3) + " triples, more than " + std::to_string(PB_MAX_ABBA_TRIPLES) +
+                  "; name the ones to report with --triple A,B,C");
+        return;
+    }
+    if (o.triples.size() > PB_MAX_ABBA_TRIPLES) fatal("abba: more than " + std::to_string(PB_MAX_ABBA_TRIPLES) + " triples given with --triple");
+    for (const std::string &spec : o.triples) {
+        std::vector<std::string> names;
+        std::string cur;
+        for (char ch : spec) {
+            if (ch == ',') { names.push_back(cur); cur.clear(); }
+            else cur += ch;
+        }
+        names.push_back(cur);
+        if (names.size() != 3) fatal("--triple " + spec + ": expected three population names A,B,C");
+        int k[3];
+        for (int i = 0; i < 3; ++i) {
+            k[i] = -1;
+            for (int q = 0; q < P; ++q) if (R.st.pops[q] == names[i]) k[i] = q;
+            if (k[i] < 0) fatal("--triple " + spec + ": unknown population " + names[i]);
+            if (k[i] == og) fatal("--triple " + spec + ": population " + names[i] + " is the outgroup's");
+        }
+        if (k[0] == k[1] || k[0] == k[2] || k[1] == k[2]) fatal("--triple " + spec + ": a population is repeated");
+        tr.insert(tr.end(), k, k + 3);
+    }
+}
+
 }  // namespace
 
 int main(int argc, char **argv) {
     if (argc < 2) {
         fprintf(stderr, "Program: popbam (B200 path; %s)\nUsage:   popbam <command> [options] <in.bam> [region]\n"
-                        "Commands: snp haplo diverge tree nucdiv ld sfs   (and: index <in.bam>)\n", pb_version());
+                        "Commands: snp haplo diverge tree nucdiv ld sfs abba   (and: index <in.bam>)\n", pb_version());
         return 1;
     }
     if (!strcmp(argv[1], "_fetch")) {
@@ -505,10 +567,12 @@ int main(int argc, char **argv) {
     else if (o.cmd == "diverge") R.analysis = o.output == 1 ? PB_AN_DIVERGE_POP : PB_AN_DIVERGE_IND;
     else if (o.cmd == "haplo") R.analysis = o.output == 1 ? PB_AN_HAPLO_EHHS : o.output == 2 ? PB_AN_HAPLO_DXY : PB_AN_HAPLO_K;
     else if (o.cmd == "tree") R.analysis = PB_AN_TREE;
+    else if (o.cmd == "abba") R.analysis = PB_AN_ABBA;
     else R.analysis = PB_AN_SNP;
     if (o.output < 0 || o.output > 2) fatal("invalid output option");
     if (o.extra_stats) R.analysis |= o.cmd == "nucdiv" ? PB_AN_THETA_W : o.cmd == "sfs" ? PB_AN_FULI : PB_AN_LD_DPRIME;
     if (o.fst) R.analysis |= PB_AN_FST;
+    if (o.cmd == "abba") abba_triples(R);
 
     // window grid of the region, then shards = runs of whole windows
     const int64_t nw = pb_window_grid(R.beg, R.end, o.window ? o.win_size : 0, 0, nullptr, nullptr);
