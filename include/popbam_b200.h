@@ -67,6 +67,7 @@ typedef enum pb_status {
 #define PB_AN_LD_DPRIME     0x4000u /* Lewontin's |D'| over the ZnS pairs              (with ld -o 0)         */
 #define PB_AN_FST           0x8000u /* F_ST (Hudson, Weir & Cockerham) and Snn per population pair (with nucdiv) */
 #define PB_AN_ABBA          0x10000u /* ABBA-BABA: Patterson's D, f_d, f_dM per triple (pb_set_abba; alone or with any) */
+#define PB_AN_GARUD         0x20000u /* Garud's H1, H12, H123, H2/H1 per population (alone or with any; haplo --garud) */
 
 #define PB_MAX_ABBA_TRIPLES 1024     /* pb_set_abba: most (P1, P2, P3) triples of one region                        */
 
@@ -252,6 +253,27 @@ typedef struct pb_region_abba {
     const double  *d, *fd, *fdm;
 } pb_region_abba;
 
+/* Garud's haplotype homozygosity statistics (Garud, Messer, Buzbas & Petrov 2015) of every window and population of the
+ * last region (PB_AN_GARUD): a struct of its own, like pb_region_fst, with the same lifetime.  Every array is NULL unless
+ * PB_AN_GARUD was requested.  All arrays [NW*P], index w*P + p; n = pop_nsmpl[p].
+ * Samples i and j of p carry the same haplotype iff bit i equals bit j in every seg_type word of the window (calls count
+ * as haploid, as for pi and dxy; with PB_FLAG_HETEROZYGOTE a heterozygous call counts as derived; no outgroup flip: the
+ * identity does not depend on allele labels).  A site is used only where every sample is covered, so every sample has a
+ * complete haplotype.  The identity classes, sorted by size, are c1 >= c2 >= c3 >= ... (ck = 0 if there are fewer than
+ * k classes; sum ci = n).  With hh = sum ci^2:
+ *   h1   = hh / n^2                                  (H1, the haplotype homozygosity)
+ *   h12  = (hh + 2 c1 c2) / n^2                      (H12: the two most frequent haplotypes pooled)
+ *   h123 = (hh + 2 (c1 c2 + c1 c3 + c2 c3)) / n^2    (H123: the three most frequent pooled)
+ *   h2h1 = (hh - c1^2) / hh                          (H2/H1)
+ * each as (double) integer / (double) integer.  The doubles are NaN if n < 2 (the integers are still filled in).  A
+ * window without segregating sites has one class: H1 = H12 = H123 = 1 and H2/H1 = 0.                                   */
+typedef struct pb_region_garud {
+    const int32_t *n_hap;               /* number of identity classes                                             */
+    const int32_t *c1, *c2, *c3;        /* the three largest class sizes                                          */
+    const int32_t *hh;                  /* sum of the squared class sizes                                         */
+    const double  *h1, *h12, *h123, *h2h1;
+} pb_region_garud;
+
 typedef struct pb_ctx pb_ctx;
 
 /* ---- life cycle ---------------------------------------------------------------------- */
@@ -310,6 +332,8 @@ int pb_region_get_abba(const pb_ctx *ctx, pb_region_abba *out);
  * pb_region_begin with PB_AN_ABBA and no list is PB_ERR_STATE.  PB_ERR_ARG for an index outside [0, n_pops), a
  * population repeated within (P1, P2, P3, O), or n_triples < 0 or > PB_MAX_ABBA_TRIPLES.                             */
 int pb_set_abba(pb_ctx *ctx, int32_t outgroup_pop, int32_t n_triples, const int32_t *triples);
+/* The PB_AN_GARUD arrays of the region pb_region_end / pb_region_wait returned last.                                 */
+int pb_region_get_garud(const pb_ctx *ctx, pb_region_garud *out);
 
 /* Asynchronous split of pb_region_end for overlap / device timing: launch enqueues every
  * kernel and the result copies on the context's stream; wait blocks and fills *out.       */
@@ -387,6 +411,11 @@ int64_t pb_format_window_fst(const pb_ctx *ctx, const pb_region_result *res, con
  * fewer than min_sites sites or the value is NaN.                                                                     */
 int64_t pb_format_window_abba(const pb_ctx *ctx, const pb_region_result *res, const pb_region_abba *abba, int32_t window,
                               const pb_print_opts *opts, char *buf, int64_t cap);
+/* haplo with Garud's H: `analysis` is one PB_AN_HAPLO_* bit OR-ed with PB_AN_GARUD.  The reference's row, then per
+ * population nHap[pop] (%d), H1[pop], H12[pop], H123[pop] and H2H1[pop] (%.5f) before the newline; each is NA where the
+ * window has fewer than min_sites sites or the value is NaN.  The other printers refuse PB_AN_GARUD.                  */
+int64_t pb_format_window_garud(const pb_ctx *ctx, const pb_region_result *res, const pb_region_garud *garud, int32_t window,
+                               uint32_t analysis, const pb_print_opts *opts, char *buf, int64_t cap);
 
 #ifdef __cplusplus
 }

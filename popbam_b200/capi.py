@@ -11,14 +11,14 @@ MAXS = 64
 
 AN = dict(NUCDIV=0x001, SFS=0x002, LD_ZNS=0x004, LD_OMEGA=0x008, LD_WALL=0x010, DIVERGE_IND=0x020,
           DIVERGE_POP=0x040, HAPLO_K=0x080, HAPLO_EHHS=0x100, HAPLO_DXY=0x200, SNP=0x400, TREE=0x800,
-          THETA_W=0x1000, FULI=0x2000, LD_DPRIME=0x4000, FST=0x8000, ABBA=0x10000)
+          THETA_W=0x1000, FULI=0x2000, LD_DPRIME=0x4000, FST=0x8000, ABBA=0x10000, GARUD=0x20000)
 FLAG = dict(ILLUMINA=0x02, SUBSTITUTE=0x10, HETEROZYGOTE=0x20, OUTGROUP=0x40, EMIT_CB=0x10000)
 
 EXPORTS = ["pb_create", "pb_destroy", "pb_last_error", "pb_version", "pb_set_contig", "pb_region_begin", "pb_push_batch", "pb_push_batch_async",
            "pb_push_record", "pb_region_reserve", "pb_region_end", "pb_region_launch", "pb_region_wait", "pb_region_relaunch", "pb_stream",
            "pb_kernel_launches", "pb_region_path", "pb_region_reruns", "pb_stage_times", "pb_window_grid", "pb_build_errmod_tables", "pb_errmod_tables_cached", "pb_errmod_tables_cached_ex", "pb_host_alloc", "pb_host_free", "pb_format_window",
            "pb_region_get_extras", "pb_format_window_ext", "pb_region_get_fst", "pb_set_snn_perms", "pb_format_window_fst",
-           "pb_region_get_abba", "pb_set_abba", "pb_format_window_abba"]
+           "pb_region_get_abba", "pb_set_abba", "pb_format_window_abba", "pb_region_get_garud", "pb_format_window_garud"]
 
 
 def _p(t):
@@ -87,6 +87,12 @@ class Abba(C.Structure):
     _fields_ = [("n_triples", C.c_int32), ("outgroup_pop", C.c_int32), ("triples", _p(C.c_int32)), ("sites", _p(C.c_int32)),
                 ("abba", _p(C.c_int64)), ("baba", _p(C.c_int64)), ("fd_den", _p(C.c_int64)), ("fdm_den", _p(C.c_int64)),
                 ("d", _p(C.c_double)), ("fd", _p(C.c_double)), ("fdm", _p(C.c_double))]
+
+
+class Garud(C.Structure):
+    """pb_region_garud: the PB_AN_GARUD arrays, [NW*P] each, index w*P + p."""
+    _fields_ = [("n_hap", _p(C.c_int32)), ("c1", _p(C.c_int32)), ("c2", _p(C.c_int32)), ("c3", _p(C.c_int32)), ("hh", _p(C.c_int32)),
+                ("h1", _p(C.c_double)), ("h12", _p(C.c_double)), ("h123", _p(C.c_double)), ("h2h1", _p(C.c_double))]
 
 
 class PrintOpts(C.Structure):
@@ -164,6 +170,9 @@ def lib():
         L.pb_set_abba.argtypes = [C.c_void_p, C.c_int32, C.c_int32, _p(C.c_int32)]
         L.pb_format_window_abba.restype = C.c_int64
         L.pb_format_window_abba.argtypes = [C.c_void_p, _p(Result), _p(Abba), C.c_int32, _p(PrintOpts), C.c_char_p, C.c_int64]
+        L.pb_region_get_garud.argtypes = [C.c_void_p, _p(Garud)]
+        L.pb_format_window_garud.restype = C.c_int64
+        L.pb_format_window_garud.argtypes = [C.c_void_p, _p(Result), _p(Garud), C.c_int32, C.c_uint32, _p(PrintOpts), C.c_char_p, C.c_int64]
         _lib = L
     return _lib
 
@@ -190,6 +199,7 @@ class Context:
         self.ext = Extras()
         self.fst = Fst()
         self.abba = Abba()
+        self.garud = Garud()
 
     def _chk(self, rc):
         if rc != 0:
@@ -226,6 +236,7 @@ class Context:
         self._chk(self.L.pb_region_get_extras(self.h, C.byref(self.ext)))
         self._chk(self.L.pb_region_get_fst(self.h, C.byref(self.fst)))
         self._chk(self.L.pb_region_get_abba(self.h, C.byref(self.abba)))
+        self._chk(self.L.pb_region_get_garud(self.h, C.byref(self.garud)))
         return self.res
 
     def launch(self):
@@ -239,6 +250,7 @@ class Context:
         self._chk(self.L.pb_region_get_extras(self.h, C.byref(self.ext)))
         self._chk(self.L.pb_region_get_fst(self.h, C.byref(self.fst)))
         self._chk(self.L.pb_region_get_abba(self.h, C.byref(self.abba)))
+        self._chk(self.L.pb_region_get_garud(self.h, C.byref(self.garud)))
         return self.res
 
     def set_snn_perms(self, n_perms, seed=0):
@@ -272,6 +284,8 @@ class Context:
         def fmt(w, buf):
             if analysis & AN["ABBA"]:
                 return self.L.pb_format_window_abba(self.h, C.byref(self.res), C.byref(self.abba), w, C.byref(opts), buf, len(buf))
+            if analysis & AN["GARUD"]:
+                return self.L.pb_format_window_garud(self.h, C.byref(self.res), C.byref(self.garud), w, analysis, C.byref(opts), buf, len(buf))
             if analysis & AN["FST"]:
                 return self.L.pb_format_window_fst(self.h, C.byref(self.res), C.byref(self.ext), C.byref(self.fst), w, analysis, C.byref(opts),
                                                    buf, len(buf))

@@ -196,15 +196,16 @@ void nj_newick(Out &out, const uint16_t *diff, int T, int num_sites, const pb_pr
 }
 
 // every printer: one reference bit, optionally with its extension, whose columns follow the reference's, and (nucdiv
-// only, checked by pb_format_window_fst) the F_ST columns after those
-int64_t format_window(const pb_ctx *ctx, const pb_region_result *r, const pb_region_extras *e, const pb_region_fst *fs, int32_t w,
-                      uint32_t an, const pb_print_opts *o, char *buf, int64_t cap) {
+// only, checked by pb_format_window_fst) the F_ST columns after those, or (haplo only, checked by pb_format_window_garud)
+// Garud's H columns
+int64_t format_window(const pb_ctx *ctx, const pb_region_result *r, const pb_region_extras *e, const pb_region_fst *fs,
+                      const pb_region_garud *g, int32_t w, uint32_t an, const pb_print_opts *o, char *buf, int64_t cap) {
     const pb_params *p = pb_ctx_params(ctx);
     if (!p || !r || !o || w < 0 || w >= r->n_windows) return PB_ERR_ARG;
     if ((r->analyses & an) != an) return PB_ERR_ARG;
     const uint32_t ext = an & (PB_AN_THETA_W | PB_AN_FULI | PB_AN_LD_DPRIME);
-    const bool with_fst = (an & PB_AN_FST) != 0;
-    an &= ~(ext | PB_AN_FST);
+    const bool with_fst = (an & PB_AN_FST) != 0, with_garud = (an & PB_AN_GARUD) != 0;
+    an &= ~(ext | PB_AN_FST | PB_AN_GARUD);
     if (ext && (!e || ext != (an == PB_AN_NUCDIV ? PB_AN_THETA_W : an == PB_AN_SFS ? PB_AN_FULI : an == PB_AN_LD_ZNS ? PB_AN_LD_DPRIME : 0u)))
         return PB_ERR_ARG;
     Out out;
@@ -353,6 +354,16 @@ int64_t format_window(const pb_ctx *ctx, const pb_region_result *r, const pb_reg
                 out.stat("Snn", nm, ok && !std::isnan(fs->snn[x]), fs->snn[x]);
                 if (fs->snn_p) out.stat("SnnP", nm, ok && !std::isnan(fs->snn_p[x]), fs->snn_p[x]);
             }
+        for (int i = 0; with_garud && i < P; ++i) {
+            const size_t x = wp + i;
+            const char *pn = o->pop_names[i];
+            if (ok) out.f("\tnHap[%s]:\t%d", pn, g->n_hap[x]);
+            else out.f("\tnHap[%s]:\t%7s", pn, "NA");
+            out.stat("H1", pn, ok && !std::isnan(g->h1[x]), g->h1[x]);
+            out.stat("H12", pn, ok && !std::isnan(g->h12[x]), g->h12[x]);
+            out.stat("H123", pn, ok && !std::isnan(g->h123[x]), g->h123[x]);
+            out.stat("H2H1", pn, ok && !std::isnan(g->h2h1[x]), g->h2h1[x]);
+        }
         out.f("\n");
         }
     }
@@ -363,21 +374,21 @@ int64_t format_window(const pb_ctx *ctx, const pb_region_result *r, const pb_reg
 
 extern "C" int64_t pb_format_window(const pb_ctx *ctx, const pb_region_result *r, int32_t w, uint32_t an, const pb_print_opts *o,
                                     char *buf, int64_t cap) {
-    if (an & (PB_AN_THETA_W | PB_AN_FULI | PB_AN_LD_DPRIME | PB_AN_FST)) return PB_ERR_ARG;
-    return format_window(ctx, r, nullptr, nullptr, w, an, o, buf, cap);
+    if (an & (PB_AN_THETA_W | PB_AN_FULI | PB_AN_LD_DPRIME | PB_AN_FST | PB_AN_GARUD)) return PB_ERR_ARG;
+    return format_window(ctx, r, nullptr, nullptr, nullptr, w, an, o, buf, cap);
 }
 
 extern "C" int64_t pb_format_window_ext(const pb_ctx *ctx, const pb_region_result *r, const pb_region_extras *e, int32_t w, uint32_t an,
                                         const pb_print_opts *o, char *buf, int64_t cap) {
-    if (an & PB_AN_FST) return PB_ERR_ARG;
-    return format_window(ctx, r, e, nullptr, w, an, o, buf, cap);
+    if (an & (PB_AN_FST | PB_AN_GARUD)) return PB_ERR_ARG;
+    return format_window(ctx, r, e, nullptr, nullptr, w, an, o, buf, cap);
 }
 
 extern "C" int64_t pb_format_window_fst(const pb_ctx *ctx, const pb_region_result *r, const pb_region_extras *e, const pb_region_fst *f,
                                         int32_t w, uint32_t an, const pb_print_opts *o, char *buf, int64_t cap) {
     if ((an & ~(PB_AN_THETA_W | PB_AN_FST)) != PB_AN_NUCDIV) return PB_ERR_ARG;
     if ((an & PB_AN_FST) && (!f || !f->fst_hudson || !f->fst_wc || !f->snn)) return PB_ERR_ARG;
-    return format_window(ctx, r, e, f, w, an, o, buf, cap);
+    return format_window(ctx, r, e, f, nullptr, w, an, o, buf, cap);
 }
 
 extern "C" int64_t pb_format_window_abba(const pb_ctx *ctx, const pb_region_result *r, const pb_region_abba *a, int32_t w,
@@ -409,4 +420,12 @@ extern "C" int64_t pb_format_window_abba(const pb_ctx *ctx, const pb_region_resu
     }
     out.f("\n");
     return out.copy_to(buf, cap);
+}
+
+extern "C" int64_t pb_format_window_garud(const pb_ctx *ctx, const pb_region_result *r, const pb_region_garud *g, int32_t w, uint32_t an,
+                                          const pb_print_opts *o, char *buf, int64_t cap) {
+    const uint32_t ref = an & ~PB_AN_GARUD;
+    if (!(an & PB_AN_GARUD) || (ref != PB_AN_HAPLO_K && ref != PB_AN_HAPLO_EHHS && ref != PB_AN_HAPLO_DXY)) return PB_ERR_ARG;
+    if (!g || !g->n_hap || !g->h1 || !g->h12 || !g->h123 || !g->h2h1) return PB_ERR_ARG;
+    return format_window(ctx, r, nullptr, nullptr, g, w, an, o, buf, cap);
 }

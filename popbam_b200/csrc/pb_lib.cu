@@ -18,6 +18,7 @@
 #include "pb_stats.cuh"
 #include "pb_ld.cuh"
 #include "pb_abba.cuh"
+#include "pb_garud.cuh"
 
 namespace {
 
@@ -102,8 +103,9 @@ struct pb_ctx {
     int32_t abba_run_og = -1;
     std::vector<PbAbbaTriple> abba_tri;    // their per-triple constants, copied to d_abba_tri
     DevBuf d_abba_tri, d_abba;             // the constants; the PB_AN_ABBA result arena (abba_layout)
+    DevBuf d_garud;                        // the PB_AN_GARUD result arena (garud_layout)
     // pinned results
-    HostBuf h_ctr, h_small, h_seg, h_span, h_abba;
+    HostBuf h_ctr, h_small, h_seg, h_span, h_abba, h_garud;
     PbCounters ctr_host;
     bool need_valid = false;
     int need_nl = 0;
@@ -113,6 +115,7 @@ struct pb_ctx {
     pb_region_extras ext;
     pb_region_fst fst;
     pb_region_abba abba;
+    pb_region_garud garud;
     // bam_fetch_f shim staging (pb_push_record)
     std::vector<int32_t> r_pos;
     std::vector<uint32_t> r_meta, r_cig_off, r_cigar, r_base_off;
@@ -247,6 +250,20 @@ AbbaLayout abba_layout(void *base, int NW, int NT) {
     L.sites = cv.take<int32_t>(wt);
     L.abba = cv.take<int64_t>(wt); L.baba = cv.take<int64_t>(wt); L.fd_den = cv.take<int64_t>(wt); L.fdm_den = cv.take<int64_t>(wt);
     L.d = cv.take<double>(wt); L.fd = cv.take<double>(wt); L.fdm = cv.take<double>(wt);
+    L.bytes = (cv.off + 255) & ~(size_t)255;
+    return L;
+}
+// the PB_AN_GARUD arrays, [NW*P] each: an arena of their own, like abba_layout
+struct GarudLayout {
+    int32_t *n_hap, *c1, *c2, *c3, *hh; double *h1, *h12, *h123, *h2h1;
+    size_t bytes;
+};
+GarudLayout garud_layout(void *base, int NW, int P) {
+    Carver cv(base);
+    GarudLayout L;
+    const size_t wp = (size_t)NW * P;
+    L.n_hap = cv.take<int32_t>(wp); L.c1 = cv.take<int32_t>(wp); L.c2 = cv.take<int32_t>(wp); L.c3 = cv.take<int32_t>(wp); L.hh = cv.take<int32_t>(wp);
+    L.h1 = cv.take<double>(wp); L.h12 = cv.take<double>(wp); L.h123 = cv.take<double>(wp); L.h2h1 = cv.take<double>(wp);
     L.bytes = (cv.off + 255) & ~(size_t)255;
     return L;
 }
@@ -711,6 +728,23 @@ int run_pipeline(pb_ctx *c, int attempt = 0, bool allow_async = true) {
         c->launches += 1;
         PB_CUDA(c, cudaGetLastError());
     }
+    // ---- Garud's H per (window, population)
+    const bool with_garud = (c->analyses & PB_AN_GARUD) != 0;
+    if (with_garud) {
+        const GarudLayout gl0 = garud_layout(nullptr, NW, P.n_pops);
+        PB_TRY(dev_reserve(c, c->d_garud, gl0.bytes));
+        PB_TRY(host_reserve(c, c->h_garud, gl0.bytes));
+        const GarudLayout gl = garud_layout(c->d_garud.p, NW, P.n_pops);
+        PbGarudArgs ga;
+        ga.n = n; ga.P = P.n_pops;
+        for (int i = 0; i < PB_MAX_SAMPLES; ++i) { ga.pop_mask[i] = P.pop_mask[i]; ga.pop_nsmpl[i] = P.pop_nsmpl[i]; }
+        ga.segsites = dl.segsites; ga.seg_off = dl.seg_off; ga.seg_type = sl.seg_type;
+        ga.n_hap = gl.n_hap; ga.c1 = gl.c1; ga.c2 = gl.c2; ga.c3 = gl.c3; ga.hh = gl.hh;
+        ga.h1 = gl.h1; ga.h12 = gl.h12; ga.h123 = gl.h123; ga.h2h1 = gl.h2h1;
+        k_garud<<<NW, PB_GARUD_WARPS * 32, 0, st>>>(ga);
+        c->launches += 1;
+        PB_CUDA(c, cudaGetLastError());
+    }
     // ---- pairwise LD (ld -o 0 / -o 1, D'): keep list, tiled pair kernel, finish
     if (c->analyses & (PB_AN_LD_ZNS | PB_AN_LD_OMEGA | PB_AN_LD_DPRIME)) {
         PbLdArgs la;
@@ -750,6 +784,7 @@ int run_pipeline(pb_ctx *c, int attempt = 0, bool allow_async = true) {
     // ---- results to pinned host memory
     PB_CUDA(c, cudaMemcpyAsync(c->h_small.p, c->d_stats.p, dl.bytes, cudaMemcpyDeviceToHost, st));
     if (with_abba) PB_CUDA(c, cudaMemcpyAsync(c->h_abba.p, c->d_abba.p, abba_layout(nullptr, NW, NT).bytes, cudaMemcpyDeviceToHost, st));
+    if (with_garud) PB_CUDA(c, cudaMemcpyAsync(c->h_garud.p, c->d_garud.p, garud_layout(nullptr, NW, P.n_pops).bytes, cudaMemcpyDeviceToHost, st));
     if (!async && S > 0) PB_CUDA(c, cudaMemcpyAsync(c->h_seg.p, c->d_seg_type.p, sl.bytes, cudaMemcpyDeviceToHost, st));
     if (P.flags & PB_FLAG_EMIT_CB) {
         Carver cv(nullptr);
@@ -846,6 +881,13 @@ int fill_result(pb_ctx *c, pb_region_result *out) {
         ab.n_triples = (int32_t)c->abba_tri.size(); ab.outgroup_pop = c->abba_run_og; ab.triples = c->abba_run.data();
         ab.sites = al.sites; ab.abba = al.abba; ab.baba = al.baba; ab.fd_den = al.fd_den; ab.fdm_den = al.fdm_den;
         ab.d = al.d; ab.fd = al.fd; ab.fdm = al.fdm;
+    }
+    pb_region_garud &g = c->garud;
+    memset(&g, 0, sizeof g);
+    if (an & PB_AN_GARUD) {
+        const GarudLayout gl = garud_layout(c->h_garud.p, NW, P.n_pops);
+        g.n_hap = gl.n_hap; g.c1 = gl.c1; g.c2 = gl.c2; g.c3 = gl.c3; g.hh = gl.hh;
+        g.h1 = gl.h1; g.h12 = gl.h12; g.h123 = gl.h123; g.h2h1 = gl.h2h1;
     }
     if (an & PB_AN_DIVERGE_POP) { r.pop_div = hl.pop_div; r.div_num_snps = hl.div_num_snps; }
     if (an & (PB_AN_HAPLO_K | PB_AN_HAPLO_EHHS)) { r.nhaps = hl.nhaps; r.hdiv = hl.hdiv; }
@@ -984,7 +1026,7 @@ void pb_destroy(pb_ctx *c) {
     if (c->stream2) cudaStreamSynchronize(c->stream2);
     if (c->stream_lo) cudaStreamSynchronize(c->stream_lo);
     for (DevBuf *b : c->bufs) if (b->p) { cudaFree(b->p); b->p = nullptr; b->cap = 0; }
-    HostBuf *hb[] = {&c->h_ctr, &c->h_small, &c->h_seg, &c->h_span, &c->h_abba};
+    HostBuf *hb[] = {&c->h_ctr, &c->h_small, &c->h_seg, &c->h_span, &c->h_abba, &c->h_garud};
     for (HostBuf *b : hb) if (b->p) cudaFreeHost(b->p);
     for (auto &ev : c->ev) if (ev) cudaEventDestroy(ev);
     for (auto &ev : c->fk) if (ev) cudaEventDestroy(ev);
@@ -1209,6 +1251,12 @@ int pb_set_snn_perms(pb_ctx *c, int64_t n_perms, uint64_t seed) {
 int pb_region_get_abba(const pb_ctx *c, pb_region_abba *out) {
     if (!c || !out) return PB_ERR_ARG;
     *out = c->abba;
+    return PB_OK;
+}
+
+int pb_region_get_garud(const pb_ctx *c, pb_region_garud *out) {
+    if (!c || !out) return PB_ERR_ARG;
+    *out = c->garud;
     return PB_OK;
 }
 

@@ -15,7 +15,8 @@
 // reference does not compute, as extra columns after its own (nucdiv: Watterson's theta; sfs: Fu & Li's D* and, with
 // -p, D; ld -o 0: mean |D'| and the number of SNP pairs in complete LD); for nucdiv only, --fst: F_ST (Hudson, and Weir &
 // Cockerham) and Hudson's Snn for every population pair, after the --extra-stats columns, with --snn-perms N: a permutation
-// p-value of Snn from N random re-partitions of the pair's samples, drawn from a stream seeded by --seed S (default 0).
+// p-value of Snn from N random re-partitions of the pair's samples, drawn from a stream seeded by --seed S (default 0); for
+// haplo only (any -o), --garud: Garud's H1, H12, H123 and H2/H1 and the number of distinct haplotypes per population.
 //
 // One subcommand the reference does not have: `abba -p SAMPLE`, per window Patterson's D, f_d and f_dM of population
 // triples (P1, P2, P3) against the population of SAMPLE as the outgroup; by default every triple with P1 < P2, or the
@@ -55,6 +56,7 @@ struct Options {
     int gpus = 1, threads = 0;
     bool extra_stats = false;
     bool fst = false, snn_opts = false;
+    bool garud = false;
     long long snn_perms = 0;
     unsigned long long seed = 0;
     std::vector<std::string> triples;      // abba: --triple A,B,C
@@ -83,6 +85,7 @@ void usage(const char *cmd) {
             "         --extra-stats  nucdiv: theta[pop]; sfs: FuLiD*[pop] (and FuLiD[pop] with -p); ld -o 0: Dp[pop], Dp1[pop]\n"
             "         --fst  nucdiv: Fst[A-B] (Hudson), FstWC[A-B] (Weir & Cockerham), Snn[A-B] (Hudson's nearest neighbours)\n"
             "         --snn-perms N  with --fst: SnnP[A-B], p-value of Snn from N permutations   --seed S  their random stream (0)\n"
+            "         --garud  haplo: nHap[pop] (distinct haplotypes), H1[pop], H12[pop], H123[pop], H2H1[pop] (Garud's H)\n"
             "         abba: -p STR a sample of the outgroup population (required)   --triple A,B,C (repeatable) the triples to\n"
             "         report, in this order (default: every P1 < P2, P3 besides them); columns S, ABBA, BABA, D, fd, fdM [A-B-C]\n", cmd);
 }
@@ -99,6 +102,7 @@ Options parse(int argc, char **argv) {
             auto val = [&]() -> const char * { if (i + 1 >= argc) fatal("missing value for " + a); return argv[++i]; };
             if (a == "--extra-stats") { o.extra_stats = true; continue; }
             if (a == "--fst") { o.fst = true; continue; }
+            if (a == "--garud") { o.garud = true; continue; }
             if (a == "--snn-perms" || a == "--seed") {
                 const char *v = val();
                 char *end = nullptr;
@@ -171,6 +175,7 @@ Options parse(int argc, char **argv) {
     if ((o.fst || o.snn_opts) && o.cmd != "nucdiv") fatal("--fst, --snn-perms and --seed are only available for nucdiv");
     if (o.snn_opts && !o.fst) fatal("--snn-perms and --seed go with --fst");
     if (!o.triples.empty() && o.cmd != "abba") fatal("--triple is only available for abba");
+    if (o.garud && o.cmd != "haplo") fatal("--garud is only available for haplo");
     if (o.cmd == "abba" && !o.has_p) fatal("abba needs -p SAMPLE: a sample of the outgroup population");
     return o;
 }
@@ -333,6 +338,7 @@ void gpu_worker(Run *R, int g, int G, int device) {
             pb_region_extras ext;
             pb_region_fst fst;
             pb_region_abba abba;
+            pb_region_garud garud;
             int rc = pb_region_begin(ctx, R->analysis, sh.w1 - sh.w0, &R->wb[sh.w0], &R->we[sh.w0]);
             {
                 int64_t nr = 0, nc = 0, nb = 0;
@@ -354,8 +360,10 @@ void gpu_worker(Run *R, int g, int G, int device) {
             if (rc == PB_OK) rc = pb_region_get_extras(ctx, &ext);
             if (rc == PB_OK) rc = pb_region_get_fst(ctx, &fst);
             if (rc == PB_OK) rc = pb_region_get_abba(ctx, &abba);
+            if (rc == PB_OK) rc = pb_region_get_garud(ctx, &garud);
             auto format = [&](int w) {
                 if (R->analysis & PB_AN_ABBA) return pb_format_window_abba(ctx, &res, &abba, w, &po, line.data(), (int64_t)line.size());
+                if (R->analysis & PB_AN_GARUD) return pb_format_window_garud(ctx, &res, &garud, w, R->analysis, &po, line.data(), (int64_t)line.size());
                 return (R->analysis & PB_AN_FST) ? pb_format_window_fst(ctx, &res, &ext, &fst, w, R->analysis, &po, line.data(), (int64_t)line.size())
                                                  : pb_format_window_ext(ctx, &res, &ext, w, R->analysis, &po, line.data(), (int64_t)line.size());
             };
@@ -572,6 +580,7 @@ int main(int argc, char **argv) {
     if (o.output < 0 || o.output > 2) fatal("invalid output option");
     if (o.extra_stats) R.analysis |= o.cmd == "nucdiv" ? PB_AN_THETA_W : o.cmd == "sfs" ? PB_AN_FULI : PB_AN_LD_DPRIME;
     if (o.fst) R.analysis |= PB_AN_FST;
+    if (o.garud) R.analysis |= PB_AN_GARUD;
     if (o.cmd == "abba") abba_triples(R);
 
     // window grid of the region, then shards = runs of whole windows
