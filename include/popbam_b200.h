@@ -68,8 +68,11 @@ typedef enum pb_status {
 #define PB_AN_FST           0x8000u /* F_ST (Hudson, Weir & Cockerham) and Snn per population pair (with nucdiv) */
 #define PB_AN_ABBA          0x10000u /* ABBA-BABA: Patterson's D, f_d, f_dM per triple (pb_set_abba; alone or with any) */
 #define PB_AN_GARUD         0x20000u /* Garud's H1, H12, H123, H2/H1 per population (alone or with any; haplo --garud) */
+#define PB_AN_SPECTRUM      0x40000u /* unfolded site frequency spectra of 1-3 populations (pb_set_spectra; alone or with any; sfs --jsfs) */
 
 #define PB_MAX_ABBA_TRIPLES 1024     /* pb_set_abba: most (P1, P2, P3) triples of one region                        */
+#define PB_MAX_SPECTRUM_SETS 4096    /* pb_set_spectra: most spectrum sets of one region                            */
+#define PB_MAX_SPECTRUM_BINS 65536   /* pb_set_spectra: most bins per window over all sets                          */
 
 /* Run parameters == the fields of popbamData the hot path reads (popbam.h:218-265) plus
  * the population tables assign_pops builds (popbam.cpp:145-171).                           */
@@ -274,6 +277,25 @@ typedef struct pb_region_garud {
     const double  *h1, *h12, *h123, *h2h1;
 } pb_region_garud;
 
+/* Site frequency spectra of every window of the last region (PB_AN_SPECTRUM, pb_set_spectra): a struct of its own, like
+ * pb_region_garud, with the same lifetime.  Every array is NULL (and n_sets, n_bins 0) unless PB_AN_SPECTRUM was requested.
+ * A spectrum set is an ordered tuple of 1, 2 or 3 distinct populations (P1[, P2[, P3]]), n_k = pop_nsmpl[P_k].  The
+ * spectrum counts the sites the window counts in num_sites (every sample covered: no missing data, no projection).  Per
+ * site a_k = popcount(seg_type & pop_mask[P_k]) (calls count as haploid, as for pi, dxy and the sfs pass; with
+ * PB_FLAG_HETEROZYGOTE a heterozygous call counts as derived).  Polarisation is the sfs pass's: with PB_FLAG_OUTGROUP, if
+ * sample outidx carries the derived allele every a_k becomes n_k - a_k; otherwise "derived" is "not the reference base".
+ * The spectra are unfolded.  The site goes to bin (a1, a2, a3), row-major with the last population fastest, prod (n_k + 1)
+ * bins per set; the num_sites - segsites sites without a segregating call go to the all-zero bin, so a window's set sums
+ * to num_sites.  For a one-population set, bins 0 < j <= n equal the sfs pass's spectrum and bin 0 is its bin 0 plus
+ * num_sites - segsites; the sum over 0 < j < n is sfs_num_snps.                                                         */
+typedef struct pb_region_spectrum {
+    int32_t        n_sets;              /* NS                                                                   */
+    int32_t        n_bins;              /* B: bins per window over all sets                                     */
+    const int32_t *sets;                /* [3*NS] population indices, -1 in unused slots, as the region ran     */
+    const int32_t *set_off;             /* [NS+1] first bin of each set within a window's B                     */
+    const int32_t *counts;              /* [NW*B] index w*B + set_off[s] + bin                                  */
+} pb_region_spectrum;
+
 typedef struct pb_ctx pb_ctx;
 
 /* ---- life cycle ---------------------------------------------------------------------- */
@@ -334,6 +356,14 @@ int pb_region_get_abba(const pb_ctx *ctx, pb_region_abba *out);
 int pb_set_abba(pb_ctx *ctx, int32_t outgroup_pop, int32_t n_triples, const int32_t *triples);
 /* The PB_AN_GARUD arrays of the region pb_region_end / pb_region_wait returned last.                                 */
 int pb_region_get_garud(const pb_ctx *ctx, pb_region_garud *out);
+/* The PB_AN_SPECTRUM arrays of the region pb_region_end / pb_region_wait returned last.                              */
+int pb_region_get_spectrum(const pb_ctx *ctx, pb_region_spectrum *out);
+/* Spectrum sets of the PB_AN_SPECTRUM regions that follow; `sets` holds 3*n_sets population indices, -1 in the unused
+ * trailing slots of a one- or two-population set.  A region keeps the list it began with (pb_region_relaunch too).
+ * n_sets = 0 clears the list; pb_region_begin with PB_AN_SPECTRUM and no list is PB_ERR_STATE.  PB_ERR_ARG for an index
+ * outside [0, n_pops), a population repeated within a set, an empty set, a -1 before a valid index, n_sets < 0 or
+ * > PB_MAX_SPECTRUM_SETS, or more than PB_MAX_SPECTRUM_BINS bins per window over all sets.                           */
+int pb_set_spectra(pb_ctx *ctx, int32_t n_sets, const int32_t *sets);
 
 /* Asynchronous split of pb_region_end for overlap / device timing: launch enqueues every
  * kernel and the result copies on the context's stream; wait blocks and fills *out.       */
@@ -416,6 +446,14 @@ int64_t pb_format_window_abba(const pb_ctx *ctx, const pb_region_result *res, co
  * window has fewer than min_sites sites or the value is NaN.  The other printers refuse PB_AN_GARUD.                  */
 int64_t pb_format_window_garud(const pb_ctx *ctx, const pb_region_result *res, const pb_region_garud *garud, int32_t window,
                                uint32_t analysis, const pb_print_opts *opts, char *buf, int64_t cap);
+/* One spectrum set (set3: 3 population indices, -1 in unused trailing slots) in the text format of dadi's
+ * Spectrum.from_file: `# <comment>` (each line of `comment` behind "# "; none when NULL), the shape line
+ * `n1+1 [n2+1 [n3+1]] unfolded "A" ["B" ["C"]]` (names from opts->pop_names), the prod (n_k + 1) counts (row-major, the
+ * last population fastest) on one line separated by single spaces, and the mask line: 1 at the all-zero and the
+ * all-derived bin, 0 elsewhere.  Returns bytes written (excluding NUL) or the required size if it exceeds cap;
+ * PB_ERR_ARG for a set pb_set_spectra would refuse.                                                                    */
+int64_t pb_format_spectrum_dadi(const pb_ctx *ctx, const int32_t *set3, const int64_t *counts, const pb_print_opts *opts,
+                                const char *comment, char *buf, int64_t cap);
 
 #ifdef __cplusplus
 }

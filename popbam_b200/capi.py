@@ -11,14 +11,15 @@ MAXS = 64
 
 AN = dict(NUCDIV=0x001, SFS=0x002, LD_ZNS=0x004, LD_OMEGA=0x008, LD_WALL=0x010, DIVERGE_IND=0x020,
           DIVERGE_POP=0x040, HAPLO_K=0x080, HAPLO_EHHS=0x100, HAPLO_DXY=0x200, SNP=0x400, TREE=0x800,
-          THETA_W=0x1000, FULI=0x2000, LD_DPRIME=0x4000, FST=0x8000, ABBA=0x10000, GARUD=0x20000)
+          THETA_W=0x1000, FULI=0x2000, LD_DPRIME=0x4000, FST=0x8000, ABBA=0x10000, GARUD=0x20000, SPECTRUM=0x40000)
 FLAG = dict(ILLUMINA=0x02, SUBSTITUTE=0x10, HETEROZYGOTE=0x20, OUTGROUP=0x40, EMIT_CB=0x10000)
 
 EXPORTS = ["pb_create", "pb_destroy", "pb_last_error", "pb_version", "pb_set_contig", "pb_region_begin", "pb_push_batch", "pb_push_batch_async",
            "pb_push_record", "pb_region_reserve", "pb_region_end", "pb_region_launch", "pb_region_wait", "pb_region_relaunch", "pb_stream",
            "pb_kernel_launches", "pb_region_path", "pb_region_reruns", "pb_stage_times", "pb_window_grid", "pb_build_errmod_tables", "pb_errmod_tables_cached", "pb_errmod_tables_cached_ex", "pb_host_alloc", "pb_host_free", "pb_format_window",
            "pb_region_get_extras", "pb_format_window_ext", "pb_region_get_fst", "pb_set_snn_perms", "pb_format_window_fst",
-           "pb_region_get_abba", "pb_set_abba", "pb_format_window_abba", "pb_region_get_garud", "pb_format_window_garud"]
+           "pb_region_get_abba", "pb_set_abba", "pb_format_window_abba", "pb_region_get_garud", "pb_format_window_garud",
+           "pb_region_get_spectrum", "pb_set_spectra", "pb_format_spectrum_dadi"]
 
 
 def _p(t):
@@ -93,6 +94,12 @@ class Garud(C.Structure):
     """pb_region_garud: the PB_AN_GARUD arrays, [NW*P] each, index w*P + p."""
     _fields_ = [("n_hap", _p(C.c_int32)), ("c1", _p(C.c_int32)), ("c2", _p(C.c_int32)), ("c3", _p(C.c_int32)), ("hh", _p(C.c_int32)),
                 ("h1", _p(C.c_double)), ("h12", _p(C.c_double)), ("h123", _p(C.c_double)), ("h2h1", _p(C.c_double))]
+
+
+class Spectrum(C.Structure):
+    """pb_region_spectrum: the PB_AN_SPECTRUM arrays; counts [NW*n_bins], index w*n_bins + set_off[s] + bin."""
+    _fields_ = [("n_sets", C.c_int32), ("n_bins", C.c_int32), ("sets", _p(C.c_int32)), ("set_off", _p(C.c_int32)),
+                ("counts", _p(C.c_int32))]
 
 
 class PrintOpts(C.Structure):
@@ -173,6 +180,10 @@ def lib():
         L.pb_region_get_garud.argtypes = [C.c_void_p, _p(Garud)]
         L.pb_format_window_garud.restype = C.c_int64
         L.pb_format_window_garud.argtypes = [C.c_void_p, _p(Result), _p(Garud), C.c_int32, C.c_uint32, _p(PrintOpts), C.c_char_p, C.c_int64]
+        L.pb_region_get_spectrum.argtypes = [C.c_void_p, _p(Spectrum)]
+        L.pb_set_spectra.argtypes = [C.c_void_p, C.c_int32, _p(C.c_int32)]
+        L.pb_format_spectrum_dadi.restype = C.c_int64
+        L.pb_format_spectrum_dadi.argtypes = [C.c_void_p, _p(C.c_int32), _p(C.c_int64), _p(PrintOpts), C.c_char_p, C.c_char_p, C.c_int64]
         _lib = L
     return _lib
 
@@ -200,6 +211,7 @@ class Context:
         self.fst = Fst()
         self.abba = Abba()
         self.garud = Garud()
+        self.spectrum = Spectrum()
 
     def _chk(self, rc):
         if rc != 0:
@@ -237,6 +249,7 @@ class Context:
         self._chk(self.L.pb_region_get_fst(self.h, C.byref(self.fst)))
         self._chk(self.L.pb_region_get_abba(self.h, C.byref(self.abba)))
         self._chk(self.L.pb_region_get_garud(self.h, C.byref(self.garud)))
+        self._chk(self.L.pb_region_get_spectrum(self.h, C.byref(self.spectrum)))
         return self.res
 
     def launch(self):
@@ -251,6 +264,7 @@ class Context:
         self._chk(self.L.pb_region_get_fst(self.h, C.byref(self.fst)))
         self._chk(self.L.pb_region_get_abba(self.h, C.byref(self.abba)))
         self._chk(self.L.pb_region_get_garud(self.h, C.byref(self.garud)))
+        self._chk(self.L.pb_region_get_spectrum(self.h, C.byref(self.spectrum)))
         return self.res
 
     def set_snn_perms(self, n_perms, seed=0):
@@ -261,6 +275,11 @@ class Context:
         """Triples [(P1, P2, P3), ...] against population outgroup_pop for the PB_AN_ABBA regions that follow; [] clears them."""
         flat = np.ascontiguousarray([k for t in triples for k in t], dtype=np.int32)
         self._chk(self.L.pb_set_abba(self.h, outgroup_pop, len(flat) // 3, flat.ctypes.data_as(_p(C.c_int32)) if len(flat) else None))
+
+    def set_spectra(self, sets):
+        """Spectrum sets [(P1,), (P1, P2), (P1, P2, P3), ...] for the PB_AN_SPECTRUM regions that follow; [] clears them."""
+        flat = np.ascontiguousarray([k for t in sets for k in (list(t) + [-1, -1])[:3]], dtype=np.int32)
+        self._chk(self.L.pb_set_spectra(self.h, len(flat) // 3, flat.ctypes.data_as(_p(C.c_int32)) if len(flat) else None))
 
     def stage_times(self):
         ms = (C.c_double * 4)()

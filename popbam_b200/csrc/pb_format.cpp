@@ -429,3 +429,49 @@ extern "C" int64_t pb_format_window_garud(const pb_ctx *ctx, const pb_region_res
     if (!g || !g->n_hap || !g->h1 || !g->h12 || !g->h123 || !g->h2h1) return PB_ERR_ARG;
     return format_window(ctx, r, nullptr, nullptr, g, w, an, o, buf, cap);
 }
+
+// the one rule for a spectrum set (pb_set_spectra, pb_format_spectrum_dadi): 1-3 distinct populations in [0, n_pops),
+// -1 only in the trailing slots; returns its number of bins, prod (n_k + 1), or -1
+extern "C" int64_t pb_spectrum_set_bins(const pb_params *p, const int32_t *k) {
+    if (!p || !k) return -1;
+    int64_t bins = 1;
+    int used = 0;
+    for (int d = 0; d < 3; ++d) {
+        if (k[d] == -1) continue;
+        if (d > used || k[d] < 0 || k[d] >= p->n_pops) return -1;
+        for (int e = 0; e < d; ++e)
+            if (k[e] == k[d]) return -1;
+        bins *= (int64_t)p->pop_nsmpl[k[d]] + 1;
+        used += 1;
+    }
+    return used ? bins : -1;
+}
+
+extern "C" int64_t pb_format_spectrum_dadi(const pb_ctx *ctx, const int32_t *set3, const int64_t *counts, const pb_print_opts *o,
+                                           const char *comment, char *buf, int64_t cap) {
+    const pb_params *p = pb_ctx_params(ctx);
+    const int64_t bins = pb_spectrum_set_bins(p, set3);
+    if (bins < 0 || !counts || !o || !o->pop_names) return PB_ERR_ARG;
+    Out out;
+    for (const char *c = comment; c; ) {        // every line of the comment behind "# "
+        const char *e = strchr(c, '\n');
+        out.s += "# ";
+        out.s.append(c, e ? (size_t)(e - c) : strlen(c));
+        out.s += '\n';
+        c = e ? e + 1 : nullptr;
+    }
+    for (int d = 0; d < 3 && set3[d] >= 0; ++d) out.f("%s%d", d ? " " : "", p->pop_nsmpl[set3[d]] + 1);
+    out.s += " unfolded";
+    for (int d = 0; d < 3 && set3[d] >= 0; ++d) {
+        out.s += " \"";
+        out.s += o->pop_names[set3[d]];
+        out.s += '"';
+    }
+    out.s += '\n';
+    for (int64_t i = 0; i < bins; ++i) out.f("%s%lld", i ? " " : "", (long long)counts[i]);
+    out.s += '\n';
+    // dadi's default mask: the all-zero and the all-derived corner
+    for (int64_t i = 0; i < bins; ++i) out.s += (i == 0 || i == bins - 1) ? (i ? " 1" : "1") : " 0";
+    out.s += '\n';
+    return out.copy_to(buf, cap);
+}

@@ -19,6 +19,10 @@
 #include "pb_ld.cuh"
 #include "pb_abba.cuh"
 #include "pb_garud.cuh"
+#include "pb_spectrum.cuh"
+
+// the number of bins of one spectrum set, or -1 for a set pb_set_spectra refuses (pb_format.cpp)
+extern "C" int64_t pb_spectrum_set_bins(const pb_params *p, const int32_t *set3);
 
 namespace {
 
@@ -104,8 +108,15 @@ struct pb_ctx {
     std::vector<PbAbbaTriple> abba_tri;    // their per-triple constants, copied to d_abba_tri
     DevBuf d_abba_tri, d_abba;             // the constants; the PB_AN_ABBA result arena (abba_layout)
     DevBuf d_garud;                        // the PB_AN_GARUD result arena (garud_layout)
+    std::vector<int32_t> spec_set;         // pb_set_spectra: 3 population indices per set (-1: unused slot)
+    int64_t spec_ver = 0;                  // ... counts the lists pb_set_spectra was given
+    std::vector<int32_t> spec_run;         // the list the open region took at pb_region_begin (relaunches keep it)
+    int64_t spec_run_ver = -1;
+    std::vector<int32_t> spec_off;         // [NS+1] first bin of each set within a window's B
+    int spec_groups = 0;                   // groups of at most PB_SPECTRUM_GROUP_BINS bins (k_spectrum's grid.y)
+    DevBuf d_spec_tab, d_spec;             // PbSpecSet[NS] then PbSpecGroup[groups]; the PB_AN_SPECTRUM result arena
     // pinned results
-    HostBuf h_ctr, h_small, h_seg, h_span, h_abba, h_garud;
+    HostBuf h_ctr, h_small, h_seg, h_span, h_abba, h_garud, h_spec;
     PbCounters ctr_host;
     bool need_valid = false;
     int need_nl = 0;
@@ -116,6 +127,7 @@ struct pb_ctx {
     pb_region_fst fst;
     pb_region_abba abba;
     pb_region_garud garud;
+    pb_region_spectrum spec;
     // bam_fetch_f shim staging (pb_push_record)
     std::vector<int32_t> r_pos;
     std::vector<uint32_t> r_meta, r_cig_off, r_cigar, r_base_off;
@@ -267,6 +279,8 @@ GarudLayout garud_layout(void *base, int NW, int P) {
     L.bytes = (cv.off + 255) & ~(size_t)255;
     return L;
 }
+// the PB_AN_SPECTRUM counts, [NW*B]: an arena of their own, like abba_layout
+size_t spectrum_bytes(int NW, int B) { return ((size_t)NW * B * sizeof(int32_t) + 255) & ~(size_t)255; }
 struct SegLayout {
     uint32_t *seg_pos, *seg_idx; uint64_t *seg_type; uint8_t *seg_ref; uint64_t *seg_cb;
     size_t bytes;
@@ -745,6 +759,23 @@ int run_pipeline(pb_ctx *c, int attempt = 0, bool allow_async = true) {
         c->launches += 1;
         PB_CUDA(c, cudaGetLastError());
     }
+    // ---- site frequency spectra per (window, group of sets)
+    const bool with_spec = (c->analyses & PB_AN_SPECTRUM) != 0;
+    const int NB = with_spec ? c->spec_off.back() : 0;
+    if (with_spec) {
+        PB_TRY(dev_reserve(c, c->d_spec, spectrum_bytes(NW, NB)));
+        PB_TRY(host_reserve(c, c->h_spec, spectrum_bytes(NW, NB)));
+        const int NS = (int)c->spec_run.size() / 3;
+        PbSpectrumArgs ka;
+        ka.sets = dp<PbSpecSet>(c->d_spec_tab);
+        ka.groups = reinterpret_cast<const PbSpecGroup *>(ka.sets + NS);
+        ka.B = NB; ka.outg = (P.flags & PB_FLAG_OUTGROUP) != 0; ka.outidx = P.outidx;
+        ka.num_sites = dl.num_sites; ka.segsites = dl.segsites; ka.seg_off = dl.seg_off; ka.seg_type = sl.seg_type;
+        ka.counts = dp<int32_t>(c->d_spec);
+        k_spectrum<<<dim3((unsigned)NW, (unsigned)c->spec_groups), PB_SPECTRUM_THREADS, 0, st>>>(ka);
+        c->launches += 1;
+        PB_CUDA(c, cudaGetLastError());
+    }
     // ---- pairwise LD (ld -o 0 / -o 1, D'): keep list, tiled pair kernel, finish
     if (c->analyses & (PB_AN_LD_ZNS | PB_AN_LD_OMEGA | PB_AN_LD_DPRIME)) {
         PbLdArgs la;
@@ -785,6 +816,7 @@ int run_pipeline(pb_ctx *c, int attempt = 0, bool allow_async = true) {
     PB_CUDA(c, cudaMemcpyAsync(c->h_small.p, c->d_stats.p, dl.bytes, cudaMemcpyDeviceToHost, st));
     if (with_abba) PB_CUDA(c, cudaMemcpyAsync(c->h_abba.p, c->d_abba.p, abba_layout(nullptr, NW, NT).bytes, cudaMemcpyDeviceToHost, st));
     if (with_garud) PB_CUDA(c, cudaMemcpyAsync(c->h_garud.p, c->d_garud.p, garud_layout(nullptr, NW, P.n_pops).bytes, cudaMemcpyDeviceToHost, st));
+    if (with_spec) PB_CUDA(c, cudaMemcpyAsync(c->h_spec.p, c->d_spec.p, spectrum_bytes(NW, NB), cudaMemcpyDeviceToHost, st));
     if (!async && S > 0) PB_CUDA(c, cudaMemcpyAsync(c->h_seg.p, c->d_seg_type.p, sl.bytes, cudaMemcpyDeviceToHost, st));
     if (P.flags & PB_FLAG_EMIT_CB) {
         Carver cv(nullptr);
@@ -889,6 +921,12 @@ int fill_result(pb_ctx *c, pb_region_result *out) {
         g.n_hap = gl.n_hap; g.c1 = gl.c1; g.c2 = gl.c2; g.c3 = gl.c3; g.hh = gl.hh;
         g.h1 = gl.h1; g.h12 = gl.h12; g.h123 = gl.h123; g.h2h1 = gl.h2h1;
     }
+    pb_region_spectrum &sp = c->spec;
+    memset(&sp, 0, sizeof sp);
+    if (an & PB_AN_SPECTRUM) {
+        sp.n_sets = (int32_t)(c->spec_run.size() / 3); sp.n_bins = c->spec_off.back();
+        sp.sets = c->spec_run.data(); sp.set_off = c->spec_off.data(); sp.counts = reinterpret_cast<const int32_t *>(c->h_spec.p);
+    }
     if (an & PB_AN_DIVERGE_POP) { r.pop_div = hl.pop_div; r.div_num_snps = hl.div_num_snps; }
     if (an & (PB_AN_HAPLO_K | PB_AN_HAPLO_EHHS)) { r.nhaps = hl.nhaps; r.hdiv = hl.hdiv; }
     if (an & PB_AN_HAPLO_EHHS) r.ehhs = hl.ehhs;
@@ -908,6 +946,7 @@ int fill_result(pb_ctx *c, pb_region_result *out) {
 }
 
 int flush_records(pb_ctx *c);
+int spectrum_tables(pb_ctx *c);
 
 }  // namespace
 
@@ -1026,7 +1065,7 @@ void pb_destroy(pb_ctx *c) {
     if (c->stream2) cudaStreamSynchronize(c->stream2);
     if (c->stream_lo) cudaStreamSynchronize(c->stream_lo);
     for (DevBuf *b : c->bufs) if (b->p) { cudaFree(b->p); b->p = nullptr; b->cap = 0; }
-    HostBuf *hb[] = {&c->h_ctr, &c->h_small, &c->h_seg, &c->h_span, &c->h_abba, &c->h_garud};
+    HostBuf *hb[] = {&c->h_ctr, &c->h_small, &c->h_seg, &c->h_span, &c->h_abba, &c->h_garud, &c->h_spec};
     for (HostBuf *b : hb) if (b->p) cudaFreeHost(b->p);
     for (auto &ev : c->ev) if (ev) cudaEventDestroy(ev);
     for (auto &ev : c->fk) if (ev) cudaEventDestroy(ev);
@@ -1062,6 +1101,7 @@ int pb_region_begin(pb_ctx *c, uint32_t analyses, int32_t n_windows, const int32
     }
     if ((int64_t)win_end[n_windows - 1] - win_beg[0] < 1) return fail(c, PB_ERR_ARG, "empty region");
     if ((analyses & PB_AN_ABBA) && c->abba_set.empty()) return fail(c, PB_ERR_STATE, "pb_region_begin with PB_AN_ABBA before pb_set_abba");
+    if ((analyses & PB_AN_SPECTRUM) && c->spec_set.empty()) return fail(c, PB_ERR_STATE, "pb_region_begin with PB_AN_SPECTRUM before pb_set_spectra");
     PB_CUDA(c, cudaSetDevice(c->prm.device));
     PB_CUDA(c, cudaStreamSynchronize(c->stream));
     c->abba_run.clear(); c->abba_tri.clear(); c->abba_run_og = -1;
@@ -1080,6 +1120,7 @@ int pb_region_begin(pb_ctx *c, uint32_t analyses, int32_t n_windows, const int32
         PB_TRY(dev_reserve(c, c->d_abba_tri, sizeof(PbAbbaTriple) * c->abba_tri.size()));
         PB_CUDA(c, cudaMemcpyAsync(c->d_abba_tri.p, c->abba_tri.data(), sizeof(PbAbbaTriple) * c->abba_tri.size(), cudaMemcpyHostToDevice, c->stream));
     }
+    if ((analyses & PB_AN_SPECTRUM) && c->spec_run_ver != c->spec_ver) PB_TRY(spectrum_tables(c));
     c->analyses = analyses; c->nw = n_windows;
     c->h_wbeg.assign(win_beg, win_beg + n_windows); c->h_wend.assign(win_end, win_end + n_windows);
     c->span_beg = win_beg[0]; c->span_end = win_end[n_windows - 1];
@@ -1260,6 +1301,29 @@ int pb_region_get_garud(const pb_ctx *c, pb_region_garud *out) {
     return PB_OK;
 }
 
+int pb_region_get_spectrum(const pb_ctx *c, pb_region_spectrum *out) {
+    if (!c || !out) return PB_ERR_ARG;
+    *out = c->spec;
+    return PB_OK;
+}
+
+int pb_set_spectra(pb_ctx *c, int32_t n_sets, const int32_t *sets) {
+    if (!c) return PB_ERR_ARG;
+    if (n_sets < 0 || n_sets > PB_MAX_SPECTRUM_SETS) return fail(c, PB_ERR_ARG, "pb_set_spectra: n_sets must be in 0 .. %d", PB_MAX_SPECTRUM_SETS);
+    if (n_sets > 0 && !sets) return fail(c, PB_ERR_ARG, "pb_set_spectra: null sets");
+    int64_t bins = 0;
+    for (int s = 0; s < n_sets; ++s) {
+        const int64_t b = pb_spectrum_set_bins(&c->prm, sets + 3 * (size_t)s);
+        if (b < 0) return fail(c, PB_ERR_ARG, "pb_set_spectra: set %d (%d, %d, %d): an index outside 0 .. %d, a repeated population, an empty set or -1 before an index",
+                               s, sets[3 * s], sets[3 * s + 1], sets[3 * s + 2], c->prm.n_pops - 1);
+        bins += b;
+    }
+    if (bins > PB_MAX_SPECTRUM_BINS) return fail(c, PB_ERR_ARG, "pb_set_spectra: %lld bins per window, more than %d", (long long)bins, PB_MAX_SPECTRUM_BINS);
+    c->spec_set.assign(sets, sets + 3 * (size_t)n_sets);
+    c->spec_ver += 1;
+    return PB_OK;
+}
+
 int pb_set_abba(pb_ctx *c, int32_t outgroup_pop, int32_t n_triples, const int32_t *triples) {
     if (!c) return PB_ERR_ARG;
     if (n_triples < 0 || n_triples > PB_MAX_ABBA_TRIPLES) return fail(c, PB_ERR_ARG, "pb_set_abba: n_triples must be in 0 .. %d", PB_MAX_ABBA_TRIPLES);
@@ -1303,6 +1367,41 @@ const pb_params *pb_ctx_params(const pb_ctx *c) { return c ? &c->prm : nullptr; 
 }  // extern "C"
 
 namespace {
+// the list pb_set_spectra took last becomes the one regions run with: bin offsets, the per-set constants and the groups
+// of at most PB_SPECTRUM_GROUP_BINS bins, uploaded once per list (pb_region_begin has synchronised the stream)
+int spectrum_tables(pb_ctx *c) {
+    const pb_params &P = c->prm;
+    c->spec_run = c->spec_set;
+    const int NS = (int)c->spec_run.size() / 3;
+    std::vector<PbSpecSet> tab((size_t)NS);
+    std::vector<PbSpecGroup> grp;
+    c->spec_off.assign(1, 0);
+    for (int s = 0; s < NS; ++s) {
+        const int32_t *k = &c->spec_run[3 * (size_t)s];
+        PbSpecSet &q = tab[(size_t)s];
+        memset(&q, 0, sizeof q);
+        int stride = 1;
+        for (int d = 2; d >= 0; --d) {
+            if (k[d] < 0) continue;
+            q.mask[d] = P.pop_mask[k[d]]; q.n[d] = P.pop_nsmpl[k[d]]; q.stride[d] = stride;
+            stride *= q.n[d] + 1;
+        }
+        const int b0 = c->spec_off.back();
+        if (grp.empty() || grp.back().nb + stride > PB_SPECTRUM_GROUP_BINS) grp.push_back(PbSpecGroup{s, s, b0, 0});
+        q.off = grp.back().nb;
+        grp.back().s1 = s + 1; grp.back().nb += stride;
+        c->spec_off.push_back(b0 + stride);
+    }
+    c->spec_groups = (int)grp.size();
+    const size_t bytes = sizeof(PbSpecSet) * tab.size() + sizeof(PbSpecGroup) * grp.size();
+    PB_TRY(dev_reserve(c, c->d_spec_tab, bytes));
+    PB_CUDA(c, cudaMemcpyAsync(c->d_spec_tab.p, tab.data(), sizeof(PbSpecSet) * tab.size(), cudaMemcpyHostToDevice, c->stream));
+    PB_CUDA(c, cudaMemcpyAsync(dp<PbSpecSet>(c->d_spec_tab) + tab.size(), grp.data(), sizeof(PbSpecGroup) * grp.size(), cudaMemcpyHostToDevice, c->stream));
+    PB_CUDA(c, cudaStreamSynchronize(c->stream));      // tab and grp go out of scope
+    c->spec_run_ver = c->spec_ver;
+    return PB_OK;
+}
+
 int flush_records(pb_ctx *c) {
     if (c->r_pos.empty()) return PB_OK;
     pb_read_batch b;

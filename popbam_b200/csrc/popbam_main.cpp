@@ -16,7 +16,11 @@
 // -p, D; ld -o 0: mean |D'| and the number of SNP pairs in complete LD); for nucdiv only, --fst: F_ST (Hudson, and Weir &
 // Cockerham) and Hudson's Snn for every population pair, after the --extra-stats columns, with --snn-perms N: a permutation
 // p-value of Snn from N random re-partitions of the pair's samples, drawn from a stream seeded by --seed S (default 0); for
-// haplo only (any -o), --garud: Garud's H1, H12, H123 and H2/H1 and the number of distinct haplotypes per population.
+// haplo only (any -o), --garud: Garud's H1, H12, H123 and H2/H1 and the number of distinct haplotypes per population;
+// for sfs only, --jsfs PREFIX: the unfolded site frequency spectra of every population and every population pair (without
+// the population of the -p sample), or of the sets --jsfs-pops A[,B[,C]] names (repeatable, in the order given), summed
+// over every window of the region and written in dadi's format to PREFIX.A.fs, PREFIX.A-B.fs, PREFIX.A-B-C.fs after the
+// last row.
 //
 // One subcommand the reference does not have: `abba -p SAMPLE`, per window Patterson's D, f_d and f_dM of population
 // triples (P1, P2, P3) against the population of SAMPLE as the outgroup; by default every triple with P1 < P2, or the
@@ -57,6 +61,8 @@ struct Options {
     bool extra_stats = false;
     bool fst = false, snn_opts = false;
     bool garud = false;
+    std::string jsfs;                      // sfs: --jsfs PREFIX
+    std::vector<std::string> jsfs_pops;    // sfs: --jsfs-pops A[,B[,C]]
     long long snn_perms = 0;
     unsigned long long seed = 0;
     std::vector<std::string> triples;      // abba: --triple A,B,C
@@ -86,6 +92,8 @@ void usage(const char *cmd) {
             "         --fst  nucdiv: Fst[A-B] (Hudson), FstWC[A-B] (Weir & Cockerham), Snn[A-B] (Hudson's nearest neighbours)\n"
             "         --snn-perms N  with --fst: SnnP[A-B], p-value of Snn from N permutations   --seed S  their random stream (0)\n"
             "         --garud  haplo: nHap[pop] (distinct haplotypes), H1[pop], H12[pop], H123[pop], H2H1[pop] (Garud's H)\n"
+            "         --jsfs PREFIX  sfs: unfolded spectra summed over the region, in dadi's format, to PREFIX.A.fs, PREFIX.A-B.fs\n"
+            "         (every population and pair, without -p's)   --jsfs-pops A[,B[,C]] (repeatable) the sets to write instead\n"
             "         abba: -p STR a sample of the outgroup population (required)   --triple A,B,C (repeatable) the triples to\n"
             "         report, in this order (default: every P1 < P2, P3 besides them); columns S, ABBA, BABA, D, fd, fdM [A-B-C]\n", cmd);
 }
@@ -113,6 +121,8 @@ Options parse(int argc, char **argv) {
                 continue;
             }
             if (a == "--triple") { o.triples.push_back(val()); continue; }
+            if (a == "--jsfs") { o.jsfs = val(); if (o.jsfs.empty()) fatal("--jsfs needs a file name prefix"); continue; }
+            if (a == "--jsfs-pops") { o.jsfs_pops.push_back(val()); continue; }
             if (a == "--gpus") o.gpus = atoi(val());
             else if (a == "--shard-mb") o.shard_mb = atof(val());
             else if (a == "--threads") o.threads = atoi(val());
@@ -176,6 +186,8 @@ Options parse(int argc, char **argv) {
     if (o.snn_opts && !o.fst) fatal("--snn-perms and --seed go with --fst");
     if (!o.triples.empty() && o.cmd != "abba") fatal("--triple is only available for abba");
     if (o.garud && o.cmd != "haplo") fatal("--garud is only available for haplo");
+    if ((!o.jsfs.empty() || !o.jsfs_pops.empty()) && o.cmd != "sfs") fatal("--jsfs and --jsfs-pops are only available for sfs");
+    if (!o.jsfs_pops.empty() && o.jsfs.empty()) fatal("--jsfs-pops goes with --jsfs");
     if (o.cmd == "abba" && !o.has_p) fatal("abba needs -p SAMPLE: a sample of the outgroup population");
     return o;
 }
@@ -189,6 +201,8 @@ struct Shard {
     std::vector<std::pair<int32_t, int32_t>> cuts;     // [lo, hi) of every piece
     int pieces_left = 0;
     std::string text;
+    std::vector<int64_t> spec;  // --jsfs: the shard's spectra summed over its windows, and its num_sites
+    int64_t spec_sites = 0;
     std::string error;
     int state = 0;              // 0 pending, 1 decoded, 2 done
 };
@@ -208,6 +222,9 @@ struct Run {
     uint32_t analysis = 0;
     int32_t abba_og = -1;                  // abba: the outgroup population and the triples (P1, P2, P3, ...)
     std::vector<int32_t> abba_triples;
+    std::vector<int32_t> spec_sets;        // --jsfs: 3 population indices per set (-1: unused slot), and their bins
+    std::vector<int64_t> spec_off;
+    pb_ctx *spec_ctx = nullptr;            // --jsfs: worker 0's context, kept for pb_format_spectrum_dadi
     // error-model tables, built once on the host (while the files are opened) and shared by every context
     std::vector<double> fk, beta, lhet;
     std::shared_future<void> tables_ready;
@@ -317,6 +334,9 @@ void gpu_worker(Run *R, int g, int G, int device) {
     else if (pb_set_snn_perms(ctx, R->opt.snn_perms, R->opt.seed) != PB_OK) err = pb_last_error(ctx);
     else if ((R->analysis & PB_AN_ABBA) &&
              pb_set_abba(ctx, R->abba_og, (int32_t)(R->abba_triples.size() / 3), R->abba_triples.data()) != PB_OK) err = pb_last_error(ctx);
+    else if ((R->analysis & PB_AN_SPECTRUM) &&
+             pb_set_spectra(ctx, (int32_t)(R->spec_sets.size() / 3), R->spec_sets.data()) != PB_OK) err = pb_last_error(ctx);
+    const uint32_t rows = R->analysis & ~PB_AN_SPECTRUM;     // the spectra add no columns
     std::vector<const char *> pops, smps;
     for (auto &s : R->st.pops) pops.push_back(s.c_str());
     for (auto &s : R->st.samples) smps.push_back(s.c_str());
@@ -339,6 +359,7 @@ void gpu_worker(Run *R, int g, int G, int device) {
             pb_region_fst fst;
             pb_region_abba abba;
             pb_region_garud garud;
+            pb_region_spectrum spec;
             int rc = pb_region_begin(ctx, R->analysis, sh.w1 - sh.w0, &R->wb[sh.w0], &R->we[sh.w0]);
             {
                 int64_t nr = 0, nc = 0, nb = 0;
@@ -361,11 +382,12 @@ void gpu_worker(Run *R, int g, int G, int device) {
             if (rc == PB_OK) rc = pb_region_get_fst(ctx, &fst);
             if (rc == PB_OK) rc = pb_region_get_abba(ctx, &abba);
             if (rc == PB_OK) rc = pb_region_get_garud(ctx, &garud);
+            if (rc == PB_OK) rc = pb_region_get_spectrum(ctx, &spec);
             auto format = [&](int w) {
-                if (R->analysis & PB_AN_ABBA) return pb_format_window_abba(ctx, &res, &abba, w, &po, line.data(), (int64_t)line.size());
-                if (R->analysis & PB_AN_GARUD) return pb_format_window_garud(ctx, &res, &garud, w, R->analysis, &po, line.data(), (int64_t)line.size());
-                return (R->analysis & PB_AN_FST) ? pb_format_window_fst(ctx, &res, &ext, &fst, w, R->analysis, &po, line.data(), (int64_t)line.size())
-                                                 : pb_format_window_ext(ctx, &res, &ext, w, R->analysis, &po, line.data(), (int64_t)line.size());
+                if (rows & PB_AN_ABBA) return pb_format_window_abba(ctx, &res, &abba, w, &po, line.data(), (int64_t)line.size());
+                if (rows & PB_AN_GARUD) return pb_format_window_garud(ctx, &res, &garud, w, rows, &po, line.data(), (int64_t)line.size());
+                return (rows & PB_AN_FST) ? pb_format_window_fst(ctx, &res, &ext, &fst, w, rows, &po, line.data(), (int64_t)line.size())
+                                          : pb_format_window_ext(ctx, &res, &ext, w, rows, &po, line.data(), (int64_t)line.size());
             };
             if (rc != PB_OK) sh.error = pb_last_error(ctx);
             else
@@ -375,6 +397,14 @@ void gpu_worker(Run *R, int g, int G, int device) {
                     if (k < 0) { sh.error = "formatting failed"; break; }
                     sh.text.append(line.data(), (size_t)k);
                 }
+            if (rc == PB_OK && (R->analysis & PB_AN_SPECTRUM)) {     // every window, whatever -k says
+                sh.spec.assign((size_t)spec.n_bins, 0);
+                for (int w = 0; w < res.n_windows; ++w) {
+                    const int32_t *x = spec.counts + (size_t)w * spec.n_bins;
+                    for (int b = 0; b < spec.n_bins; ++b) sh.spec[(size_t)b] += x[b];
+                    sh.spec_sites += res.num_sites[w];
+                }
+            }
         } else if (sh.error.empty()) sh.error = err;
         for (pbio::Batch &b : sh.pieces) R->give_batch(std::move(b));       // (pb_region_end has waited for the copies)
         sh.pieces.clear();
@@ -382,7 +412,83 @@ void gpu_worker(Run *R, int g, int G, int device) {
         sh.state = 2;
         R->cv.notify_all();
     }
-    if (ctx) pb_destroy(ctx);
+    if (g == 0 && (R->analysis & PB_AN_SPECTRUM)) R->spec_ctx = ctx;       // main writes the spectra with it
+    else if (ctx) pb_destroy(ctx);
+}
+
+// sfs --jsfs: the spectrum sets, from --jsfs-pops or every population and then every pair i < j (dxy order), without the
+// population of the -p sample
+void spectrum_sets(Run &R) {
+    const Options &o = R.opt;
+    const int P = (int)R.st.pops.size();
+    const int og = (R.prm.flags & PB_FLAG_OUTGROUP) ? R.st.sample_pop[R.prm.outidx] : -1;
+    std::vector<int32_t> &ss = R.spec_sets;
+    if (o.jsfs_pops.empty()) {
+        for (int i = 0; i < P; ++i) if (i != og) ss.insert(ss.end(), {i, -1, -1});
+        for (int i = 0; i < P; ++i)
+            for (int j = i + 1; j < P; ++j)
+                if (i != og && j != og) ss.insert(ss.end(), {i, j, -1});
+    }
+    for (const std::string &spec : o.jsfs_pops) {
+        std::vector<std::string> names;
+        std::string cur;
+        for (char ch : spec) {
+            if (ch == ',') { names.push_back(cur); cur.clear(); }
+            else cur += ch;
+        }
+        names.push_back(cur);
+        if (names.size() > 3) fatal("--jsfs-pops " + spec + ": at most three population names");
+        int32_t k[3] = {-1, -1, -1};
+        for (size_t i = 0; i < names.size(); ++i) {
+            for (int q = 0; q < P; ++q) if (R.st.pops[q] == names[i]) k[i] = q;
+            if (k[i] < 0) fatal("--jsfs-pops " + spec + ": unknown population " + names[i]);
+            for (size_t e = 0; e < i; ++e) if (k[e] == k[i]) fatal("--jsfs-pops " + spec + ": population " + names[i] + " is repeated");
+        }
+        ss.insert(ss.end(), k, k + 3);
+    }
+    R.spec_off.assign(1, 0);
+    for (size_t s = 0; s < ss.size(); s += 3) {
+        int64_t b = 1;
+        for (int d = 0; d < 3 && ss[s + d] >= 0; ++d) b *= R.st.pop_nsmpl[ss[s + d]] + 1;
+        R.spec_off.push_back(R.spec_off.back() + b);
+    }
+    const std::string hint = o.jsfs_pops.empty() ? "; name the sets to write with --jsfs-pops" : "";
+    if (ss.empty()) fatal("--jsfs: no population besides the outgroup's");
+    if (ss.size() / 3 > PB_MAX_SPECTRUM_SETS)
+        fatal("--jsfs: " + std::to_string(ss.size() / 3) + " spectrum sets, more than " + std::to_string(PB_MAX_SPECTRUM_SETS) + hint);
+    if (R.spec_off.back() > PB_MAX_SPECTRUM_BINS)
+        fatal("--jsfs: " + std::to_string(R.spec_off.back()) + " bins per window over all spectrum sets, more than " +
+              std::to_string(PB_MAX_SPECTRUM_BINS) + hint);
+}
+
+// sfs --jsfs: one file per set, PREFIX.A[-B[-C]].fs
+void write_spectra(Run &R, const std::vector<int64_t> &total, int64_t sites) {
+    const Options &o = R.opt;
+    std::vector<const char *> pops;
+    for (auto &s : R.st.pops) pops.push_back(s.c_str());
+    pb_print_opts po;
+    memset(&po, 0, sizeof po);
+    po.chrom = R.hdr.names[R.tid].c_str();
+    po.pop_names = pops.data();
+    const std::string comment = "popbam sfs " + R.hdr.names[R.tid] + ":" + std::to_string(R.beg + 1) + "-" + std::to_string(R.end) + ", " +
+                                std::to_string(R.wb.size()) + " windows, " + std::to_string(sites) + " sites, polarised by " +
+                                ((R.prm.flags & PB_FLAG_OUTGROUP) ? R.st.samples[R.prm.outidx] : std::string("the reference base"));
+    if (!R.spec_ctx) fatal("no GPU context to format the spectra with");
+    std::vector<char> buf;
+    for (size_t s = 0; s * 3 < R.spec_sets.size(); ++s) {
+        const int32_t *k = &R.spec_sets[3 * s];
+        std::string path = o.jsfs;
+        for (int d = 0; d < 3 && k[d] >= 0; ++d) path += (d ? "-" : ".") + R.st.pops[k[d]];
+        path += ".fs";
+        const int64_t *x = total.data() + R.spec_off[s];
+        int64_t len = pb_format_spectrum_dadi(R.spec_ctx, k, x, &po, comment.c_str(), nullptr, 0);
+        if (len < 0) fatal("formatting the spectrum of " + path + " failed");
+        buf.resize((size_t)len + 1);
+        pb_format_spectrum_dadi(R.spec_ctx, k, x, &po, comment.c_str(), buf.data(), (int64_t)buf.size());
+        FILE *f = fopen(path.c_str(), "w");
+        const bool ok = f && fwrite(buf.data(), 1, (size_t)len, f) == (size_t)len;
+        if (!f || fclose(f) != 0 || !ok) fatal("Cannot write spectrum file " + path);
+    }
 }
 
 // abba: the outgroup population (that of sample -p) and the triples, from --triple or every P1 < P2, P3 besides them
@@ -582,6 +688,10 @@ int main(int argc, char **argv) {
     if (o.fst) R.analysis |= PB_AN_FST;
     if (o.garud) R.analysis |= PB_AN_GARUD;
     if (o.cmd == "abba") abba_triples(R);
+    if (!o.jsfs.empty()) {
+        R.analysis |= PB_AN_SPECTRUM;
+        spectrum_sets(R);
+    }
 
     // window grid of the region, then shards = runs of whole windows
     const int64_t nw = pb_window_grid(R.beg, R.end, o.window ? o.win_size : 0, 0, nullptr, nullptr);
@@ -642,6 +752,8 @@ int main(int argc, char **argv) {
     for (int i = 0; i < D; ++i) th.emplace_back(decode_worker, &R);
     for (int w = 0; w < W; ++w) th.emplace_back(gpu_worker, &R, w, W, w % G);
     int rc = 0;
+    std::vector<int64_t> spec_total(R.spec_off.empty() ? 0 : (size_t)R.spec_off.back(), 0);    // --jsfs: the region's sums
+    int64_t spec_sites = 0;
     for (size_t s = 0; s < R.shards.size(); ++s) {
         Shard &sh = R.shards[s];
         {
@@ -651,6 +763,8 @@ int main(int argc, char **argv) {
         if (!sh.error.empty()) { fflush(stdout); fprintf(stderr, "popbam runtime error:\n%s\nExiting program\n", sh.error.c_str()); rc = 1; }
         else fwrite(sh.text.data(), 1, sh.text.size(), stdout);
         sh.text.clear(); sh.text.shrink_to_fit();
+        for (size_t b = 0; b < sh.spec.size(); ++b) spec_total[b] += sh.spec[b];
+        spec_sites += sh.spec_sites;
         {
             std::lock_guard<std::mutex> lk(R.mu);
             R.printed = (int)s + 1;
@@ -660,5 +774,9 @@ int main(int argc, char **argv) {
     }
     for (auto &t : th) t.join();
     fflush(stdout);
+    if (R.analysis & PB_AN_SPECTRUM) {
+        write_spectra(R, spec_total, spec_sites);
+        pb_destroy(R.spec_ctx);
+    }
     return rc;
 }
