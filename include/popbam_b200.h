@@ -69,6 +69,7 @@ typedef enum pb_status {
 #define PB_AN_ABBA          0x10000u /* ABBA-BABA: Patterson's D, f_d, f_dM per triple (pb_set_abba; alone or with any) */
 #define PB_AN_GARUD         0x20000u /* Garud's H1, H12, H123, H2/H1 per population (alone or with any; haplo --garud) */
 #define PB_AN_SPECTRUM      0x40000u /* unfolded site frequency spectra of 1-3 populations (pb_set_spectra; alone or with any; sfs --jsfs) */
+#define PB_AN_NUCDIV_MISSING 0x80000u /* pi and dxy over sites with missing calls, pixy-style sums (alone or with any; nucdiv --missing) */
 
 #define PB_MAX_ABBA_TRIPLES 1024     /* pb_set_abba: most (P1, P2, P3) triples of one region                        */
 #define PB_MAX_SPECTRUM_SETS 4096    /* pb_set_spectra: most spectrum sets of one region                            */
@@ -296,6 +297,37 @@ typedef struct pb_region_spectrum {
     const int32_t *counts;              /* [NW*B] index w*B + set_off[s] + bin                                  */
 } pb_region_spectrum;
 
+/* pi and dxy over positions where some samples have no call (PB_AN_NUCDIV_MISSING), as window sums of pairwise
+ * differences and pairwise comparisons among the samples called at each position (Korunes & Samuk 2021, pixy): a struct
+ * of its own, like pb_region_garud, with the same lifetime.  Every array is NULL unless PB_AN_NUCDIV_MISSING was
+ * requested.  Every other statistic uses a position only where every sample passes qfilter (site_flag bit 0); these
+ * use every position x of the window [win_beg, win_end):
+ *   cov(x)  the samples whose cell passes qfilter (the bits whose popcount decides site_flag bit 0)
+ *   der(x)  site_type(x), the samples whose final cb word has (cb & 3) == 3 (a subset of cov; calls count as haploid, as
+ *           for pi and dxy; with PB_FLAG_HETEROZYGOTE a heterozygous call counts as derived)
+ *   fq(x)   segbase's value over all samples' calls; where fq(x) < 0 (two different derived bases) der(x) := 0: the
+ *           position still counts, with no differences, as the reference counts such a site in num_sites only
+ *   k_p = popcount(cov & pop_mask[p]), c_p = popcount(der & pop_mask[p]), n_p = pop_nsmpl[p].
+ * Within p, a position counts where k_p >= 2:   pi_sites += 1, pi_diffs += c_p (k_p - c_p),
+ *   pi_comps += k_p (k_p - 1) / 2, pi_missing += n_p (n_p - 1) / 2 - k_p (k_p - 1) / 2.
+ * Between i < j, a position counts where k_i >= 1 and k_j >= 1:   dxy_sites += 1,
+ *   dxy_diffs += c_i (k_j - c_j) + c_j (k_i - c_i), dxy_comps += k_i k_j, dxy_missing += n_i n_j - k_i k_j.
+ * pi = (double) pi_diffs / (double) pi_comps and dxy = (double) dxy_diffs / (double) dxy_comps, NaN where the denominator
+ * is 0 (a one-sample population has pi_sites = 0 and pi NaN; its dxy is defined).  Every sum is an exact integer, so the
+ * result does not depend on summation order, shards or GPUs; 0 <= diffs <= comps.  Windows combine by summing the
+ * counts.  Restricted to the positions with site_flag bit 0, pi_sites = num_sites, pi_comps = num_sites C(n_p, 2) and
+ * pi_diffs = piw C(n_p, 2) for n_p >= 2, and dxy_diffs = pib n_i n_j where every sample of i precedes every sample of j.
+ * The pi arrays are [NW*P], index w*P + p; the dxy arrays [NW*P*P], index i*P + (j-(i+1)) like pib, 0 in the slots that
+ * name no pair.                                                                                                        */
+typedef struct pb_region_nucdiv_missing {
+    const int32_t *pi_sites;            /* [NW*P]   positions with k_p >= 2                                       */
+    const int64_t *pi_diffs, *pi_comps, *pi_missing;
+    const double  *pi;
+    const int32_t *dxy_sites;           /* [NW*P*P] positions with k_i >= 1 and k_j >= 1                          */
+    const int64_t *dxy_diffs, *dxy_comps, *dxy_missing;
+    const double  *dxy;
+} pb_region_nucdiv_missing;
+
 typedef struct pb_ctx pb_ctx;
 
 /* ---- life cycle ---------------------------------------------------------------------- */
@@ -364,6 +396,8 @@ int pb_region_get_spectrum(const pb_ctx *ctx, pb_region_spectrum *out);
  * outside [0, n_pops), a population repeated within a set, an empty set, a -1 before a valid index, n_sets < 0 or
  * > PB_MAX_SPECTRUM_SETS, or more than PB_MAX_SPECTRUM_BINS bins per window over all sets.                           */
 int pb_set_spectra(pb_ctx *ctx, int32_t n_sets, const int32_t *sets);
+/* The PB_AN_NUCDIV_MISSING arrays of the region pb_region_end / pb_region_wait returned last.                         */
+int pb_region_get_nucdiv_missing(const pb_ctx *ctx, pb_region_nucdiv_missing *out);
 
 /* Asynchronous split of pb_region_end for overlap / device timing: launch enqueues every
  * kernel and the result copies on the context's stream; wait blocks and fills *out.       */
@@ -454,6 +488,16 @@ int64_t pb_format_window_garud(const pb_ctx *ctx, const pb_region_result *res, c
  * PB_ERR_ARG for a set pb_set_spectra would refuse.                                                                    */
 int64_t pb_format_spectrum_dadi(const pb_ctx *ctx, const int32_t *set3, const int64_t *counts, const pb_print_opts *opts,
                                 const char *comment, char *buf, int64_t cap);
+/* One window of `popbam nucdiv --missing` in the column layout of pixy's output files, tab-separated, one line each:
+ *   pairs = 0 (PREFIX_pi.txt):  pop chromosome window_pos_1 window_pos_2 avg_pi no_sites count_diffs count_comparisons
+ *                               count_missing, one line per population in population order
+ *   pairs = 1 (PREFIX_dxy.txt): pop1 pop2 chromosome window_pos_1 window_pos_2 avg_dxy no_sites count_diffs
+ *                               count_comparisons count_missing, one line per pair i < j in dxy order
+ * window_pos_1 = win_beg + 1 and window_pos_2 = win_end (1-based, inclusive); the ratio as %.10g, NA where its denominator
+ * is 0; names from opts->pop_names, opts->chrom.  Every window is written (opts->min_sites plays no part).  Returns bytes
+ * written (excluding NUL) or the required size if it exceeds cap; PB_ERR_ARG without the arrays.                       */
+int64_t pb_format_window_nucdiv_missing(const pb_ctx *ctx, const pb_region_result *res, const pb_region_nucdiv_missing *md,
+                                        int32_t window, int32_t pairs, const pb_print_opts *opts, char *buf, int64_t cap);
 
 #ifdef __cplusplus
 }

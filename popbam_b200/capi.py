@@ -11,7 +11,8 @@ MAXS = 64
 
 AN = dict(NUCDIV=0x001, SFS=0x002, LD_ZNS=0x004, LD_OMEGA=0x008, LD_WALL=0x010, DIVERGE_IND=0x020,
           DIVERGE_POP=0x040, HAPLO_K=0x080, HAPLO_EHHS=0x100, HAPLO_DXY=0x200, SNP=0x400, TREE=0x800,
-          THETA_W=0x1000, FULI=0x2000, LD_DPRIME=0x4000, FST=0x8000, ABBA=0x10000, GARUD=0x20000, SPECTRUM=0x40000)
+          THETA_W=0x1000, FULI=0x2000, LD_DPRIME=0x4000, FST=0x8000, ABBA=0x10000, GARUD=0x20000, SPECTRUM=0x40000,
+          NUCDIV_MISSING=0x80000)
 FLAG = dict(ILLUMINA=0x02, SUBSTITUTE=0x10, HETEROZYGOTE=0x20, OUTGROUP=0x40, EMIT_CB=0x10000)
 
 EXPORTS = ["pb_create", "pb_destroy", "pb_last_error", "pb_version", "pb_set_contig", "pb_region_begin", "pb_push_batch", "pb_push_batch_async",
@@ -19,7 +20,8 @@ EXPORTS = ["pb_create", "pb_destroy", "pb_last_error", "pb_version", "pb_set_con
            "pb_kernel_launches", "pb_region_path", "pb_region_reruns", "pb_stage_times", "pb_window_grid", "pb_build_errmod_tables", "pb_errmod_tables_cached", "pb_errmod_tables_cached_ex", "pb_host_alloc", "pb_host_free", "pb_format_window",
            "pb_region_get_extras", "pb_format_window_ext", "pb_region_get_fst", "pb_set_snn_perms", "pb_format_window_fst",
            "pb_region_get_abba", "pb_set_abba", "pb_format_window_abba", "pb_region_get_garud", "pb_format_window_garud",
-           "pb_region_get_spectrum", "pb_set_spectra", "pb_format_spectrum_dadi"]
+           "pb_region_get_spectrum", "pb_set_spectra", "pb_format_spectrum_dadi", "pb_region_get_nucdiv_missing",
+           "pb_format_window_nucdiv_missing"]
 
 
 def _p(t):
@@ -100,6 +102,13 @@ class Spectrum(C.Structure):
     """pb_region_spectrum: the PB_AN_SPECTRUM arrays; counts [NW*n_bins], index w*n_bins + set_off[s] + bin."""
     _fields_ = [("n_sets", C.c_int32), ("n_bins", C.c_int32), ("sets", _p(C.c_int32)), ("set_off", _p(C.c_int32)),
                 ("counts", _p(C.c_int32))]
+
+
+class NucdivMissing(C.Structure):
+    """pb_region_nucdiv_missing: the PB_AN_NUCDIV_MISSING arrays; pi_* [NW*P] (w*P + p), dxy_* [NW*P*P] (w*P*P + i*P + (j-(i+1)))."""
+    _fields_ = [("pi_sites", _p(C.c_int32)), ("pi_diffs", _p(C.c_int64)), ("pi_comps", _p(C.c_int64)), ("pi_missing", _p(C.c_int64)),
+                ("pi", _p(C.c_double)), ("dxy_sites", _p(C.c_int32)), ("dxy_diffs", _p(C.c_int64)), ("dxy_comps", _p(C.c_int64)),
+                ("dxy_missing", _p(C.c_int64)), ("dxy", _p(C.c_double))]
 
 
 class PrintOpts(C.Structure):
@@ -184,6 +193,10 @@ def lib():
         L.pb_set_spectra.argtypes = [C.c_void_p, C.c_int32, _p(C.c_int32)]
         L.pb_format_spectrum_dadi.restype = C.c_int64
         L.pb_format_spectrum_dadi.argtypes = [C.c_void_p, _p(C.c_int32), _p(C.c_int64), _p(PrintOpts), C.c_char_p, C.c_char_p, C.c_int64]
+        L.pb_region_get_nucdiv_missing.argtypes = [C.c_void_p, _p(NucdivMissing)]
+        L.pb_format_window_nucdiv_missing.restype = C.c_int64
+        L.pb_format_window_nucdiv_missing.argtypes = [C.c_void_p, _p(Result), _p(NucdivMissing), C.c_int32, C.c_int32, _p(PrintOpts),
+                                                      C.c_char_p, C.c_int64]
         _lib = L
     return _lib
 
@@ -212,6 +225,7 @@ class Context:
         self.abba = Abba()
         self.garud = Garud()
         self.spectrum = Spectrum()
+        self.nucdiv_missing = NucdivMissing()
 
     def _chk(self, rc):
         if rc != 0:
@@ -250,6 +264,7 @@ class Context:
         self._chk(self.L.pb_region_get_abba(self.h, C.byref(self.abba)))
         self._chk(self.L.pb_region_get_garud(self.h, C.byref(self.garud)))
         self._chk(self.L.pb_region_get_spectrum(self.h, C.byref(self.spectrum)))
+        self._chk(self.L.pb_region_get_nucdiv_missing(self.h, C.byref(self.nucdiv_missing)))
         return self.res
 
     def launch(self):
@@ -265,6 +280,7 @@ class Context:
         self._chk(self.L.pb_region_get_abba(self.h, C.byref(self.abba)))
         self._chk(self.L.pb_region_get_garud(self.h, C.byref(self.garud)))
         self._chk(self.L.pb_region_get_spectrum(self.h, C.byref(self.spectrum)))
+        self._chk(self.L.pb_region_get_nucdiv_missing(self.h, C.byref(self.nucdiv_missing)))
         return self.res
 
     def set_snn_perms(self, n_perms, seed=0):
@@ -316,5 +332,20 @@ class Context:
             if k >= len(buf):
                 buf = C.create_string_buffer(int(k) + 16)
                 k = fmt(w, buf)
+            out.append(buf.raw[:k].decode())
+        return "".join(out)
+
+    def missing_text(self, pairs, opts, windows=None):
+        """Lines of `nucdiv --missing`'s PREFIX_pi.txt (pairs = 0) or PREFIX_dxy.txt (pairs = 1), without the header line."""
+        out = []
+        buf = C.create_string_buffer(1 << 16)
+        for w in (range(self.res.n_windows) if windows is None else windows):
+            k = self.L.pb_format_window_nucdiv_missing(self.h, C.byref(self.res), C.byref(self.nucdiv_missing), w, pairs, C.byref(opts), buf, len(buf))
+            if k < 0:
+                raise PopbamError("pb_format_window_nucdiv_missing failed: %d" % k)
+            if k >= len(buf):
+                buf = C.create_string_buffer(int(k) + 16)
+                k = self.L.pb_format_window_nucdiv_missing(self.h, C.byref(self.res), C.byref(self.nucdiv_missing), w, pairs, C.byref(opts), buf,
+                                                           len(buf))
             out.append(buf.raw[:k].decode())
         return "".join(out)

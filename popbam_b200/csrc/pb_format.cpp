@@ -475,3 +475,36 @@ extern "C" int64_t pb_format_spectrum_dadi(const pb_ctx *ctx, const int32_t *set
     out.s += '\n';
     return out.copy_to(buf, cap);
 }
+
+extern "C" int64_t pb_format_window_nucdiv_missing(const pb_ctx *ctx, const pb_region_result *r, const pb_region_nucdiv_missing *md,
+                                                   int32_t w, int32_t pairs, const pb_print_opts *o, char *buf, int64_t cap) {
+    const pb_params *p = pb_ctx_params(ctx);
+    if (!p || !r || !md || !o || !o->chrom || !o->pop_names || w < 0 || w >= r->n_windows || (pairs != 0 && pairs != 1)) return PB_ERR_ARG;
+    if (!md->pi_sites || !md->pi_diffs || !md->pi_comps || !md->pi_missing || !md->pi || !md->dxy_sites || !md->dxy_diffs ||
+        !md->dxy_comps || !md->dxy_missing || !md->dxy)
+        return PB_ERR_ARG;
+    const int P = p->n_pops;
+    const long long b1 = (long long)r->win_beg[w] + 1, b2 = r->win_end[w];
+    Out out;
+    // one line: the ratio (%.10g, NA without comparisons), then the four counts
+    auto line = [&](double v, int32_t sites, int64_t diffs, int64_t comps, int64_t missing) {
+        if (comps) out.f("\t%.10g", v);
+        else out.s += "\tNA";
+        out.f("\t%d\t%lld\t%lld\t%lld\n", sites, (long long)diffs, (long long)comps, (long long)missing);
+    };
+    if (!pairs) {
+        for (int i = 0; i < P; ++i) {
+            const size_t x = (size_t)w * P + i;
+            out.f("%s\t%s\t%lld\t%lld", o->pop_names[i], o->chrom, b1, b2);
+            line(md->pi[x], md->pi_sites[x], md->pi_diffs[x], md->pi_comps[x], md->pi_missing[x]);
+        }
+    } else {
+        for (int i = 0; i < P - 1; ++i)
+            for (int j = i + 1; j < P; ++j) {
+                const size_t x = (size_t)w * P * P + i * P + (j - (i + 1));
+                out.f("%s\t%s\t%s\t%lld\t%lld", o->pop_names[i], o->pop_names[j], o->chrom, b1, b2);
+                line(md->dxy[x], md->dxy_sites[x], md->dxy_diffs[x], md->dxy_comps[x], md->dxy_missing[x]);
+            }
+    }
+    return out.copy_to(buf, cap);
+}

@@ -562,6 +562,8 @@ struct PbPileArgs {
     uint64_t *site_type;            // [span]
     uint8_t *site_flag;             // [span]  bit0 used, bit1 segregating
     uint64_t *cb_out;               // [span * n_samples] or null
+    uint64_t *acc_cov;              // [span] coverage masks, or null (PB_AN_NUCDIV_MISSING: the counting path's layout in d_acc)
+    uint32_t *acc_cnt4;             // [span] derived-base counts, or null with acc_cov
 };
 
 #define PB_WCAP 32                // segment records staged per warp and chunk
@@ -813,6 +815,7 @@ __global__ void __launch_bounds__(TP, TP == 256 ? 5 : 8) k_pileup_call(const PbP
         const int64_t o = (int64_t)p - a.span_beg;
         a.site_type[o] = s_type[lane];
         a.site_flag[o] = (uint8_t)((used ? 1 : 0) | ((used && fq > 0) ? 2 : 0));
+        if (a.acc_cov) { a.acc_cov[o] = s_cov[lane]; a.acc_cnt4[o] = s_cnt4[lane]; }
     }
 }
 

@@ -20,6 +20,7 @@
 #include "pb_abba.cuh"
 #include "pb_garud.cuh"
 #include "pb_spectrum.cuh"
+#include "pb_missing.cuh"
 
 // the number of bins of one spectrum set, or -1 for a set pb_set_spectra refuses (pb_format.cpp)
 extern "C" int64_t pb_spectrum_set_bins(const pb_params *p, const int32_t *set3);
@@ -115,8 +116,9 @@ struct pb_ctx {
     std::vector<int32_t> spec_off;         // [NS+1] first bin of each set within a window's B
     int spec_groups = 0;                   // groups of at most PB_SPECTRUM_GROUP_BINS bins (k_spectrum's grid.y)
     DevBuf d_spec_tab, d_spec;             // PbSpecSet[NS] then PbSpecGroup[groups]; the PB_AN_SPECTRUM result arena
+    DevBuf d_miss;                         // the PB_AN_NUCDIV_MISSING result arena (missing_layout)
     // pinned results
-    HostBuf h_ctr, h_small, h_seg, h_span, h_abba, h_garud, h_spec;
+    HostBuf h_ctr, h_small, h_seg, h_span, h_abba, h_garud, h_spec, h_miss;
     PbCounters ctr_host;
     bool need_valid = false;
     int need_nl = 0;
@@ -128,6 +130,7 @@ struct pb_ctx {
     pb_region_abba abba;
     pb_region_garud garud;
     pb_region_spectrum spec;
+    pb_region_nucdiv_missing miss;
     // bam_fetch_f shim staging (pb_push_record)
     std::vector<int32_t> r_pos;
     std::vector<uint32_t> r_meta, r_cig_off, r_cigar, r_base_off;
@@ -281,6 +284,23 @@ GarudLayout garud_layout(void *base, int NW, int P) {
 }
 // the PB_AN_SPECTRUM counts, [NW*B]: an arena of their own, like abba_layout
 size_t spectrum_bytes(int NW, int B) { return ((size_t)NW * B * sizeof(int32_t) + 255) & ~(size_t)255; }
+// the PB_AN_NUCDIV_MISSING arrays, [NW*P] and [NW*P*P]: an arena of their own, like abba_layout
+struct MissingLayout {
+    int32_t *pi_sites; int64_t *pi_diffs, *pi_comps, *pi_missing; double *pi;
+    int32_t *dxy_sites; int64_t *dxy_diffs, *dxy_comps, *dxy_missing; double *dxy;
+    size_t bytes;
+};
+MissingLayout missing_layout(void *base, int NW, int P) {
+    Carver cv(base);
+    MissingLayout L;
+    const size_t wp = (size_t)NW * P, wpp = (size_t)NW * P * P;
+    L.pi_sites = cv.take<int32_t>(wp); L.pi_diffs = cv.take<int64_t>(wp); L.pi_comps = cv.take<int64_t>(wp); L.pi_missing = cv.take<int64_t>(wp);
+    L.pi = cv.take<double>(wp);
+    L.dxy_sites = cv.take<int32_t>(wpp); L.dxy_diffs = cv.take<int64_t>(wpp); L.dxy_comps = cv.take<int64_t>(wpp); L.dxy_missing = cv.take<int64_t>(wpp);
+    L.dxy = cv.take<double>(wpp);
+    L.bytes = (cv.off + 255) & ~(size_t)255;
+    return L;
+}
 struct SegLayout {
     uint32_t *seg_pos, *seg_idx; uint64_t *seg_type; uint8_t *seg_ref; uint64_t *seg_cb;
     size_t bytes;
@@ -377,7 +397,10 @@ int run_pipeline(pb_ctx *c, int attempt = 0, bool allow_async = true) {
                           P.min_baseQ + qoff <= 128 && span * n < (int64_t)0x7fffffff;
     const int n_strips = (int)((span + 31) >> 5);
     PB_TRY(dev_reserve(c, c->d_site_type, sizeof(uint64_t) * (size_t)span));
-    if (fast_try) PB_TRY(dev_reserve(c, c->d_acc, (size_t)span * 12 + 16));
+    // coverage masks and derived-base counts of every position: the counting path's accumulators, also stored by the
+    // single-kernel path when PB_AN_NUCDIV_MISSING needs them
+    const bool with_miss = (c->analyses & PB_AN_NUCDIV_MISSING) != 0;
+    if (fast_try || with_miss) PB_TRY(dev_reserve(c, c->d_acc, (size_t)span * 12 + 16));
     PB_CUDA(c, cudaEventRecord(c->fk[2], s2));
     if (c->dbg[1]) cudaEventRecord(c->dbg[1], s2);
     if (c->dbg[2]) cudaEventRecord(c->dbg[2], st);
@@ -520,6 +543,8 @@ int run_pipeline(pb_ctx *c, int attempt = 0, bool allow_async = true) {
     pa.rms_thr = dp<int32_t>(c->d_rms_thr);
     pa.site_type = dp<uint64_t>(c->d_site_type); pa.site_flag = dp<uint8_t>(c->d_site_flag);
     pa.cb_out = want_cb ? dp<uint64_t>(c->d_cb) : nullptr;
+    pa.acc_cov = with_miss ? dp<uint64_t>(c->d_acc) : nullptr;
+    pa.acc_cnt4 = with_miss ? reinterpret_cast<uint32_t *>(pa.acc_cov + span) : nullptr;
     PB_CUDA(c, cudaEventRecord(c->ev[6], st));     // a per-base pass of the single-kernel path (base codes) counts as preparation: ev[6] .. ev[2]
     if (getenv("POPBAM_B200_DEBUG"))
         fprintf(stderr, "[popbam_b200] pileup path: fast=%d cap=%d want_cb=%d min_depth=%d min_snpQ=%d classic=%d N=%lld records=%u nl=%d depth_bound=%d max_span=%d ceiling=%d robust=%d\n",
@@ -776,6 +801,29 @@ int run_pipeline(pb_ctx *c, int attempt = 0, bool allow_async = true) {
         c->launches += 1;
         PB_CUDA(c, cudaGetLastError());
     }
+    // ---- pi and dxy over sites with missing calls, per (window, slice of positions), then the ratios
+    if (with_miss) {
+        const MissingLayout ml0 = missing_layout(nullptr, NW, P.n_pops);
+        PB_TRY(dev_reserve(c, c->d_miss, ml0.bytes));
+        PB_TRY(host_reserve(c, c->h_miss, ml0.bytes));
+        const MissingLayout ml = missing_layout(c->d_miss.p, NW, P.n_pops);
+        PB_CUDA(c, cudaMemsetAsync(c->d_miss.p, 0, ml.bytes, st));
+        PbMissingArgs ma;
+        memset(&ma, 0, sizeof ma);
+        ma.P = P.n_pops; ma.stripes = pb_missing_stripes(P.n_pops);
+        for (int i = 0; i < PB_MAX_SAMPLES; ++i) { ma.pop_mask[i] = P.pop_mask[i]; ma.pop_nsmpl[i] = P.pop_nsmpl[i]; }
+        ma.span_beg = c->span_beg; ma.win_beg = pa.win_beg; ma.win_end = pa.win_end;
+        ma.acc_cov = dp<uint64_t>(c->d_acc); ma.acc_cnt4 = reinterpret_cast<const uint32_t *>(ma.acc_cov + span); ma.site_type = pa.site_type;
+        ma.pi_sites = ml.pi_sites; ma.pi_diffs = ml.pi_diffs; ma.pi_comps = ml.pi_comps; ma.pi_missing = ml.pi_missing; ma.pi = ml.pi;
+        ma.dxy_sites = ml.dxy_sites; ma.dxy_diffs = ml.dxy_diffs; ma.dxy_comps = ml.dxy_comps; ma.dxy_missing = ml.dxy_missing; ma.dxy = ml.dxy;
+        int max_len = 1;
+        for (int w = 0; w < NW; ++w) max_len = std::max(max_len, c->h_wend[w] - c->h_wbeg[w]);
+        const unsigned slices = (unsigned)std::min(65535, (max_len + PB_MISSING_SLICE - 1) / PB_MISSING_SLICE);
+        k_nucdiv_missing<<<dim3((unsigned)NW, slices), PB_MISSING_THREADS, 0, st>>>(ma);
+        k_nucdiv_missing_ratio<<<nblk((int64_t)NW * P.n_pops * P.n_pops, 256), 256, 0, st>>>(ma, NW);
+        c->launches += 2;
+        PB_CUDA(c, cudaGetLastError());
+    }
     // ---- pairwise LD (ld -o 0 / -o 1, D'): keep list, tiled pair kernel, finish
     if (c->analyses & (PB_AN_LD_ZNS | PB_AN_LD_OMEGA | PB_AN_LD_DPRIME)) {
         PbLdArgs la;
@@ -817,6 +865,7 @@ int run_pipeline(pb_ctx *c, int attempt = 0, bool allow_async = true) {
     if (with_abba) PB_CUDA(c, cudaMemcpyAsync(c->h_abba.p, c->d_abba.p, abba_layout(nullptr, NW, NT).bytes, cudaMemcpyDeviceToHost, st));
     if (with_garud) PB_CUDA(c, cudaMemcpyAsync(c->h_garud.p, c->d_garud.p, garud_layout(nullptr, NW, P.n_pops).bytes, cudaMemcpyDeviceToHost, st));
     if (with_spec) PB_CUDA(c, cudaMemcpyAsync(c->h_spec.p, c->d_spec.p, spectrum_bytes(NW, NB), cudaMemcpyDeviceToHost, st));
+    if (with_miss) PB_CUDA(c, cudaMemcpyAsync(c->h_miss.p, c->d_miss.p, missing_layout(nullptr, NW, P.n_pops).bytes, cudaMemcpyDeviceToHost, st));
     if (!async && S > 0) PB_CUDA(c, cudaMemcpyAsync(c->h_seg.p, c->d_seg_type.p, sl.bytes, cudaMemcpyDeviceToHost, st));
     if (P.flags & PB_FLAG_EMIT_CB) {
         Carver cv(nullptr);
@@ -926,6 +975,13 @@ int fill_result(pb_ctx *c, pb_region_result *out) {
     if (an & PB_AN_SPECTRUM) {
         sp.n_sets = (int32_t)(c->spec_run.size() / 3); sp.n_bins = c->spec_off.back();
         sp.sets = c->spec_run.data(); sp.set_off = c->spec_off.data(); sp.counts = reinterpret_cast<const int32_t *>(c->h_spec.p);
+    }
+    pb_region_nucdiv_missing &md = c->miss;
+    memset(&md, 0, sizeof md);
+    if (an & PB_AN_NUCDIV_MISSING) {
+        const MissingLayout ml = missing_layout(c->h_miss.p, NW, P.n_pops);
+        md.pi_sites = ml.pi_sites; md.pi_diffs = ml.pi_diffs; md.pi_comps = ml.pi_comps; md.pi_missing = ml.pi_missing; md.pi = ml.pi;
+        md.dxy_sites = ml.dxy_sites; md.dxy_diffs = ml.dxy_diffs; md.dxy_comps = ml.dxy_comps; md.dxy_missing = ml.dxy_missing; md.dxy = ml.dxy;
     }
     if (an & PB_AN_DIVERGE_POP) { r.pop_div = hl.pop_div; r.div_num_snps = hl.div_num_snps; }
     if (an & (PB_AN_HAPLO_K | PB_AN_HAPLO_EHHS)) { r.nhaps = hl.nhaps; r.hdiv = hl.hdiv; }
@@ -1065,7 +1121,7 @@ void pb_destroy(pb_ctx *c) {
     if (c->stream2) cudaStreamSynchronize(c->stream2);
     if (c->stream_lo) cudaStreamSynchronize(c->stream_lo);
     for (DevBuf *b : c->bufs) if (b->p) { cudaFree(b->p); b->p = nullptr; b->cap = 0; }
-    HostBuf *hb[] = {&c->h_ctr, &c->h_small, &c->h_seg, &c->h_span, &c->h_abba, &c->h_garud, &c->h_spec};
+    HostBuf *hb[] = {&c->h_ctr, &c->h_small, &c->h_seg, &c->h_span, &c->h_abba, &c->h_garud, &c->h_spec, &c->h_miss};
     for (HostBuf *b : hb) if (b->p) cudaFreeHost(b->p);
     for (auto &ev : c->ev) if (ev) cudaEventDestroy(ev);
     for (auto &ev : c->fk) if (ev) cudaEventDestroy(ev);
@@ -1304,6 +1360,12 @@ int pb_region_get_garud(const pb_ctx *c, pb_region_garud *out) {
 int pb_region_get_spectrum(const pb_ctx *c, pb_region_spectrum *out) {
     if (!c || !out) return PB_ERR_ARG;
     *out = c->spec;
+    return PB_OK;
+}
+
+int pb_region_get_nucdiv_missing(const pb_ctx *c, pb_region_nucdiv_missing *out) {
+    if (!c || !out) return PB_ERR_ARG;
+    *out = c->miss;
     return PB_OK;
 }
 

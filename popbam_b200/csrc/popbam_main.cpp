@@ -20,7 +20,9 @@
 // for sfs only, --jsfs PREFIX: the unfolded site frequency spectra of every population and every population pair (without
 // the population of the -p sample), or of the sets --jsfs-pops A[,B[,C]] names (repeatable, in the order given), summed
 // over every window of the region and written in dadi's format to PREFIX.A.fs, PREFIX.A-B.fs, PREFIX.A-B-C.fs after the
-// last row.
+// last row; for nucdiv only, --missing PREFIX: pi and dxy of every window over the positions where some samples have no
+// call, as sums of pairwise differences and comparisons among the samples called there (the estimator of pixy), written
+// in the column layout of pixy's output to PREFIX_pi.txt and PREFIX_dxy.txt (stdout is unchanged).
 //
 // One subcommand the reference does not have: `abba -p SAMPLE`, per window Patterson's D, f_d and f_dM of population
 // triples (P1, P2, P3) against the population of SAMPLE as the outgroup; by default every triple with P1 < P2, or the
@@ -63,6 +65,8 @@ struct Options {
     bool garud = false;
     std::string jsfs;                      // sfs: --jsfs PREFIX
     std::vector<std::string> jsfs_pops;    // sfs: --jsfs-pops A[,B[,C]]
+    std::string missing;                   // nucdiv: --missing PREFIX
+    bool has_missing = false;
     long long snn_perms = 0;
     unsigned long long seed = 0;
     std::vector<std::string> triples;      // abba: --triple A,B,C
@@ -95,7 +99,10 @@ void usage(const char *cmd) {
             "         --jsfs PREFIX  sfs: unfolded spectra summed over the region, in dadi's format, to PREFIX.A.fs, PREFIX.A-B.fs\n"
             "         (every population and pair, without -p's)   --jsfs-pops A[,B[,C]] (repeatable) the sets to write instead\n"
             "         abba: -p STR a sample of the outgroup population (required)   --triple A,B,C (repeatable) the triples to\n"
-            "         report, in this order (default: every P1 < P2, P3 besides them); columns S, ABBA, BABA, D, fd, fdM [A-B-C]\n", cmd);
+            "         report, in this order (default: every P1 < P2, P3 besides them); columns S, ABBA, BABA, D, fd, fdM [A-B-C]\n"
+            "         --missing PREFIX  nucdiv: pi and dxy per window over sites with missing calls, as pixy's sums of differences\n"
+            "         and comparisons among the called samples, to PREFIX_pi.txt and PREFIX_dxy.txt in pixy's columns (each sample\n"
+            "         is one consensus call, counted as haploid, so the numbers are not pixy's diploid-genotype ones)\n", cmd);
 }
 
 Options parse(int argc, char **argv) {
@@ -123,6 +130,7 @@ Options parse(int argc, char **argv) {
             if (a == "--triple") { o.triples.push_back(val()); continue; }
             if (a == "--jsfs") { o.jsfs = val(); if (o.jsfs.empty()) fatal("--jsfs needs a file name prefix"); continue; }
             if (a == "--jsfs-pops") { o.jsfs_pops.push_back(val()); continue; }
+            if (a == "--missing") { o.missing = val(); o.has_missing = true; continue; }
             if (a == "--gpus") o.gpus = atoi(val());
             else if (a == "--shard-mb") o.shard_mb = atof(val());
             else if (a == "--threads") o.threads = atoi(val());
@@ -188,6 +196,8 @@ Options parse(int argc, char **argv) {
     if (o.garud && o.cmd != "haplo") fatal("--garud is only available for haplo");
     if ((!o.jsfs.empty() || !o.jsfs_pops.empty()) && o.cmd != "sfs") fatal("--jsfs and --jsfs-pops are only available for sfs");
     if (!o.jsfs_pops.empty() && o.jsfs.empty()) fatal("--jsfs-pops goes with --jsfs");
+    if (o.has_missing && o.cmd != "nucdiv") fatal("--missing is only available for nucdiv");
+    if (o.has_missing && o.missing.empty()) fatal("--missing needs a file name prefix");
     if (o.cmd == "abba" && !o.has_p) fatal("abba needs -p SAMPLE: a sample of the outgroup population");
     return o;
 }
@@ -203,6 +213,7 @@ struct Shard {
     std::string text;
     std::vector<int64_t> spec;  // --jsfs: the shard's spectra summed over its windows, and its num_sites
     int64_t spec_sites = 0;
+    std::string miss_pi, miss_dxy;   // --missing: the shard's lines of PREFIX_pi.txt and PREFIX_dxy.txt
     std::string error;
     int state = 0;              // 0 pending, 1 decoded, 2 done
 };
@@ -225,6 +236,7 @@ struct Run {
     std::vector<int32_t> spec_sets;        // --jsfs: 3 population indices per set (-1: unused slot), and their bins
     std::vector<int64_t> spec_off;
     pb_ctx *spec_ctx = nullptr;            // --jsfs: worker 0's context, kept for pb_format_spectrum_dadi
+    FILE *miss_pi = nullptr, *miss_dxy = nullptr;   // --missing: PREFIX_pi.txt, PREFIX_dxy.txt
     // error-model tables, built once on the host (while the files are opened) and shared by every context
     std::vector<double> fk, beta, lhet;
     std::shared_future<void> tables_ready;
@@ -336,7 +348,7 @@ void gpu_worker(Run *R, int g, int G, int device) {
              pb_set_abba(ctx, R->abba_og, (int32_t)(R->abba_triples.size() / 3), R->abba_triples.data()) != PB_OK) err = pb_last_error(ctx);
     else if ((R->analysis & PB_AN_SPECTRUM) &&
              pb_set_spectra(ctx, (int32_t)(R->spec_sets.size() / 3), R->spec_sets.data()) != PB_OK) err = pb_last_error(ctx);
-    const uint32_t rows = R->analysis & ~PB_AN_SPECTRUM;     // the spectra add no columns
+    const uint32_t rows = R->analysis & ~(PB_AN_SPECTRUM | PB_AN_NUCDIV_MISSING);     // the spectra and --missing add no columns
     std::vector<const char *> pops, smps;
     for (auto &s : R->st.pops) pops.push_back(s.c_str());
     for (auto &s : R->st.samples) smps.push_back(s.c_str());
@@ -360,6 +372,7 @@ void gpu_worker(Run *R, int g, int G, int device) {
             pb_region_abba abba;
             pb_region_garud garud;
             pb_region_spectrum spec;
+            pb_region_nucdiv_missing miss;
             int rc = pb_region_begin(ctx, R->analysis, sh.w1 - sh.w0, &R->wb[sh.w0], &R->we[sh.w0]);
             {
                 int64_t nr = 0, nc = 0, nb = 0;
@@ -383,6 +396,7 @@ void gpu_worker(Run *R, int g, int G, int device) {
             if (rc == PB_OK) rc = pb_region_get_abba(ctx, &abba);
             if (rc == PB_OK) rc = pb_region_get_garud(ctx, &garud);
             if (rc == PB_OK) rc = pb_region_get_spectrum(ctx, &spec);
+            if (rc == PB_OK) rc = pb_region_get_nucdiv_missing(ctx, &miss);
             auto format = [&](int w) {
                 if (rows & PB_AN_ABBA) return pb_format_window_abba(ctx, &res, &abba, w, &po, line.data(), (int64_t)line.size());
                 if (rows & PB_AN_GARUD) return pb_format_window_garud(ctx, &res, &garud, w, rows, &po, line.data(), (int64_t)line.size());
@@ -403,6 +417,16 @@ void gpu_worker(Run *R, int g, int G, int device) {
                     const int32_t *x = spec.counts + (size_t)w * spec.n_bins;
                     for (int b = 0; b < spec.n_bins; ++b) sh.spec[(size_t)b] += x[b];
                     sh.spec_sites += res.num_sites[w];
+                }
+            }
+            for (int pairs = 0; rc == PB_OK && sh.error.empty() && (R->analysis & PB_AN_NUCDIV_MISSING) && pairs < 2; ++pairs) {
+                std::string &txt = pairs ? sh.miss_dxy : sh.miss_pi;         // every window, whatever -k says
+                for (int w = 0; w < res.n_windows; ++w) {
+                    auto fmt = [&]() { return pb_format_window_nucdiv_missing(ctx, &res, &miss, w, pairs, &po, line.data(), (int64_t)line.size()); };
+                    int64_t k = fmt();
+                    if (k >= (int64_t)line.size()) { line.resize((size_t)k + 16); k = fmt(); }
+                    if (k < 0) { sh.error = "formatting failed"; break; }
+                    txt.append(line.data(), (size_t)k);
                 }
             }
         } else if (sh.error.empty()) sh.error = err;
@@ -692,10 +716,28 @@ int main(int argc, char **argv) {
         R.analysis |= PB_AN_SPECTRUM;
         spectrum_sets(R);
     }
+    if (o.has_missing) {
+        R.analysis |= PB_AN_NUCDIV_MISSING;
+        R.miss_pi = fopen((o.missing + "_pi.txt").c_str(), "w");
+        if (!R.miss_pi) fatal("Cannot write file " + o.missing + "_pi.txt");
+        R.miss_dxy = fopen((o.missing + "_dxy.txt").c_str(), "w");
+        if (!R.miss_dxy) fatal("Cannot write file " + o.missing + "_dxy.txt");
+        // pixy's columns (each sample is one consensus call here, counted as haploid)
+        fputs("pop\tchromosome\twindow_pos_1\twindow_pos_2\tavg_pi\tno_sites\tcount_diffs\tcount_comparisons\tcount_missing\n", R.miss_pi);
+        fputs("pop1\tpop2\tchromosome\twindow_pos_1\twindow_pos_2\tavg_dxy\tno_sites\tcount_diffs\tcount_comparisons\tcount_missing\n", R.miss_dxy);
+    }
+    // --missing: close the files (after the last shard's lines), a failed write is fatal
+    auto close_missing = [&R]() {
+        if (!R.miss_pi) return;
+        const bool ok_pi = !ferror(R.miss_pi) && fclose(R.miss_pi) == 0, ok_dxy = !ferror(R.miss_dxy) && fclose(R.miss_dxy) == 0;
+        R.miss_pi = R.miss_dxy = nullptr;
+        if (!ok_pi) fatal("Cannot write file " + R.opt.missing + "_pi.txt");
+        if (!ok_dxy) fatal("Cannot write file " + R.opt.missing + "_dxy.txt");
+    };
 
     // window grid of the region, then shards = runs of whole windows
     const int64_t nw = pb_window_grid(R.beg, R.end, o.window ? o.win_size : 0, 0, nullptr, nullptr);
-    if (nw < 1) return 0;       // region shorter than one window: the reference's loop does not execute
+    if (nw < 1) { close_missing(); return 0; }       // region shorter than one window: the reference's loop does not execute
     R.wb.resize((size_t)nw); R.we.resize((size_t)nw);
     pb_window_grid(R.beg, R.end, o.window ? o.win_size : 0, nw, R.wb.data(), R.we.data());
     const int64_t shard_bp = std::max<int64_t>(1, (int64_t)(o.shard_mb * 1e6));
@@ -761,8 +803,12 @@ int main(int argc, char **argv) {
             R.cv.wait(lk, [&] { return sh.state == 2; });
         }
         if (!sh.error.empty()) { fflush(stdout); fprintf(stderr, "popbam runtime error:\n%s\nExiting program\n", sh.error.c_str()); rc = 1; }
-        else fwrite(sh.text.data(), 1, sh.text.size(), stdout);
+        else {
+            fwrite(sh.text.data(), 1, sh.text.size(), stdout);
+            if (R.miss_pi) { fwrite(sh.miss_pi.data(), 1, sh.miss_pi.size(), R.miss_pi); fwrite(sh.miss_dxy.data(), 1, sh.miss_dxy.size(), R.miss_dxy); }
+        }
         sh.text.clear(); sh.text.shrink_to_fit();
+        sh.miss_pi.clear(); sh.miss_pi.shrink_to_fit(); sh.miss_dxy.clear(); sh.miss_dxy.shrink_to_fit();
         for (size_t b = 0; b < sh.spec.size(); ++b) spec_total[b] += sh.spec[b];
         spec_sites += sh.spec_sites;
         {
@@ -774,6 +820,7 @@ int main(int argc, char **argv) {
     }
     for (auto &t : th) t.join();
     fflush(stdout);
+    close_missing();
     if (R.analysis & PB_AN_SPECTRUM) {
         write_spectra(R, spec_total, spec_sites);
         pb_destroy(R.spec_ctx);
